@@ -8,6 +8,10 @@ captions/sec as a secondary figure), contract of the task prompt:
 Prints ONE JSON line.  Default workload = BASELINE.json configs[1]: teacher-forced training step (forward +
 backward + Adam, dropout on), bf16, batch 256 per GPU, 36 regions x 2048-d, caption length 22 (T = 21 decoder
 positions), vocab 10k, ctor-default Transformer (d512/8h/2048/6+6).  Synthetic data, random-init weights.
+`--dump-outputs DIR` writes the loss and the updated parameters of the last timed train step as DIR/<name>.npy; inputs,
+weights and dropout streams are seeded, so two builds run with the same arguments can be compared array for array.
+Not bit for bit: the step reduces weight gradients with fp32 atomics, so two runs of one build already differ (B200 at
+1000 W, --steps 20 --warmup 5: losses by 1e-6 relative, single sampled weights by up to 9e-2 of their tensor's max).
 N > 1 = data parallel (weak scaling, 256 samples per rank), gradients summed by bucketed NCCL all-reduces that
 overlap the backward.  Other BASELINE configs through `--workload`:
     modelA      configs[1] (+ configs[2] beam-5/3/greedy decode of 512 images, configs[0] model B greedy B=8 as extras)
@@ -41,6 +45,7 @@ MODEL_C = dict(num_vocab=30000, max_length=22, encode_dim_positions=84, encode_d
                decode_q_k_dim=1024, decode_v_dim=1024, decode_hidden_size=4096, decode_num_blocks=6, decode_num_heads=16)
 CAP_LEN = 22
 DECODE_BATCH = 512
+DUMP_SAMPLE = 1 << 16      # --dump-outputs: elements kept per parameter tensor (190 tensors of model A / C: < 26 MB)
 
 # SURVEY.md §8(d): algorithmic matmul FLOPs as the reference executes them (fwd+bwd) / KV-cached beam-5, 21 steps
 WORKLOADS = {
@@ -116,6 +121,27 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def output_sample(loss: torch.Tensor, named_params) -> dict:
+    """What a caller of the training step holds after its last step, as float32 host arrays keyed by file name: the
+    loss and every updated parameter -- whole up to DUMP_SAMPLE elements, larger ones at DUMP_SAMPLE positions drawn
+    from a generator seeded per tensor, so that two runs or two builds sample the same elements."""
+    out = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+    for name, q in named_params:
+        flat = q.detach().reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            idx = torch.randint(flat.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            flat = flat[idx.to(flat.device)]
+        out["param." + name] = flat.float().cpu().numpy()
+    return out
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------- the reference on the CPU
@@ -373,6 +399,8 @@ def run_ours(args):
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
     final_loss = float(loss_dev)
+    if args.dump_outputs and rank == 0:    # before the end-to-end loops below step the weights further
+        write_outputs(args.dump_outputs, output_sample(loss_dev, model.named_parameters()))
     value = world * BATCH * args.steps / (ms / 1e3)
 
     # ---------------- end-to-end: pinned host inputs -> H2D (copy stream, double buffered) -> step -> D2H loss
@@ -637,7 +665,12 @@ def main():
     ap.add_argument("--no-decode", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ncu-region", action="store_true", help="wrap one eager step in cudaProfilerStart/Stop")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and the updated parameters of the last timed train step as DIR/<name>.npy "
+                         "(float32; parameters above %d elements as a fixed seeded sample)" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
     if args.steps is None:
         args.steps = 20 if args.impl == "reference" else 100
     if args.impl == "reference":

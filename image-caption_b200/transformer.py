@@ -8,6 +8,8 @@ is what the fused Adam / gradient all-reduce operate on.
 """
 from __future__ import annotations
 
+import contextlib
+import gc
 import math
 import os
 from typing import List, Optional
@@ -45,6 +47,23 @@ def _set_nested(root: nn.Module, dotted: str, value, is_buffer: bool) -> None:
         mod.register_buffer(parts[-1], value)
     else:
         mod.register_parameter(parts[-1], value)
+
+
+@contextlib.contextmanager
+def _graph_capture(graph: torch.cuda.CUDAGraph):
+    """`torch.cuda.graph(graph)` with Python's cycle collector held off.  A model and its captured steps reference each
+    other, so a dropped model lives until a collection; if that collection runs inside a capture, it destroys the
+    model's CUDA graphs there, and destroying a graph while a stream captures invalidates the capture
+    (cudaErrorStreamCaptureInvalidated).  torch does not collect before a capture, so dead models are collected here."""
+    enabled = gc.isenabled()
+    gc.collect()
+    gc.disable()
+    try:
+        with torch.cuda.graph(graph):
+            yield
+    finally:
+        if enabled:
+            gc.enable()
 
 
 def _check_tape(eng: CaptionEngine, gen: int) -> None:
@@ -728,7 +747,7 @@ class GraphedDecode:
             nsplit = max(1, min(int(os.environ.get("ICAP_DECODE_STREAMS", "1")), B // 64 if B >= 128 else 1))
             while B % nsplit:
                 nsplit -= 1
-            with torch.cuda.graph(self.graph):
+            with _graph_capture(self.graph):
                 if nsplit == 1:
                     self.out = eng.decode(self.feats, self.pos, **self.kw)
                 else:
@@ -840,12 +859,12 @@ class GraphedTrainStep:
         self.graph = torch.cuda.CUDAGraph()
         n0 = _native.launch_count
         if self.dp is None:
-            with torch.cuda.graph(self.graph):
+            with _graph_capture(self.graph):
                 self.out2 = self._one_step()
         elif self.dp.overlap:
             # ONE graph: forward, backward with the bucketed NCCL all-reduces on the communication stream, Adam
             try:
-                with torch.cuda.graph(self.graph):
+                with _graph_capture(self.graph):
                     self.out2 = self.dp.step_eager(eng, self.feats, self.pos, self.cap, self.lr)
                 self.single_graph_dp = True
             except Exception as exc:     # NCCL not capturable in this build: fall back to the split graphs below
@@ -857,10 +876,10 @@ class GraphedTrainStep:
                 self.graph = torch.cuda.CUDAGraph()
         if self.dp is not None and not self.dp.overlap:
             # graph 1: zero_grad/forward/backward ; NCCL all-reduce (eager) ; graph 2: 1/count + Adam
-            with torch.cuda.graph(self.graph):
+            with _graph_capture(self.graph):
                 self.out2 = eng.forward_backward(self.feats, self.pos, self.cap)
             self.graph2 = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self.graph2):
+            with _graph_capture(self.graph2):
                 self.dp.finish(eng, self.lr)
         self.launches_per_step = _native.launch_count - n0
 

@@ -16,9 +16,8 @@ product package (``image-caption_b200/``) never does and has no CPU fallback.
 Parity pin: the reference ships no tests / golden vectors (SURVEY.md §4, §8c), so
 this oracle is pinned against OUTPUTS OF THE REFERENCE ITSELF: the fixtures in
 ``tests/golden/*.pt`` were produced by ``tests/golden/make_golden.py`` importing the
-unmodified reference classes from /root/reference, and ``tests/test_oracle.py``
-checks every function here against them (and, when /root/reference is mounted,
-against the live reference at more configs).
+unmodified reference classes, and ``tests/test_oracle.py`` checks every function
+here against them.
 
 All hot-path arithmetic in the reference is PyTorch ATen (pinned torch==1.7.1,
 requirements.txt:57); the oracle uses the same ATen CPU operators through

@@ -1,11 +1,14 @@
 """CPU-side checks of the measurement harness (no GPU): the nvidia-smi clock / throttle parser of bench.py, the
 reference arm's JSON line (contract keys, bounded per-step sample, every host thread even under torchrun's
-OMP_NUM_THREADS=1), and the bucket schedule of the data-parallel gradient exchange as a property over random tapes."""
+OMP_NUM_THREADS=1), the --dump-outputs sample, and the bucket schedule of the data-parallel gradient exchange as a
+property over random tapes."""
 import json
 import os
 import random
 import subprocess
 import sys
+
+import numpy as np
 
 import icap_loader
 
@@ -104,6 +107,40 @@ def test_reference_arm_bounds_its_sample_by_the_step_count():
         assert 4 <= bs <= 256 and bs % 4 == 0
         assert bs * (steps + warm) / rate <= 200.0 or bs == 4
     assert max(4, min(256, int(110.0 * 180.0 / 25) // 4 * 4)) == 256       # the driver's --steps 20 --warmup 5: full batch
+
+
+def test_output_sample_is_seeded_float32_and_bounded(monkeypatch):
+    """--dump-outputs: the same model gives the same arrays (fixed sample positions), every array is float32, small
+    parameters are kept whole, and every workload's dump stays under 64 MB."""
+    import math
+
+    import torch
+    b = _bench()
+    kw = dict(num_vocab=97, max_length=6, encode_dim_positions=12, encode_dim_features=300, output_name="x",
+              encode_input_size=32, encode_q_k_dim=32, encode_v_dim=32, encode_hidden_size=64, encode_num_blocks=1,
+              encode_num_heads=4, dim_word_embedding=32, decode_input_size=32, decode_q_k_dim=32, decode_v_dim=32,
+              decode_hidden_size=64, decode_num_blocks=1, decode_num_heads=4)
+    torch.manual_seed(0)
+    m = pkg.Transformer(device=None, **kw)
+    with monkeypatch.context() as mp:
+        mp.setattr(b, "DUMP_SAMPLE", 1000)         # below the 300 x 32 input projection: exercises the sampled branch
+        a1 = b.output_sample(torch.tensor(2.5), m.named_parameters())
+        a2 = b.output_sample(torch.tensor(2.5), m.named_parameters())
+    params = dict(m.named_parameters())
+    assert set(a1) == {"loss"} | {"param." + n for n in params} and float(a1["loss"][0]) == 2.5
+    for name, arr in a1.items():
+        assert arr.dtype == np.float32 and np.array_equal(arr, a2[name]), name
+        if name != "loss":
+            q = params[name[len("param."):]]
+            assert arr.shape == ((q.numel(),) if q.numel() <= 1000 else (1000,)), name
+            if q.numel() <= 1000:
+                assert np.array_equal(arr, q.detach().reshape(-1).numpy()), name
+            else:
+                assert np.isin(arr, q.detach().reshape(-1).numpy()).all(), name
+    assert any(q.numel() > 1000 for q in params.values())
+    for wl in b.WORKLOADS.values():
+        shapes = pkg.param_layout(pkg.ModelConfig(**wl["kw"])).values()
+        assert 4 * (1 + sum(min(math.prod(s), b.DUMP_SAMPLE) for s in shapes)) <= 64 << 20
 
 
 def test_grad_buckets_property_random_tapes():
