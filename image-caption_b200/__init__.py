@@ -9,6 +9,7 @@ from .engine import ModelConfig, CaptionEngine, param_layout, flat_offsets   # n
 from .transformer import Transformer, PolicyNetwork, GraphedTrainStep, GraphedDecode, DataParallel, GradBuckets                       # noqa: F401
 from .engine import RegionBatch                                              # noqa: F401
 from .feed import RegionCache, PrefetchLoader                                # noqa: F401
+from .metrics import CaptionScorer, CaptionReward                           # noqa: F401
 from . import _native                                                        # noqa: F401
 
-__all__ = ["Transformer", "PolicyNetwork", "GraphedTrainStep", "GraphedDecode", "DataParallel", "GradBuckets", "RegionCache", "RegionBatch", "PrefetchLoader", "ModelConfig", "CaptionEngine", "param_layout", "flat_offsets"]
+__all__ = ["Transformer", "PolicyNetwork", "GraphedTrainStep", "GraphedDecode", "DataParallel", "GradBuckets", "RegionCache", "RegionBatch", "PrefetchLoader", "ModelConfig", "CaptionEngine", "param_layout", "flat_offsets", "CaptionScorer", "CaptionReward"]

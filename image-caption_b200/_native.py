@@ -63,6 +63,10 @@ SIGNATURES = {
     "icap_p2p_reduce_scatter": [P, I, I, L, L, I, P],
     "icap_p2p_all_gather": [P, I, I, L, L, I, P],
     "icap_p2p_allreduce_nvls": [P, I, I, L, L, I, P],
+    "icap_caption_cook": [P, I, L, L, L, P, P, P, P, P, P],
+    "icap_caption_df": [L, P, L, P, P, P, P, L, P, P],
+    "icap_caption_ref_prep": [L, L, P, P, P, L, P, P, L, P, P],
+    "icap_caption_score": [P, I, L, L, L, P, L, P, L, P, P, P, P, P, P, P, P, L, P, P, F, F, P, P],
 }
 
 

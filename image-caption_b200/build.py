@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libicap.so")
-SOURCES = ["misc.cu", "gemm_simt.cu", "gemm_tc.cu", "norm.cu", "attention.cu", "attention_mma.cu", "loss.cu", "gemm_ln.cu", "gemm_small.cu", "conv.cu", "p2p.cu"]
+SOURCES = ["misc.cu", "gemm_simt.cu", "gemm_tc.cu", "norm.cu", "attention.cu", "attention_mma.cu", "loss.cu", "gemm_ln.cu", "gemm_small.cu", "conv.cu", "p2p.cu", "metrics.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

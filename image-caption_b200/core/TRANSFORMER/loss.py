@@ -1,15 +1,17 @@
 """Losses of the RL fine-tuning mode -- the reference's shipped default CAPTION_MODEL='RL_Transformer'
 (core/config.py:14 -> core/models.py:138-211 -> core/TRANSFORMER/loss.py:31-219) -- for the drop-in PolicyNetwork.
 
-The reference's reward is CIDEr-D / BLEU-4 from pycocoevalcap on decoded strings (loss.py:160-186): CPU string metrics
-of an un-vendored third-party package (README.md:10-17), outside the hot path.  Here the reward is an INJECTABLE
-callable `reward_fn(target_ids [B, T] ndarray, sample_ids [B, T] ndarray) -> [B] ndarray` (plug pycocoevalcap in when it
-is installed); the default is a clipped n-gram precision on token ids.  Everything differentiable follows the reference:
+The reference's reward is CIDEr-D / BLEU-4 from pycocoevalcap on decoded strings (loss.py:160-186).  Here the reward is an
+INJECTABLE callable `reward_fn(target_ids [B, T] ndarray, sample_ids [B, T] ndarray) -> [B] ndarray`; the default is a
+clipped n-gram precision on token ids.  `image_caption_b200.CaptionReward(CIDER_REWARD_WEIGHT, BLEU_REWARD_WEIGHT)` is
+the reference's reward computed on the GPU from the ids; a reward_fn with an `on_device(target, sample)` method is
+called with the device tensors and its [B] result never leaves the device.  Everything differentiable follows the
+reference:
   loss = (1 - w) * CrossEntropy(logits, target[:, 1:]; ignore pad)  +  w * structure loss          (loss.py:53-73)
   structure loss = sum(-log p(sample_t) * mask_t * (score - baseline)) / sum(mask)                  (loss.py:127-158)
 with mask_t = 1 for t = 0 and for every position after a non-pad sampled token, and the "baseline" of loss.py:146
 ((sum over the size-1 score axis - score) / 1 = 0).  Tensors stay on the device (the reference moves the [B, T, V]
-logits to the CPU first, models.py:190-193); only the sampled ids cross PCIe for the reward.
+logits to the CPU first, models.py:190-193); only a host reward_fn makes the sampled ids cross PCIe.
 """
 import numpy as np
 import torch
@@ -64,8 +66,11 @@ class StructureCriterion(nn.Module):
     def forward(self, output, sequence, target):
         mask = (sequence > 0).to(output)
         mask = torch.cat([mask.new_ones(mask.size(0), 1), mask[:, :-1]], 1)
-        scores = self.reward_fn(target.cpu().numpy(), sequence.cpu().numpy())
-        scores = torch.as_tensor(np.asarray(scores, dtype=np.float32)).to(output).view(-1, 1)
+        if hasattr(self.reward_fn, 'on_device'):
+            scores = self.reward_fn.on_device(target, sequence).to(output).view(-1, 1).clone()
+        else:
+            scores = self.reward_fn(target.cpu().numpy(), sequence.cpu().numpy())
+            scores = torch.as_tensor(np.asarray(scores, dtype=np.float32)).to(output).view(-1, 1)
         out = {'reward': scores}
         if self.entropy_reward_weight > 0:
             entropy = -(F.softmax(output, dim=2) * F.log_softmax(output, dim=2)).sum(2).detach()
@@ -80,7 +85,13 @@ class StructureCriterion(nn.Module):
 
 class ReinforcementLearningLoss(nn.Module):
     """loss.py:31-76.  The reference's scorer weights (cider / bleu / self-cider) configure pycocoevalcap and are
-    accepted for signature compatibility; the reward itself comes from `reward_fn`."""
+    accepted for signature compatibility; the reward itself comes from `reward_fn` (pass
+    `CaptionReward(cider_reward_weight, bleu_reward_weight)` for the reference's reward).
+
+    `forward` receives only `target`, so the reward scores sample i against the single reference target_i[1:]
+    (gts = {i: [target_i]} over the batch: document frequencies from the batch's targets, ref_len = log(B)).  The
+    reference's loss.py:160-186 is not part of this port; that reading is the one its signature allows.  The self-CIDEr
+    weight stays unused: the arg-max sampler draws one sample per image."""
 
     def __init__(self, structure_loss_weight, cider_reward_weight=0, bleu_reward_weight=0, entropy_reward_weight=0,
                  self_cider_reward_weight=0, word_to_idx_path=None, pad_idx=0, reward_fn=None):

@@ -49,19 +49,22 @@ class MODEL_init:
     def compute_loss(self):
         raise NotImplementedError
 
-    def generate_caption(self, object_features, position_features, beam_size=None):
+    def generate_caption_ids(self, object_features, position_features, beam_size=None):
+        """generate_caption without the decoding: (caption id rows on the device, attention list or None), the
+        input of image_caption_b200.CaptionScorer."""
         if beam_size in [None, 1]:
-            caption_vector, attention_list = self.model.generate_caption_vector(
-                object_features=object_features.to(DEVICE), position_features=position_features.to(DEVICE))
-            return self.decode_captions(caption_vector.cpu().numpy()), attention_list
+            return self.model.generate_caption_vector(object_features=object_features.to(DEVICE),
+                                                      position_features=position_features.to(DEVICE))
         elif isinstance(beam_size, int) and beam_size > 1:
-            caption_vector = self.model.beam_search(object_features=object_features.to(DEVICE),
-                                                    position_features=position_features.to(DEVICE),
-                                                    beam_size=beam_size)
-            return self.decode_captions(caption_vector.cpu().numpy()), None
+            return self.model.beam_search(object_features=object_features.to(DEVICE),
+                                          position_features=position_features.to(DEVICE), beam_size=beam_size), None
         else:
             assert isinstance(beam_size, int)
             assert beam_size > 1 or beam_size in [None, 1]
+
+    def generate_caption(self, object_features, position_features, beam_size=None):
+        caption_vector, attention_list = self.generate_caption_ids(object_features, position_features, beam_size)
+        return self.decode_captions(caption_vector.cpu().numpy()), attention_list
 
     def decode_captions(self, caption_vector):
         return decode_captions(captions=caption_vector, index_to_word=self.idx_to_word)
@@ -120,20 +123,23 @@ class TRANSFORMER(MODEL_init):
             return self.model(object_features=cache.batch(image_idxs), position_features=None,
                               target_caption=target_caption.to(DEVICE))
 
-    def generate_caption_cached(self, cache, image_idxs, beam_size=None):
+    def generate_caption_ids_cached(self, cache, image_idxs, beam_size=None):
         batch = cache.batch(image_idxs)
         if beam_size in [None, 1]:
-            caption_vector, attention_list = self.model.generate_caption_vector(batch, None)
-            return self.decode_captions(caption_vector.cpu().numpy()), attention_list
+            return self.model.generate_caption_vector(batch, None)
         assert isinstance(beam_size, int) and beam_size > 1
-        caption_vector = self.model.beam_search(batch, None, beam_size=beam_size)
-        return self.decode_captions(caption_vector.cpu().numpy()), None
+        return self.model.beam_search(batch, None, beam_size=beam_size), None
+
+    def generate_caption_cached(self, cache, image_idxs, beam_size=None):
+        caption_vector, attention_list = self.generate_caption_ids_cached(cache, image_idxs, beam_size)
+        return self.decode_captions(caption_vector.cpu().numpy()), attention_list
 
 
 class SelfCriticNetwork(MODEL_init):
     """core/models.py:138-211: PolicyNetwork (logits out) + ReinforcementLearningLoss, torch.optim.Adam on the flat
-    parameter views.  `reward_fn(target_ids, sample_ids) -> [B]` replaces the pycocoevalcap scorers (un-vendored CPU
-    string metrics); forward, the log-softmax/arg-max "sampler" and the whole backward run on libicap."""
+    parameter views.  `reward_fn(target_ids, sample_ids) -> [B]` is injectable (default: clipped n-gram precision);
+    `image_caption_b200.CaptionReward(CIDER_REWARD_WEIGHT, BLEU_REWARD_WEIGHT)` is the reference's CIDEr-D + BLEU-4
+    reward on the GPU.  Forward, the log-softmax/arg-max "sampler" and the whole backward run on libicap."""
 
     def __init__(self, reward_fn=None):
         super(SelfCriticNetwork, self).__init__()

@@ -1,7 +1,8 @@
 """`python main.py train | evaluation | demo` -- same entry points and arguments as the reference's main.py
 (main.py:25,156,193).  `fire` is not installable offline, so a small fire-compatible argv shim dispatches
 `--beam-size 5` / `--beam_size=5` style flags.  Without the COCO artefacts (data/<MODEL_NAME>/...) the loops run
-on synthetic data of the reference's shapes; metric scoring (pycocoevalcap, Java) is out of scope."""
+on synthetic data of the reference's shapes.  Captions are scored on the GPU from their ids (BLEU-1..4, ROUGE-L, CIDEr,
+CIDEr-D: image_caption_b200.CaptionScorer); METEOR needs Java and is not computed."""
 import os
 import sys
 import time
@@ -14,7 +15,8 @@ from core.models import DEVICE, TRANSFORMER, SelfCriticNetwork
 from core.TRANSFORMER.model import PrefetchLoader
 from core.config import *          # noqa: F401,F403
 from core.dataset import IndexedCaptions, SyntheticCaptionDataset, TestDataset, TrainDataset
-from core.utils import save_pickle
+from core.utils import save_pickle, write_scores
+from image_caption_b200.metrics import MAX_VOCAB, CaptionReward, CaptionScorer     # registered by core.models
 
 MODEL = None
 
@@ -37,16 +39,47 @@ def _dataset(with_captions, n_images, split='train'):
                                    _model().num_vocab, with_captions=with_captions, seed=seed)
 
 
+def _scorer(ds, num_vocab):
+    """CaptionScorer over the split's reference captions (None when the vocabulary is too large for the id packing)."""
+    if num_vocab > MAX_VOCAB:
+        print(f'[scores] a vocabulary of {num_vocab} words is above {MAX_VOCAB}: captions are not scored')
+        return None
+    return CaptionScorer(ds.data['captions'], ds.data['image_idxs'], num_vocab, DEVICE)
+
+
+def _score(scorer, id_batches, n_img):
+    """Scores of the caption ids decoded per image ([(image numbers, id rows)]) -> (corpus dict, seconds)."""
+    t0 = time.time()
+    width = id_batches[0][1].shape[1]
+    ids = torch.zeros(n_img, width, dtype=torch.long, device=DEVICE)
+    for idxs, rows in id_batches:
+        ids[torch.as_tensor(idxs).to(DEVICE, torch.long)] = rows.to(DEVICE, torch.long)
+    _, corpus = scorer.score(ids, torch.arange(n_img, device=DEVICE))
+    return corpus, time.time() - t0
+
+
+def _scores_line(corpus):
+    return '  '.join(f'{k} {v:.4f}' for k, v in corpus.items())
+
+
 def _collate_idx(items):
     cols = list(zip(*items))
     return tuple(torch.as_tensor(np.asarray(c)) for c in cols)
 
 
-def train(num_images=64, max_iters=None, region_cache=REGION_CACHE):
-    """main.py:25-153 without TensorBoard / metric scoring: train_step per batch, train/valid loss every 100
-    iterations, validation captions + checkpoint per epoch.  With `region_cache` (default) both splits' region features
-    are packed into HBM once and the loaders yield (image number, caption) only."""
+def train(num_images=64, max_iters=None, region_cache=REGION_CACHE, reward='ngram'):
+    """main.py:25-153 without TensorBoard: train_step per batch, train/valid loss every 100 iterations, validation
+    captions, their scores (valid_scores.txt) and a checkpoint per epoch.  With `region_cache` (default) both splits'
+    region features are packed into HBM once and the loaders yield (image number, caption) only.
+    `reward` (RL_Transformer): 'ngram' = the clipped n-gram precision stand-in, 'cider' = the reference's
+    CIDER_REWARD_WEIGHT * CIDEr-D + BLEU_REWARD_WEIGHT * BLEU-4 computed on the GPU."""
+    if reward not in ('ngram', 'cider'):
+        raise ValueError(f"--reward must be 'ngram' or 'cider', not {reward!r}")
     model = _model()
+    if reward == 'cider':
+        if not isinstance(model, SelfCriticNetwork):
+            raise ValueError("--reward cider needs CAPTION_MODEL = 'RL_Transformer' (the Transformer has no reward)")
+        model.loss.structure_criterion.reward_fn = CaptionReward(CIDER_REWARD_WEIGHT, BLEU_REWARD_WEIGHT)
     model_dir = os.path.join(OUTPUT_PATH, 'model/')
     target_dir = os.path.join(DATA_PATH, f'valid/{OUTPUT_NAME}/')
     os.makedirs(model_dir, exist_ok=True)
@@ -64,15 +97,16 @@ def train(num_images=64, max_iters=None, region_cache=REGION_CACHE):
                                   collate_fn=_collate_idx)
         step = lambda b: model.train_step_cached(t_cache, b[0], b[1])                                     # noqa: E731
         loss_of = lambda cache, b: model.compute_loss_cached(cache, b[0], b[1])                           # noqa: E731
-        caption_of = lambda b: (model.generate_caption_cached(v_cache, b[0])[0], b[0])                    # noqa: E731
+        caption_of = lambda b: (model.generate_caption_ids_cached(v_cache, b[0])[0], b[0])                # noqa: E731
     else:
         t_cache = v_cache = None
         train_loader = DataLoader(train_ds, batch_size=BATCH_SIZE, shuffle=True)
         valid_loader = DataLoader(valid_ds, batch_size=BATCH_SIZE, shuffle=False)
         step = lambda b: model.train_step(b[0], b[1], b[2])                                               # noqa: E731
         loss_of = lambda cache, b: model.compute_loss(b[0], b[1], b[2])                                   # noqa: E731
-        caption_of = lambda b: (model.generate_caption(b[0], b[1])[0], b[3])                              # noqa: E731
+        caption_of = lambda b: (model.generate_caption_ids(b[0], b[1])[0], b[3])                          # noqa: E731
     eval_t, eval_v = next(iter(train_loader)), next(iter(valid_loader))
+    valid_scorer = _scorer(valid_ds, model.num_vocab)
     it = 0
     for epoch in range(1, NUM_EPOCH + 1):
         print(f'Epoch {epoch}')
@@ -88,12 +122,17 @@ def train(num_images=64, max_iters=None, region_cache=REGION_CACHE):
             if max_iters and it >= max_iters:
                 break
         model.model.eval()
-        valid_caption = [''] * valid_ds.len_image
+        valid_caption, id_batches = [''] * valid_ds.len_image, []
         for batch in valid_loader:
-            captions, idxs = caption_of(batch)
-            for idx, caption in zip(idxs, captions):
+            ids, idxs = caption_of(batch)
+            id_batches.append((idxs, ids))
+            for idx, caption in zip(idxs, model.decode_captions(ids.cpu().numpy())):
                 valid_caption[int(idx)] = caption
         save_pickle(valid_caption, os.path.join(target_dir, 'valid.candidate.captions.pkl'))
+        if valid_scorer is not None:
+            corpus, dt = _score(valid_scorer, id_batches, valid_ds.len_image)
+            print(f'  valid scores ({dt:.2f}s): {_scores_line(corpus)}')
+            write_scores(corpus, target_dir, epoch, 'valid')
         model.save(path=os.path.join(model_dir, f'model_{epoch}.pt'))
         model.save_optimizer(path=os.path.join(model_dir, f'optimizer_{epoch}.pt'))
         if t_cache is not None:
@@ -112,7 +151,7 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
         print(f'[evaluation] {model_path} not found: using the current (random-init) weights')
         model.model.eval()
     ds = _dataset(False, num_images, split)
-    captions_out = [''] * ds.len_image
+    captions_out, id_batches = [''] * ds.len_image, []
     t0 = time.time()
     region_cache = region_cache and hasattr(model, 'cache_regions')
     if region_cache:        # every image once (the reference decodes it once per ground-truth caption, dataset.py:36-43)
@@ -120,7 +159,9 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
         loader = DataLoader(IndexedCaptions(ds, with_captions=False, unique_images=True), batch_size=BATCH_SIZE,
                             shuffle=False, collate_fn=_collate_idx)
         for (idxs,) in loader:
-            captions, _ = model.generate_caption_cached(cache, idxs, beam_size=beam_size)
+            ids, _ = model.generate_caption_ids_cached(cache, idxs, beam_size=beam_size)
+            id_batches.append((idxs, ids))
+            captions = model.decode_captions(ids.cpu().numpy())
             for i, idx in enumerate(idxs):
                 captions_out[int(idx)] = captions[i]
         cache.check()
@@ -128,8 +169,10 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
         # host -> device copies of batch i + 1 run on a copy stream while batch i decodes
         loader = DataLoader(ds, batch_size=BATCH_SIZE, shuffle=False, pin_memory=True)
         for features, positions, idxs in PrefetchLoader(loader, DEVICE):
-            captions, _ = model.generate_caption(object_features=features, position_features=positions,
-                                                 beam_size=beam_size)
+            ids, _ = model.generate_caption_ids(object_features=features, position_features=positions,
+                                                beam_size=beam_size)
+            id_batches.append((idxs, ids))
+            captions = model.decode_captions(ids.cpu().numpy())
             for i, idx in enumerate(idxs.tolist()):
                 captions_out[int(idx)] = captions[i]
     dt = time.time() - t0
@@ -137,7 +180,14 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
     os.makedirs(target_dir, exist_ok=True)
     save_pickle(captions_out, os.path.join(target_dir, f'{split}.candidate.captions.pkl'))
     print(f'[evaluation] {len(captions_out)} captions in {dt:.2f}s ({len(captions_out) / dt:.1f} captions/s); '
-          f'BLEU/METEOR/CIDEr scoring needs pycocoevalcap + Java and is out of scope')
+          f'METEOR needs Java and is out of scope')
+    # the references: the split's caption file, or the synthetic split generated with its captions (same seed, so the
+    # same images)
+    scorer = _scorer(ds if 'captions' in ds.data else _dataset(True, num_images, split), model.num_vocab)
+    if scorer is not None:
+        corpus, dt = _score(scorer, id_batches, ds.len_image)
+        print(f'[evaluation] scores ({dt:.2f}s): {_scores_line(corpus)}')
+        write_scores(corpus, target_dir, epoch, split)
     return captions_out
 
 

@@ -434,7 +434,8 @@ class PolicyNetwork(Transformer):
     core/config.py:14): same Encoder / Decoder / classifer parameters, but `forward` returns the teacher-forced
     LOGITS [B, T, V] (differentiable: any PyTorch loss on top back-propagates through the CUDA path), `sample`
     is the argmax "sampler" of model_RL.py:93-97 and beam search scores with LogSoftmax (model_RL.py:72,157,182).
-    The reward computation of SelfCriticNetwork (CIDEr / BLEU on CPU strings) stays in user code."""
+    The reward of SelfCriticNetwork is its injectable reward_fn (image_caption_b200.CaptionReward: CIDEr-D + BLEU-4 on
+    the GPU)."""
 
     def __init__(self, num_vocab, max_length, encode_dim_positions, encode_dim_features, device, pad_idx=0, dropout=0.2,
                  encode_mask=False, encode_input_size=512, encode_q_k_dim=512, encode_v_dim=512, encode_hidden_size=2048,

@@ -282,6 +282,35 @@ int icap_maxpool_nhwc(int dtype, const void* x, int64_t N, int64_t H, int64_t W,
                       void* y, void* stream);
 int icap_avgpool_nhwc(int dtype, const void* x, int64_t N, int64_t HW, int64_t C, float* y, void* stream);
 
+/* ---- caption metrics on token ids: BLEU-1..4, ROUGE-L, CIDEr, CIDEr-D, the scores of core/evaluations.py:12-34 (coco-
+ * caption / pyciderevalcap arithmetic, METEOR and SPICE excluded) and the self-critical reward of loss.py:160-186.
+ * A row of W <= 128 ids (int32 or int64, leading dimension ld) is read like core/utils.py::decode_captions: a <START> (1)
+ * at position 0 is skipped, <NULL> (0) dropped, the row ends at the first <END> (2), which counts as a token.  Ids must
+ * be < 32768: an n-gram (n = 1..4) is the key n << 60 | t0 << 45 | t1 << 30 | t2 << 15 | t3.
+ * icap_caption_cook: per row the distinct keys ascending (keys / counts [N, 4W], zero-filled), their number nkeys[N],
+ *   the token count lens[N] and the tokens after the cut toks [N, W].
+ * icap_caption_df: document frequencies over a cooked reference set grouped by image (rows img_off[i] .. img_off[i+1]-1
+ *   belong to image i): a key counts once per image.  table_keys / table_df (cap slots, power of two, zeroed by the
+ *   caller; 0 = empty) receive the counts by linear probing; n_unique (nullable, int64) += the number of counted
+ *   (image, key) pairs -- size the table from it (cap >= 1.5 x n_unique leaves no overflow path).  table_keys = NULL:
+ *   count only.
+ * icap_caption_ref_prep: norms [N, 4] fp64 = per-order L2 norms of count * (log(n_img) - log(max(1, df))).
+ * icap_caption_score: one candidate row per image cand_img[m] (int64; outside [0, n_img) or without refs: 0).
+ *   scores [M, 7] fp32 (nullable) = CIDEr-D, CIDEr, ROUGE-L, sentence BLEU-1..4; reward [M] (nullable) =
+ *   cider_weight * CIDEr-D + bleu_weight * BLEU-4; corpus (nullable, int64 [10]) += BLEU's correct[1..4], guess[1..4],
+ *   candidate length, closest reference length, so corpus BLEU is exact. */
+int icap_caption_cook(const void* tokens, int tok_is_int64, int64_t N, int64_t W, int64_t ld, uint64_t* keys, int* counts,
+                      int* nkeys, int* lens, int* toks, void* stream);
+int icap_caption_df(int64_t n_img, const int64_t* img_off, int64_t W, const uint64_t* keys, const int* nkeys,
+                    uint64_t* table_keys, int* table_df, int64_t cap, long long* n_unique, void* stream);
+int icap_caption_ref_prep(int64_t N, int64_t W, const uint64_t* keys, const int* counts, const int* nkeys, int64_t n_img,
+                          const uint64_t* table_keys, const int* table_df, int64_t cap, double* norms, void* stream);
+int icap_caption_score(const void* cand, int cand_is_int64, int64_t M, int64_t Wc, int64_t ldc, const int64_t* cand_img,
+                       int64_t n_img, const int64_t* img_off, int64_t W, const uint64_t* keys, const int* counts,
+                       const int* nkeys, const int* lens, const int* toks, const double* norms, const uint64_t* table_keys,
+                       const int* table_df, int64_t cap, float* scores, float* reward, float cider_weight,
+                       float bleu_weight, long long* corpus, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
