@@ -646,13 +646,24 @@ mha_decode_row_kernel(int rows, int wpr, int Lk, const T* __restrict__ q, int64_
   const int row = gw / wpr, part = gw % wpr;          // part: which 32*EPL-wide slice of the row this warp owns
   const bool live = row < rows;
   const int col = (part * 32 + lane) * EPL;           // first element of this lane within a K / V / q / o row
-  // lane l: physical cache row of position l, or -1 (position masked / beyond Lk).  The token buffer, the slot table and
-  // the cached positions 0..pos_new-1 were written by EARLIER decode steps (not by the kernel that produces q): they are
-  // read -- and the cache lines are pulled into L2 -- BEFORE the grid dependency resolves, i.e. while the QKV projection
-  // of this step is still running on the tensor cores (its HBM traffic is small, this kernel's is all there is).
-  int myrow = -1;
-  if (live && lane < Lk && tokens[(int64_t)row * tok_ld + lane] != pad_idx)
-    myrow = (slot ? slot[(int64_t)row * slot_ld + lane] : row) * kv_rows_per_seq + lane;
+  // lane l: physical cache row of position l, or -1 (position masked / beyond Lk).  The cached positions 0..pos_new-1
+  // are pulled into L2 BEFORE the grid dependency resolves, i.e. while the QKV projection of this step is still running
+  // on the tensor cores (its HBM traffic is small, this kernel's is all there is).  The token buffer and the slot table
+  // that locate them may still be in flight at that point: in beam search the kernel that starts the step
+  // (icap_decode_embed_ln) writes them, and the QKV GEMM in between lets this kernel become resident before it waits.
+  // So the pre-wait lookup only steers the prefetch (a stale row costs bandwidth, never a wrong result) and the lookup
+  // is repeated after griddepcontrol.wait for the loads that feed the result.  Both read through L2 (ld.global.cg):
+  // the early read must not leave a stale line in L1 for the second one to hit.
+  auto cache_row = [&]() {
+    int r = -1;
+    if (live && lane < Lk) {                          // both loads in flight together
+      const int tk = __ldcg(tokens + (int64_t)row * tok_ld + lane);
+      const int sl = slot ? __ldcg(slot + (int64_t)row * slot_ld + lane) : row;
+      if (tk != pad_idx) r = sl * kv_rows_per_seq + lane;
+    }
+    return r;
+  };
+  int myrow = cache_row();
   for (int j = 0; j < Lk; ++j) {
     const int r = __shfl_sync(0xffffffffu, myrow, j);
     if (r >= 0 && j != pos_new) {
@@ -662,6 +673,7 @@ mha_decode_row_kernel(int rows, int wpr, int Lk, const T* __restrict__ q, int64_
   }
   pdl_prologue();
   if (!live) return;
+  myrow = cache_row();                                // tokens / slot of this step are final now
   float qv[EPL];
   {
     RawVec<T, EPL> r;

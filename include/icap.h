@@ -35,8 +35,11 @@ extern "C" {
  * The classifier of a beam-search step (model.py:176-186): icap_beam_select takes the buffer instead of making its own
  * statistics pass over the V logits of every row. */
 #define ICAP_EPI_ROWSTATS 3
-/* flag, OR-ed into `epilogue`: B and bias are WEIGHTS that the kernel launched immediately before on this stream does
- * not write; the small-footprint kernel then fetches its first B stages before its grid dependency has resolved. */
+/* flag, OR-ed into `epilogue`: B and bias are WEIGHTS; the tcgen05 kernels then fetch their first B stages before their
+ * grid dependency has resolved.  Such a pre-wait read may overlap every kernel of the stream back to, and including, the
+ * nearest earlier kernel that waits before it lets its dependents start (every kernel of this library except the
+ * tcgen05 GEMMs of icap_gemm and icap_gemm_ln, which let them start first; a kernel launched without PDL also counts):
+ * none of those kernels may write the data read early. */
 #define ICAP_EPI_B_STATIC 16
 
 int icap_version(void);
@@ -114,8 +117,8 @@ int icap_add_ln_bwd_params(int act_dtype, int64_t M, int64_t d, const void* dy1,
  * with its own TMA -> tcgen05.mma main loop; the row statistics are exchanged through distributed shared memory.
  * sum_out (nullable) receives the pre-norm sum, mean_out / rstd_out (nullable, fp32 [M]) the statistics: exactly
  * what icap_add_ln_fwd(write_sum=1) leaves for icap_add_ln_bwd, with the same dropout decisions (seed, element).
- * W, bias, gamma, beta are model parameters: they must not be written by the kernel launched just before on this stream
- * (the kernel requests its first W stages before its grid dependency has resolved).
+ * W, bias, gamma, beta are model parameters: the kernel requests its first W stages before its grid dependency has
+ * resolved, so the pre-wait rule of ICAP_EPI_B_STATIC applies to them.
  * Returns -2 (nothing launched) for other shapes / unaligned rows: call icap_gemm + icap_add_ln_fwd instead.
  * Replaces joint_linear / position_wise_2 -> Dropout -> LayerNorm(out + residual) [-> *= non_pad_mask],
  * modules.py:86-90,117-120,154-155,203-204. */
@@ -171,8 +174,8 @@ int icap_beam_reorder(int64_t B, int64_t k, int64_t Tmax, int64_t t, const int* 
  *                    slot[row*slot_ld+j] (own row when slot == NULL); position j is masked iff
  *                    tokens[row*tok_ld+j] == pad_idx  (model.py:421-430).
  *   cross-attention (tokens == NULL): keys are the Lk regions of image row / rows_per_image, masked by kvalid;
- *                    kc / vc / kvalid must NOT be written by the kernel launched just before on this stream (they are
- *                    produced once per decode): the kernel fetches them before its grid dependency has resolved.
+ *                    kc / vc / kvalid are produced once per decode: the kernel may fetch them before its grid
+ *                    dependency has resolved, so the pre-wait rule of ICAP_EPI_B_STATIC applies to them.
  *   cache rows: k at kc + (slot*Tmax_or_Lk + j)*ldk + h*dk. */
 int icap_mha_decode(int dtype, int64_t rows, int64_t H, int64_t Lk, int64_t dk, int64_t dv, const void* q, int64_t ldq,
                     const void* kc, int64_t ldk, const void* vc, int64_t ldv, int64_t kv_rows_per_seq, void* o,
@@ -183,9 +186,9 @@ int icap_mha_decode(int dtype, int64_t rows, int64_t H, int64_t Lk, int64_t dk, 
  * v_new, leading dimension ld_new) are written to the row's own cache line (kc/vc + (row*kv_rows_per_seq + pos)*ld)
  * and attended together with the cached positions 0..pos-1 (slot table / pad-token mask as in icap_mha_decode).
  * rows_per_image (>= 1, beam width): consecutive rows that belong to one image -- a scheduling hint only (their cache
- * lines overlap through the slot table, so they are processed by one thread block).  tokens, slot and the cached
- * positions 0..pos-1 must not be written by the kernel launched just before on this stream (they come from earlier
- * decode steps): they are read / prefetched into L2 before the grid dependency has resolved.
+ * lines overlap through the slot table, so they are processed by one thread block).  tokens, slot and the cache are
+ * in ordinary stream order: before its grid dependency has resolved the kernel only prefetches the cached positions into
+ * L2 from a provisional lookup of tokens / slot, and it reads both tables again after the wait.
  * Replaces the per-step prefix recomputation of model.py:114-122,169-180 (decoder self-attention, modules.py:190-194). */
 int icap_mha_decode_self(int dtype, int64_t rows, int64_t H, int64_t pos, int64_t dk, int64_t dv, const void* q,
                          int64_t ldq, const void* k_new, const void* v_new, int64_t ld_new, void* kc, int64_t ldk, void* vc,
