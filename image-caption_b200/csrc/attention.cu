@@ -31,6 +31,7 @@ constexpr int NT = 128;
 
 struct AttnDims {
   int Lq, Lk, LkP, dk, dv, H;
+  int ldD;      // row stride of the dropout element index, attn_drop_ld(Lk) (the smem row stride is LkP)
 };
 
 template <typename T>
@@ -100,7 +101,7 @@ __device__ __forceinline__ void scores_softmax(float* P, float* Praw, const floa
       if (j >= D.Lk) p = 0.f;
       if (Praw) Praw[i * D.LkP + j] = p;
       if (p_drop > 0.f) {
-        const uint64_t e = (bh * D.Lq + i) * (uint64_t)D.LkP + j;
+        const uint64_t e = (bh * D.Lq + i) * (uint64_t)D.ldD + j;
         const uint32_t keep = dropout_keep2(seed_fold(seed), e >> 1, thresh);
         p = ((keep >> (e & 1)) & 1u) ? p * keep_scale : 0.f;
       }
@@ -975,7 +976,7 @@ extern "C" int icap_mha_fwd(int dtype, int64_t B, int64_t H, int64_t Lq, int64_t
       (uintptr_t)o % 16 == 0)
     return icap_mha_fwd_mma(B, H, Lq, Lk, q, ldq, k, ldk, v, ldv, o, ldo, kvalid, causal, p_drop, seed, seed_dev,
                             (cudaStream_t)stream);
-  AttnDims D{(int)Lq, (int)Lk, (int)((Lk + 3) & ~3), (int)dk, (int)dv, (int)H};
+  AttnDims D{(int)Lq, (int)Lk, (int)((Lk + 3) & ~3), (int)dk, (int)dv, (int)H, attn_drop_ld(Lk)};
   const size_t smem = sizeof(float) * ((size_t)D.Lq * D.dk + (size_t)D.dk * D.LkP + (size_t)D.Lk * D.dv +
                                        (size_t)D.Lq * D.LkP);
   ICAP_ARG(smem <= 227 * 1024, "icap_mha_fwd: (Lq=%d, Lk=%d, dk=%d, dv=%d) needs %zu B of shared memory", D.Lq, D.Lk,
@@ -1010,7 +1011,7 @@ extern "C" int icap_mha_bwd(int dtype, int64_t B, int64_t H, int64_t Lq, int64_t
       (uintptr_t)dk_out % 16 == 0 && (uintptr_t)dv_out % 16 == 0)
     return icap_mha_bwd_mma(B, H, Lq, Lk, q, ldq, k, ldk, v, ldv, dout, lddo, dq, lddq, dk_out, lddk, dv_out, lddv,
                             kvalid, causal, p_drop, seed, seed_dev, (cudaStream_t)stream);
-  AttnDims D{(int)Lq, (int)Lk, (int)((Lk + 3) & ~3), (int)dk, (int)dv, (int)H};
+  AttnDims D{(int)Lq, (int)Lk, (int)((Lk + 3) & ~3), (int)dk, (int)dv, (int)H, attn_drop_ld(Lk)};
   const size_t smem = sizeof(float) * ((size_t)D.Lq * D.dk + (size_t)D.Lk * D.dk + (size_t)D.dk * D.LkP +
                                        (size_t)D.dv * D.LkP + (size_t)D.Lq * D.dv + 2 * (size_t)D.Lq * D.LkP);
   ICAP_ARG(smem <= 227 * 1024, "icap_mha_bwd: (Lq=%d, Lk=%d, dk=%d, dv=%d) needs %zu B of shared memory", D.Lq, D.Lk,

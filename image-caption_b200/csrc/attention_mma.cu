@@ -140,7 +140,8 @@ __device__ __forceinline__ void softmax_tile(float (&s)[NT8][4], int m0, int lan
 }
 
 // keep-mask bits for this thread's elements: bit (nt*4 + e).  The element pair (row, columns 8*nt + 2*(lane%4) + {0,1})
-// has pair index ((bh*Lq + row) * NT8 + nt) * 4 + lane%4  -- identical in forward and backward
+// has pair index ((bh*Lq + row) * NT8 + nt) * 4 + lane%4, i.e. element (bh*Lq + row) * attn_drop_ld(Lk) + column
+// (NT8 * 8 == attn_drop_ld(Lk) by DISPATCH_NT8) -- identical in forward and backward and in the SIMT kernels
 template <int NT8>
 __device__ __forceinline__ uint64_t dropout_bits(uint64_t seed, uint32_t thresh, uint64_t bh, int Lq, int m0, int lane) {
   uint64_t bits = 0;
@@ -367,13 +368,16 @@ bool icap_mha_mma_ok(int dtype, int64_t Lq, int64_t Lk, int64_t dk, int64_t dv, 
          ldv % 8 == 0 && (uintptr_t)q % 16 == 0 && (uintptr_t)k % 16 == 0 && (uintptr_t)v % 16 == 0;
 }
 
+// NT8 * 8 = attn_drop_ld(Lk): the key tile of the kernel is the row stride of the dropout element index
 #define DISPATCH_NT8(LK, CALL)                \
   do {                                        \
-    if ((LK) <= 16) { CALL(2); }              \
-    else if ((LK) <= 32) { CALL(4); }         \
-    else if ((LK) <= 48) { CALL(6); }         \
-    else if ((LK) <= 64) { CALL(8); }         \
-    else { CALL(16); }                        \
+    switch (attn_drop_ld(LK)) {               \
+      case 16: CALL(2); break;                \
+      case 32: CALL(4); break;                \
+      case 48: CALL(6); break;                \
+      case 64: CALL(8); break;                \
+      default: CALL(16); break;               \
+    }                                         \
   } while (0)
 
 int icap_mha_fwd_mma(int64_t B, int64_t H, int64_t Lq, int64_t Lk, const void* q, int64_t ldq, const void* k,

@@ -169,6 +169,13 @@ __device__ __forceinline__ void dropout_apply8(float (&v)[8], uint32_t sf, uint3
     v[2 * i + 1] = (h >> 16) >= t16 ? v[2 * i + 1] * keep_scale : 0.f;
   }
 }
+// Row stride of the attention dropout element index: probability (b, h, i, j) of icap_mha_fwd / icap_mha_bwd is
+// element ((b*H + h)*Lq + i) * attn_drop_ld(Lk) + j for every kernel, forward and backward, so a forward on one kernel
+// and a backward on another apply the same mask.  For Lk <= 128 it is the key bucket of the mma kernels (16, 32, 48,
+// 64, 128; DISPATCH_NT8 picks the kernel from it), above that Lk rounded up to 4.
+__host__ __device__ __forceinline__ int attn_drop_ld(int64_t Lk) {
+  return Lk <= 16 ? 16 : Lk <= 32 ? 32 : Lk <= 48 ? 48 : Lk <= 64 ? 64 : Lk <= 128 ? 128 : (int)((Lk + 3) & ~3ll);
+}
 static inline uint32_t dropout_threshold(float p) {
   double t = (double)p * 4294967296.0;
   if (t < 0) t = 0;

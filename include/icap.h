@@ -75,6 +75,9 @@ int icap_debug_trace(unsigned long long* buf, int nslots);
  *   key j of batch b is masked iff (kvalid && !kvalid[b*Lk+j]) || (causal && j > i).
  *   p_drop / seed: dropout on the probabilities (fixed 0.1 in the reference, modules.py:8,24); the effective
  *   seed is seed + seed_dev[0] * golden-ratio (seed_dev nullable) so a replayed CUDA graph gets fresh masks.
+ *   Probability (b, h, i, j) is dropout element ((b*H + h)*Lq + i) * ld + j with ld = 16, 32, 48, 64 or 128 (the
+ *   smallest of these >= Lk) for Lk <= 128 and (Lk + 3) & ~3 above.  Every kernel that icap_mha_fwd and icap_mha_bwd
+ *   may choose uses this index, so the backward regenerates the forward's mask whichever kernel runs each of them.
  *   attn_mean (nullable, fp32 [B,Lq,Lk], pre-zeroed): += P / H  (greedy visualisation, model.py:123).
  * Replaces ScaledDotProductAttention.forward and the head split/merge, modules.py:16-27,72-84. */
 int icap_mha_fwd(int dtype, int64_t B, int64_t H, int64_t Lq, int64_t Lk, int64_t dk, int64_t dv, const void* q,
@@ -89,6 +92,8 @@ int icap_mha_bwd(int dtype, int64_t B, int64_t H, int64_t Lq, int64_t Lk, int64_
 /* y = (LayerNorm(dropout(a) + res[row % res_rows]) * gamma + beta) * rowscale[row]   (eps given).
  *   a: [M,d] of a_dtype (the GEMM output); res/y: act_dtype; write_sum=1 stores the pre-norm sum
  *   back into a (needed by the backward); mean/rstd: fp32 [M] (nullable in inference).
+ *   Dropout element index of a[row, col]: row*d + col (same seed rule as icap_mha_fwd); icap_add_ln_bwd(_rows)
+ *   regenerates the mask from the same seed / seed_dev.
  * Replaces Dropout + residual + LayerNorm of modules.py:86-90,117-120, the embedding norms
  * model.py:307-309,433-436 and `output *= non_pad_mask`, modules.py:154-155,203-204. */
 int icap_add_ln_fwd(int a_dtype, int act_dtype, int64_t M, int64_t d, void* a, const void* res, int64_t res_rows,
@@ -116,7 +121,8 @@ int icap_add_ln_bwd_params(int act_dtype, int64_t M, int64_t d, const void* dy1,
  * {128, 256, 512, 1024}): the N columns of a 128-row block are split over a thread-block cluster of N/128 CTAs, each
  * with its own TMA -> tcgen05.mma main loop; the row statistics are exchanged through distributed shared memory.
  * sum_out (nullable) receives the pre-norm sum, mean_out / rstd_out (nullable, fp32 [M]) the statistics: exactly
- * what icap_add_ln_fwd(write_sum=1) leaves for icap_add_ln_bwd, with the same dropout decisions (seed, element).
+ * what icap_add_ln_fwd(write_sum=1) leaves for icap_add_ln_bwd, with the same dropout decisions: the dropout element
+ * index of output (row, col) is row*N + col, as in icap_add_ln_fwd.
  * W, bias, gamma, beta are model parameters: the kernel requests its first W stages before its grid dependency has
  * resolved, so the pre-wait rule of ICAP_EPI_B_STATIC applies to them.
  * Returns -2 (nothing launched) for other shapes / unaligned rows: call icap_gemm + icap_add_ln_fwd instead.

@@ -352,37 +352,6 @@ def test_add_ln_fwd_bwd(act, M, d):
     assert rel_err(dbias2, a64.grad.sum(0)) < (5e-4 if act == F32 else 5e-2)
 
 
-def test_add_ln_dropout_consistency():
-    """Dropout: keep-rate ~ 1-p, kept values scaled by 1/(1-p), and backward regenerates the same mask."""
-    M, d, p, seed = 512, 512, 0.2, 77
-    a = torch.ones(M, d, device=dev())
-    gamma, beta = torch.ones(d, device=dev()), torch.zeros(d, device=dev())
-    y = torch.empty(M, d, device=dev())
-    mean, rstd = torch.empty(M, device=dev()), torch.empty(M, device=dev())
-    work = a.clone()
-    N.call("icap_add_ln_fwd", F32, F32, M, d, work.data_ptr(), None, 1, gamma.data_ptr(), beta.data_ptr(), None,
-           y.data_ptr(), mean.data_ptr(), rstd.data_ptr(), 1, p, seed, None, 1e-6, S())
-    kept = work != 0
-    assert abs(float(kept.float().mean()) - (1 - p)) < 5e-3
-    assert torch.allclose(work[kept], torch.full_like(work[kept], 1 / (1 - p)))
-    dy = torch.randn(M, d, device=dev())
-    ds = torch.empty(M, d, device=dev())
-    da = torch.empty(M, d, device=dev())
-    z, z2 = torch.zeros(d, device=dev()), torch.zeros(d, device=dev())
-    N.call("icap_add_ln_bwd", F32, M, d, dy.data_ptr(), None, work.data_ptr(), mean.data_ptr(), rstd.data_ptr(),
-           gamma.data_ptr(), None, ds.data_ptr(), da.data_ptr(), z.data_ptr(), z2.data_ptr(), None, p, seed, None, S())
-    torch.cuda.synchronize()
-    assert torch.equal(da != 0, kept & (ds != 0))
-    assert torch.allclose(da[kept], ds[kept] / (1 - p), rtol=1e-6, atol=1e-7)
-    # a different step counter on the device gives a different mask (CUDA-graph replays)
-    step = torch.tensor([5], dtype=torch.int32, device=dev())
-    work2 = a.clone()
-    N.call("icap_add_ln_fwd", F32, F32, M, d, work2.data_ptr(), None, 1, gamma.data_ptr(), beta.data_ptr(), None,
-           y.data_ptr(), mean.data_ptr(), rstd.data_ptr(), 1, p, seed, step.data_ptr(), 1e-6, S())
-    torch.cuda.synchronize()
-    assert not torch.equal(work2 != 0, kept)
-
-
 # ------------------------------------------------------------------------------------------ attention
 def _ref_attention(q, k, v, kvalid, causal, H):
     B, Lq, _ = q.shape
@@ -450,57 +419,6 @@ def test_mha_fwd_bwd(act, B, H, Lq, Lk, dk, dv, causal, usevalid):
     assert rel_err(dq[:, :H * dk], q64.grad.view(B * Lq, -1)) < tolb
     assert rel_err(dkv[:, :H * dk], k64.grad.view(B * Lk, -1)) < tolb
     assert rel_err(dkv[:, H * dk:], v64.grad.view(B * Lk, -1)) < tolb
-
-
-def test_mha_dropout_is_consistent_between_fwd_and_bwd():
-    """With V = identity-like probes the forward output exposes the dropped probabilities; the
-    backward must use the same mask: check dV = Pd^T dO numerically."""
-    B, H, L, dkk = 2, 2, 16, 16
-    g = torch.Generator(device="cuda").manual_seed(3)
-    q = torch.randn(B * L, H * dkk, device=dev(), generator=g)
-    k = torch.randn(B * L, H * dkk, device=dev(), generator=g)
-    v = torch.eye(L, device=dev()).repeat(B, H)[:, :H * dkk].contiguous()       # V[j, h*16 + c] = (j == c)
-    o = torch.empty(B * L, H * dkk, device=dev())
-    p, seed = 0.3, 11
-    N.call("icap_mha_fwd", F32, B, H, L, L, dkk, dkk, q.data_ptr(), H * dkk, k.data_ptr(), H * dkk, v.data_ptr(), H * dkk,
-           o.data_ptr(), H * dkk, None, 0, p, seed, None, None, S())
-    Pd = o.view(B, L, H, L).permute(0, 2, 1, 3)            # [B,H,i,j] dropped probabilities
-    frac0 = float((Pd == 0).float().mean())
-    assert abs(frac0 - p) < 0.05
-    dout = torch.randn(B * L, H * dkk, device=dev(), generator=g)
-    dq = torch.empty_like(q); dk_ = torch.empty_like(k); dv_ = torch.empty_like(v)
-    N.call("icap_mha_bwd", F32, B, H, L, L, dkk, dkk, q.data_ptr(), H * dkk, k.data_ptr(), H * dkk, v.data_ptr(), H * dkk,
-           dout.data_ptr(), H * dkk, dq.data_ptr(), H * dkk, dk_.data_ptr(), H * dkk, dv_.data_ptr(), H * dkk, None, 0, p,
-           seed, None, S())
-    torch.cuda.synchronize()
-    dO = dout.view(B, L, H, dkk).permute(0, 2, 1, 3)
-    dV_ref = (Pd.transpose(2, 3) @ dO).permute(0, 2, 1, 3).reshape(B * L, H * dkk)
-    assert rel_err(dv_, dV_ref) < 1e-5
-
-
-def test_mha_mma_dropout_is_consistent_between_fwd_and_bwd():
-    """Same probe for the tensor-core kernels (bf16, head dim 64): V = I exposes the dropped probabilities."""
-    B, H, L, dh = 2, 2, 64, 64
-    g = torch.Generator(device="cuda").manual_seed(13)
-    q = (torch.randn(B * L, H * dh, device=dev(), generator=g) * 0.5).bfloat16()
-    k = (torch.randn(B * L, H * dh, device=dev(), generator=g) * 0.5).bfloat16()
-    v = torch.eye(L, device=dev()).repeat(B, H).bfloat16().contiguous()
-    o = torch.empty(B * L, H * dh, device=dev(), dtype=torch.bfloat16)
-    p, seed = 0.25, 5
-    N.call("icap_mha_fwd", BF16, B, H, L, L, dh, dh, q.data_ptr(), H * dh, k.data_ptr(), H * dh, v.data_ptr(), H * dh,
-           o.data_ptr(), H * dh, None, 0, p, seed, None, None, S())
-    Pd = o.float().view(B, L, H, L).permute(0, 2, 1, 3)
-    assert abs(float((Pd == 0).float().mean()) - p) < 0.03
-    assert torch.allclose(Pd.sum(-1).mean(), torch.tensor(1.0, device=dev()), atol=0.05)     # E[sum] = 1
-    dout = torch.randn(B * L, H * dh, device=dev(), generator=g).bfloat16()
-    dq = torch.empty_like(q); dk_ = torch.empty_like(k); dv_ = torch.empty_like(v)
-    N.call("icap_mha_bwd", BF16, B, H, L, L, dh, dh, q.data_ptr(), H * dh, k.data_ptr(), H * dh, v.data_ptr(), H * dh,
-           dout.data_ptr(), H * dh, dq.data_ptr(), H * dh, dk_.data_ptr(), H * dh, dv_.data_ptr(), H * dh, None, 0, p,
-           seed, None, S())
-    torch.cuda.synchronize()
-    dO = dout.float().view(B, L, H, dh).permute(0, 2, 1, 3)
-    dV_ref = (Pd.transpose(2, 3) @ dO).permute(0, 2, 1, 3).reshape(B * L, H * dh)
-    assert rel_err(dv_, dV_ref) < 2e-2
 
 
 def test_mha_decode_matches_full_attention():
