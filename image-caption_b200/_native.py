@@ -34,6 +34,7 @@ SIGNATURES = {
     "icap_xent": [I, L, L, P, L, P, I, P, P, I, P],
     "icap_xent_finalize": [L, P, P, I, P, P],
     "icap_argmax": [I, L, L, P, L, P, L, P, P],
+    "icap_sample_tokens": [I, L, L, P, L, F, U, P, L, L, P, P, L, I, I, P],
     "icap_beam_select": [I, L, L, L, P, L, P, L, P, P, P, P, I, P, L, P],
     "icap_beam_reorder": [L, L, L, L, P, P, P, P, P, P, P],
     "icap_decode_embed_ln": [I, L, L, L, L, L, P, P, P, P, P, P, P, P, P, P, P, P, I, F, P],

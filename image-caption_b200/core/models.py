@@ -66,6 +66,16 @@ class MODEL_init:
         caption_vector, attention_list = self.generate_caption_ids(object_features, position_features, beam_size)
         return self.decode_captions(caption_vector.cpu().numpy()), attention_list
 
+    def sample_caption_ids(self, object_features, position_features, num_samples=1, temperature=1.0, seed=None):
+        """num_samples captions per image drawn from the model (Transformer.sample_captions): (ids [B, n, L] and their
+        log-probabilities [B, n, L - 1] on the device)."""
+        return self.model.sample_captions(object_features.to(DEVICE), position_features.to(DEVICE),
+                                          num_samples=num_samples, temperature=temperature, seed=seed)
+
+    def sample_caption_ids_cached(self, cache, image_idxs, num_samples=1, temperature=1.0, seed=None):
+        return self.model.sample_captions(cache.batch(image_idxs), None, num_samples=num_samples,
+                                          temperature=temperature, seed=seed)
+
     def decode_captions(self, caption_vector):
         return decode_captions(captions=caption_vector, index_to_word=self.idx_to_word)
 

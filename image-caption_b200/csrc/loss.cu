@@ -252,6 +252,122 @@ argmax_kernel(int V, const T* __restrict__ logits, int64_t ldl, int* __restrict_
   }
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// Sampled decoding step (icap_sample_tokens): one block per row, inverse-CDF draw from p_j ~ exp((x_j - max) / tau) and
+// the tau = 1 log-probability of the drawn token.  Thread i owns the contiguous columns [i*per, (i+1)*per) (per = a
+// multiple of 8, so its loads are 16-byte vectors), which fixes the order of the running sum: the running sum at column j
+// of chunk i is fl(P_i + L_j), P_i the block's exclusive scan of the chunk sums and L_j the chunk's own sequential sum up
+// to j.  It is non-decreasing inside a chunk and ends at fl(P_i + c_i), so the first chunk whose end exceeds u * sum
+// holds the token, and only its thread walks its columns a second time.
+__device__ __forceinline__ float sample_weight(float v, float mx, float inv_tau, bool tau_one) {
+  return tau_one ? expf(v - mx) : expf((v - mx) * inv_tau);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(NT)
+sample_kernel(int V, const T* __restrict__ logits, int64_t ldl, float inv_tau, uint64_t seed,
+              const int* __restrict__ seed_dev, int t, int Tmax, int* __restrict__ tokens, float* __restrict__ logp,
+              int64_t ldp, int end_idx, int pad_idx) {
+  pdl_prologue();                                   // the classifier GEMM writes the logits: nothing is read before
+  __shared__ float red[NT / 32];
+  __shared__ float s_wsum[NT / 32];
+  __shared__ unsigned s_flag[NT / 32];
+  __shared__ int s_last[NT / 32];
+  __shared__ int s_tok;
+  const int row = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int* tok = tokens + (int64_t)row * Tmax;
+  float* lp = logp + (int64_t)row * ldp + t;
+  if (t >= 1) {                                     // finished row (the StructureCriterion mask rule): pad, log-prob 0
+    const int prev = tok[t];
+    if (prev == end_idx || prev == pad_idx) {
+      if (threadIdx.x == 0) { tok[t + 1] = pad_idx; *lp = 0.f; }
+      return;
+    }
+  }
+  const T* x = logits + (int64_t)row * ldl;
+  const bool vec = ((uintptr_t)logits % 16 == 0) && (ldl * sizeof(T)) % 16 == 0;
+  const int per = ((V + 7) / 8 + NT - 1) / NT * 8;
+  const int jb = min(threadIdx.x * per, V), je = min(jb + per, V);
+  float mx = -INFINITY;
+  for (int j = jb; j < je; j += 8) {
+    float c[8];
+    load_chunk8(x, j, V, vec, c);                   // columns >= V read as -inf
+#pragma unroll
+    for (int i = 0; i < 8; ++i) mx = fmaxf(mx, c[i]);
+  }
+  mx = block_max(mx, red);
+  const bool tau_one = inv_tau == 1.f;
+  float csum = 0.f, s1 = 0.f;                       // chunk sum of the tempered weights; sum of exp(x - max)
+  int last = -1;                                    // last column of the chunk with a non-zero weight
+  for (int j = jb; j < je; j += 8) {
+    float c[8];
+    const int n = load_chunk8(x, j, V, vec, c);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      if (i >= n) break;
+      const float e = expf(c[i] - mx);
+      const float w = tau_one ? e : sample_weight(c[i], mx, inv_tau, false);
+      csum += w;
+      s1 += e;
+      if (w > 0.f) last = j + i;
+    }
+  }
+  // exclusive scan of the chunk sums (fixed order), the total, and the sum of exp(x - max)
+  float incl = csum;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const float y = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += y;
+  }
+  float excl = __shfl_up_sync(0xffffffffu, incl, 1);
+  if (lane == 0) excl = 0.f;
+  const int wlast = __reduce_max_sync(0xffffffffu, last + 1) - 1;
+  if (lane == 31) s_wsum[warp] = incl;
+  if (lane == 0) s_last[warp] = wlast;
+  s1 = block_sum(s1, red);                          // its barriers also publish s_wsum / s_last
+  float pre = 0.f, total = 0.f;
+  int glast = -1;
+  for (int w = 0; w < NT / 32; ++w) {
+    if (w < warp) pre += s_wsum[w];
+    total += s_wsum[w];
+    glast = max(glast, s_last[w]);
+  }
+  const float P = pre + excl;
+  // u in (0, 1) with 24 random bits; u * total is exact in double, and so is every comparison with it
+  const uint64_t es = seed + (seed_dev ? (uint64_t)(*seed_dev) * 0x9E3779B97F4A7C15ull : 0ull);
+  const uint32_t h = rand32(seed_fold(es), (uint64_t)row * Tmax + t);
+  const double target = ((double)(h >> 8) + 0.5) * 0x1p-24 * (double)total;
+  const bool flag = csum > 0.f && (double)(P + csum) > target;
+  const unsigned ball = __ballot_sync(0xffffffffu, flag);
+  if (lane == 0) s_flag[warp] = ball;
+  __syncthreads();
+  int owner = -1;
+  for (int w = 0; w < NT / 32; ++w) {
+    if (s_flag[w]) { owner = w * 32 + __ffs(s_flag[w]) - 1; break; }
+  }
+  if (owner < 0) {                                  // rounding left no column above u * sum: the last non-zero weight
+    if (threadIdx.x == 0) s_tok = glast >= 0 ? glast : 0;
+  } else if ((int)threadIdx.x == owner) {
+    float L = 0.f;
+    int pick = -1;
+    for (int j = jb; j < je && pick < 0; j += 8) {
+      float c[8];
+      const int n = load_chunk8(x, j, V, vec, c);
+      for (int i = 0; i < n; ++i) {
+        L += sample_weight(c[i], mx, inv_tau, tau_one);
+        if ((double)(P + L) > target) { pick = j + i; break; }
+      }
+    }
+    s_tok = pick >= 0 ? pick : last;                // not reached: the chunk's end exceeds the target
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const int k = s_tok;
+    tok[t + 1] = k;
+    *lp = (float)((double)to_f32(x[k]) - (double)mx - log((double)s1));
+  }
+}
+
 constexpr int CAND_CAP = 1024;   // fast-path candidate list of beam_select
 constexpr int KMAX = 8;   // beam width limit; lists hold KMAX+1 entries so the k/(k+1) gap can be reported
 
@@ -815,6 +931,25 @@ extern "C" int icap_argmax(int dtype, int64_t M, int64_t V, const void* logits, 
   if (dtype == ICAP_F32) icap_launch(argmax_kernel<float>, (unsigned)M, NT, 0, st, (int)V, (const float*)logits, ldl, out, out_stride, gap);
   else icap_launch(argmax_kernel<bf16>, (unsigned)M, NT, 0, st, (int)V, (const bf16*)logits, ldl, out, out_stride, gap);
   ICAP_LAUNCH_CHECK("icap_argmax");
+  return 0;
+}
+
+extern "C" int icap_sample_tokens(int dtype, int64_t M, int64_t V, const void* logits, int64_t ldl, float inv_temperature,
+                                  uint64_t seed, const int* seed_dev, int64_t t, int64_t Tmax, int* tokens, float* logp,
+                                  int64_t ldp, int end_idx, int pad_idx, void* stream) {
+  ICAP_ARG(M > 0 && V > 0 && logits && tokens && logp, "icap_sample_tokens: null/empty argument");
+  ICAP_ARG(isfinite(inv_temperature) && inv_temperature > 0.f,
+           "icap_sample_tokens: the temperature must be finite and > 0 (inverse %g)", (double)inv_temperature);
+  ICAP_ARG(ldl >= V && V < (1 << 30) && M < (1ll << 31), "icap_sample_tokens: bad logits shape");
+  ICAP_ARG(t >= 0 && t + 1 < Tmax && ldp > t, "icap_sample_tokens: position %lld out of range", (long long)t);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == ICAP_F32)
+    icap_launch(sample_kernel<float>, (unsigned)M, NT, 0, st, (int)V, (const float*)logits, ldl, inv_temperature, seed,
+                seed_dev, (int)t, (int)Tmax, tokens, logp, ldp, end_idx, pad_idx);
+  else
+    icap_launch(sample_kernel<bf16>, (unsigned)M, NT, 0, st, (int)V, (const bf16*)logits, ldl, inv_temperature, seed,
+                seed_dev, (int)t, (int)Tmax, tokens, logp, ldp, end_idx, pad_idx);
+  ICAP_LAUNCH_CHECK("icap_sample_tokens");
   return 0;
 }
 

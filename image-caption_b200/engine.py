@@ -66,6 +66,7 @@ class ModelConfig:
 
 ATTN_DROPOUT = 0.1      # ScaledDotProductAttention default, never overridden (modules.py:8,55-56)
 LN_EPS = 1e-6
+END_IDX = 2             # <END> of the vocabulary (preprocess.py:303); sampled rows stop there
 
 
 def param_layout(cfg: ModelConfig) -> "Dict[str, Tuple[int, ...]]":
@@ -197,6 +198,9 @@ class CaptionEngine:
         self.adam_m: Optional[torch.Tensor] = None
         self.adam_v: Optional[torch.Tensor] = None
         self.step_dev = torch.zeros(1, dtype=torch.int32, device=self.dev)
+        # sampled decoding: its own counter (neither the dropout masks nor Adam's step see it) and base seed
+        self.sample_dev = torch.zeros(1, dtype=torch.int32, device=self.dev)
+        self.sample_seed = 0x243F6A8885A308D3
         self.pos_table32 = pos_table.reshape(-1, pos_table.shape[-1]).contiguous()
         self.pos_table_act = self.pos_table32.to(self.tdt)
         self.base_seed = 0x1234ABCD
@@ -950,7 +954,8 @@ class CaptionEngine:
 
     # ------------------------------------------------------------------ KV-cached decoding
     def decode(self, feats: torch.Tensor, pos: torch.Tensor, beam_size: int = 1, log_domain: bool = False,
-               want_attention: bool = False, want_gaps: bool = False):
+               want_attention: bool = False, want_gaps: bool = False, num_samples: int = 0, temperature: float = 1.0,
+               sample_counter: Optional[torch.Tensor] = None):
         """Greedy (beam_size=1: Transformer.generate_caption_vector, model.py:101-132) or beam search
         (Transformer.beam_search, model.py:135-200) with a KV cache: the reference re-runs the decoder on
         the whole prefix every step (and once per beam); here every step computes ONE position for all
@@ -959,14 +964,27 @@ class CaptionEngine:
         scores (log-domain for the PolicyNetwork variant), no EOS handling, pad-token (id 0) masking of
         generated tokens, result = beam slot 0.
 
+        num_samples = n > 0: sampled decoding instead (icap_sample_tokens): B*n independent rows, n per image, each
+        token drawn from softmax(logits / temperature); a row that has emitted <END> or <NULL> continues with <NULL>
+        and log-probability 0.  The uniforms are keyed by the int32 device counter `sample_counter` (the engine's
+        sample_dev by default), which the decode advances by one at its end.
+
         Returns dict(ids int32 [B, T+1] (col 0 = <START>), attention fp32 [T, B, R] | None,
-                     gaps fp32 [T, B] | None)  -- all device tensors, no host sync."""
+                     gaps fp32 [T, B] | None)  -- all device tensors, no host sync.
+        Sampling: dict(ids int32 [B, n, T+1], logp fp32 [B, n, T] (log_softmax of the token at temperature 1))."""
         cfg = self.cfg
         assert self.tape is None
         self.training = False
         self.refresh_shadow()
         self._site = 0
-        k = int(beam_size)
+        sampling = num_samples > 0
+        if sampling:
+            assert not (want_attention or want_gaps), "sampled decoding returns ids and log-probabilities only"
+            assert math.isfinite(temperature) and temperature > 0, "the temperature must be finite and > 0"
+            if sample_counter is None:
+                sample_counter = self.sample_dev
+        k = int(num_samples) if sampling else int(beam_size)        # rows per image
+        beam = not sampling and k > 1
         B, R, _ = feats.shape
         T, d, V, E = cfg.T, cfg.decode_input_size, cfg.num_vocab, cfg.dim_word_embedding
         H, dk_tot, dv_tot, hid = cfg.decode_num_heads, cfg.decode_q_k_dim, cfg.decode_v_dim, cfg.decode_hidden_size
@@ -991,7 +1009,7 @@ class CaptionEngine:
         tok = [torch.zeros(rows, Tmax, dtype=torch.int32, device=self.dev) for _ in range(2)]
         tok[0][:, 0] = 1                                  # <START> (model.py:111,144)
         slot = None
-        if k > 1:
+        if beam:
             slot = [torch.zeros(rows, Tmax, dtype=torch.int32, device=self.dev) for _ in range(2)]
             slot[0][:, 0] = torch.arange(rows, dtype=torch.int32, device=self.dev)
             score = [torch.zeros(B, k, dtype=torch.float32, device=self.dev) for _ in range(2)]
@@ -1000,6 +1018,7 @@ class CaptionEngine:
         caches = [self.new(rows, T, nkv) for _ in range(cfg.decode_num_blocks)]
         attn = torch.zeros(T, rows, R, dtype=torch.float32, device=self.dev) if want_attention else None
         gaps = torch.zeros(T, B, dtype=torch.float32, device=self.dev) if want_gaps else None
+        logp = torch.zeros(rows, T, dtype=torch.float32, device=self.dev) if sampling else None
         ldl = (V + 7) // 8 * 8
         cur = 0
         fused_start = d % 8 == 0 and d <= 1024 and os.environ.get("ICAP_DECODE_FUSED_START", "1") != "0"
@@ -1073,14 +1092,19 @@ class CaptionEngine:
             # beam search in bf16: the classifier's epilogue leaves per-128-column (max, 2nd max, sum exp) statistics,
             # so that beam_select does not make its own statistics pass over the k * V logits of every image
             stats = None
-            if k > 1 and self.precision == "bf16":
+            if beam and self.precision == "bf16":
                 stats = self.new(rows, 8 * ((V + 255) // 256), dtype=torch.float32)
             self.gemm(x, True, self.w("classifer.weight"), d, True, rows, V, d, logits, ldc=ldl,
                       bias=self.p("classifer.bias"), b_static=True, epi=N.EPI_ROWSTATS if stats is not None else 0,
                       aux=stats)
-            if k == 1:
-                call("icap_argmax", self.act, rows, V, logits.data_ptr(), ldl, tk.data_ptr() + 4 * (t + 1), Tmax,
-                     gaps[t].data_ptr() if gaps is not None else None, s())
+            if not beam:
+                if sampling:
+                    call("icap_sample_tokens", self.act, rows, V, logits.data_ptr(), ldl, 1.0 / temperature,
+                         self.sample_seed, sample_counter.data_ptr(), t, Tmax, tk.data_ptr(), logp.data_ptr(), T,
+                         END_IDX, cfg.pad_idx, s())
+                else:
+                    call("icap_argmax", self.act, rows, V, logits.data_ptr(), ldl, tk.data_ptr() + 4 * (t + 1), Tmax,
+                         gaps[t].data_ptr() if gaps is not None else None, s())
                 if t + 1 < T:
                     x, rowscale = step_input(t + 1, tk)
             else:
@@ -1095,6 +1119,9 @@ class CaptionEngine:
                     call("icap_beam_reorder", B, k, Tmax, t, parent.data_ptr(), newtok.data_ptr(), tk.data_ptr(),
                          tok[cur ^ 1].data_ptr(), slot[cur].data_ptr(), slot[cur ^ 1].data_ptr(), s())
                 cur ^= 1
+        if sampling:
+            call("icap_step_tick", sample_counter.data_ptr(), s())        # the next decode draws fresh uniforms
+            return {"ids": tok[cur].view(B, k, Tmax), "logp": logp.view(B, k, T)}
         ids = tok[cur].view(B, k, Tmax)[:, 0, :]
         if attn is not None:
             attn = attn.view(T, B, k, R)[:, :, 0, :]

@@ -191,9 +191,11 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
     return captions_out
 
 
-def demo(image_path=None, beam_size=None, epoch=90, save_img=False, max_obj=False, features_path=None):
+def demo(image_path=None, beam_size=None, epoch=90, save_img=False, max_obj=False, features_path=None, num_samples=None,
+         temperature=1.0, seed=None):
     """The reference runs YOLOv5 + ResNet-101 on `image_path` first (main.py:195-197); offline, pass
-    `--features-path file.pt` holding {'features': [R,2048], 'positions': [R,84]} or omit it for a synthetic image."""
+    `--features-path file.pt` holding {'features': [R,2048], 'positions': [R,84]} or omit it for a synthetic image.
+    `--num-samples N [--temperature T] [--seed S]` prints N captions sampled from the model instead."""
     model = _model()
     start = time.time()
     if features_path:
@@ -207,6 +209,14 @@ def demo(image_path=None, beam_size=None, epoch=90, save_img=False, max_obj=Fals
         model.load(path=model_path)
     else:
         model.model.eval()
+    if num_samples is not None:
+        ids, logp = model.sample_caption_ids(feature, position, num_samples=int(num_samples),
+                                             temperature=float(temperature), seed=seed)
+        captions = model.decode_captions(ids[0].cpu().numpy())
+        for caption, lp in zip(captions, logp[0].sum(dim=1).tolist()):
+            print(f'Sampled Caption: {caption}  (log-probability {lp:.3f})')
+        print('Spending Time:', time.time() - start)
+        return captions
     caption, attention_list = model.generate_caption(object_features=feature, position_features=position,
                                                      beam_size=beam_size)
     print('Generated Caption:', caption[0])

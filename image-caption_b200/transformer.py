@@ -331,24 +331,30 @@ class Transformer(nn.Module):
         B, T = c.shape[0], c.shape[1] - 1
         return lg[:, :self.num_vocab].float().view(B, T, self.num_vocab)
 
-    def _decode(self, f, p, beam_size: int, log_domain: bool, want_attention: bool):
+    def _decode(self, f, p, beam_size: int, log_domain: bool, want_attention: bool, num_samples: int = 0,
+                temperature: float = 1.0, seed: Optional[int] = None):
         """KV-cached decode of one batch; the whole fixed-trip-count loop (encoder + max_length-1 steps, ~2000
-        launches) is ONE CUDA graph per (batch, regions, beam) shape unless ICAP_DECODE_GRAPH=0."""
+        launches) is ONE CUDA graph per (batch, regions, beam) shape -- per (batch, regions, samples, temperature) when
+        sampling -- unless ICAP_DECODE_GRAPH=0.  seed (sampling): the value of the sampling counter for this call."""
         eng = self._engine()
         eng.shadow_fresh = False                       # an external optimizer may have stepped the fp32 weights
+        sample_kw = dict(num_samples=int(num_samples), temperature=float(temperature)) if num_samples else {}
         if os.environ.get("ICAP_DECODE_GRAPH", "1") == "0":
+            if seed is not None:
+                eng.sample_dev.fill_(seed)
             return eng.decode(f, p, beam_size=beam_size, log_domain=log_domain, want_attention=want_attention,
-                              want_gaps=True)
+                              want_gaps=not num_samples, **sample_kw)
         cache = f.cache if isinstance(f, RegionBatch) else None
-        key = (f.shape[0], f.shape[1], int(beam_size), bool(log_domain), bool(want_attention), id(eng), id(cache))
+        key = (f.shape[0], f.shape[1], int(beam_size), bool(log_domain), bool(want_attention), id(eng), id(cache),
+               int(num_samples), float(temperature))
         gd = self._decode_graphs.get(key)
         if gd is None:
             if len(self._decode_graphs) >= 4:          # each graph owns its KV-cache pool: keep only a few shapes
                 self._decode_graphs.pop(next(iter(self._decode_graphs)))
             gd = GraphedDecode(self, f.shape[0], f.shape[1], beam_size, log_domain=log_domain,
-                               want_attention=want_attention, want_gaps=True, cache=cache)
+                               want_attention=want_attention, want_gaps=not num_samples, cache=cache, **sample_kw)
             self._decode_graphs[key] = gd
-        return gd.run(f.idx) if cache is not None else gd.run(f, p)
+        return gd.run(f.idx, seed=seed) if cache is not None else gd.run(f, p, seed=seed)
 
     def generate_caption_vector(self, object_features, position_features):
         """model.py:101-132 -> (LongTensor [B, max_length+1], list of max_length-1 float32 arrays [B, R])."""
@@ -372,6 +378,30 @@ class Transformer(nn.Module):
             out = self._decode(f, p, int(beam_size), self.log_domain_beam, False)
             self.last_gaps = out["gaps"]
             return out["ids"].long().contiguous()
+
+    def sample_captions(self, object_features, position_features, num_samples=1, temperature=1.0, seed=None):
+        """num_samples captions per image drawn from the model: every token from softmax(logits / temperature) by the
+        KV-cached decoder (icap_sample_tokens).  A caption ends at its first <END> (or <NULL>); the positions after it
+        hold <NULL> with log-probability 0.  Inputs are tensors or a RegionBatch (position_features=None), as for
+        beam_search.  seed (0 <= seed < 2**31) makes the call reproducible; without it every call advances the model's
+        sampling counter and draws new captions.
+        -> (ids LongTensor [B, num_samples, max_length] with <START> first,
+            logp FloatTensor [B, num_samples, max_length - 1]: log_softmax(logits)[token] at temperature 1, the model's
+            log-probability of each token, as a policy gradient needs it)."""
+        n = int(num_samples)
+        if not 1 <= n <= 16:
+            raise ValueError(f"num_samples must be in [1, 16], got {num_samples}")
+        temperature = float(temperature)
+        if not (math.isfinite(temperature) and temperature > 0 and 1.0 / temperature < 3e38):   # 1 / tau is a float32
+            raise ValueError(f"temperature must be finite and > 0, got {temperature}")
+        if seed is not None and not 0 <= int(seed) < 2 ** 31:
+            raise ValueError(f"seed must be in [0, 2**31), got {seed}")
+        with torch.no_grad():
+            eng = self._engine()
+            f, p, _ = eng.prepare_inputs(object_features, position_features)
+            out = self._decode(f, p, 1, False, False, num_samples=n, temperature=temperature,
+                               seed=None if seed is None else int(seed))
+            return out["ids"].long(), out["logp"].clone()
 
     def get_attention_key_pad_mask(self, k, q):
         """model.py:202-209 (host-visible helper kept for API parity; kernels build the mask in-register)."""
@@ -706,17 +736,21 @@ class DataParallel:
 
 
 class GraphedDecode:
-    """The complete KV-cached greedy / beam decode of a fixed (batch, regions, beam) shape as ONE CUDA graph:
+    """The complete KV-cached greedy / beam / sampled decode of a fixed (batch, regions, beam) shape as ONE CUDA graph:
     encoder, cross-K/V projection, and all max_length-1 steps (the reference's loops have a fixed trip count and
     no EOS exit, model.py:114,169).  Replays cost one launch instead of ~2000 ctypes calls."""
 
     def __init__(self, model: Transformer, batch: int, regions: int, beam_size: int, log_domain: bool = False,
-                 want_attention: bool = False, want_gaps: bool = False, cache=None):
+                 want_attention: bool = False, want_gaps: bool = False, cache=None, num_samples: int = 0,
+                 temperature: float = 1.0):
         eng = model._engine()
         cfg = model.cfg
         self.eng = eng
         self.kw = dict(beam_size=int(beam_size), log_domain=log_domain, want_attention=want_attention,
                        want_gaps=want_gaps)
+        self.sampling = num_samples > 0                # the graph ticks the sampling counter: replays draw new samples
+        if self.sampling:
+            self.kw.update(num_samples=int(num_samples), temperature=float(temperature))
         self.cache = cache
         if cache is not None:                          # inputs = image numbers into a device-resident RegionCache
             assert regions == cache.regions
@@ -733,11 +767,14 @@ class GraphedDecode:
     def capture(self) -> None:
         eng = self.eng
         with torch.no_grad():
+            counter0 = eng.sample_dev.clone() if self.sampling else None
             side = eng.warm_stream()
             side.wait_stream(torch.cuda.current_stream(eng.dev))
             with torch.cuda.stream(side):
                 eng.decode(self.feats, self.pos, **self.kw)            # warm-up: function attributes, allocator
             torch.cuda.current_stream(eng.dev).wait_stream(side)
+            if counter0 is not None:
+                eng.sample_dev.copy_(counter0)                         # the warm-up does not count as a draw
             torch.cuda.synchronize(eng.dev)
             eng.refresh_shadow()
             self.graph = torch.cuda.CUDAGraph()
@@ -746,6 +783,8 @@ class GraphedDecode:
             # no gain -- the per-step kernels do not overlap usefully -- so the default is one stream.
             B = self.feats.shape[0]
             nsplit = max(1, min(int(os.environ.get("ICAP_DECODE_STREAMS", "1")), B // 64 if B >= 128 else 1))
+            if self.sampling:
+                nsplit = 1                             # the uniforms are keyed by the row number within the whole batch
             while B % nsplit:
                 nsplit -= 1
             with _graph_capture(self.graph):
@@ -770,9 +809,9 @@ class GraphedDecode:
                         "gaps": torch.cat([o["gaps"] for o in outs], dim=1) if outs[0]["gaps"] is not None else None,
                     }
 
-    def run(self, feats: torch.Tensor, pos: Optional[torch.Tensor] = None):
+    def run(self, feats: torch.Tensor, pos: Optional[torch.Tensor] = None, seed: Optional[int] = None):
         """Returns the engine's output dict (static device tensors, overwritten by the next run).  With a region
-        cache `feats` is the vector of image numbers."""
+        cache `feats` is the vector of image numbers.  seed (sampling): set the sampling counter first."""
         if self.graph is None:
             self.capture()
         if self.cache is not None:
@@ -780,6 +819,8 @@ class GraphedDecode:
         else:
             self.feats.copy_(feats, non_blocking=True)
             self.pos.copy_(pos, non_blocking=True)
+        if seed is not None:
+            self.eng.sample_dev.fill_(seed)
         self.eng.refresh_shadow()                      # weights may have been stepped since the capture
         self.graph.replay()
         return self.out

@@ -144,6 +144,20 @@ int icap_xent_finalize(int64_t M, const float* row_loss, const float* inv_count,
  * Replaces argmax(Softmax(classifer(.))), model.py:125-128. */
 int icap_argmax(int dtype, int64_t M, int64_t V, const void* logits, int64_t ldl, int* out, int64_t out_stride,
                 float* gap, void* stream);
+/* Sampled decoding step for M rows (row r = image * n + sample; tokens / logp rows of stride Tmax / ldp):
+ *   finished row: t >= 1 and tokens[r, t] is end_idx or pad_idx  ->  tokens[r, t+1] = pad_idx, logp[r, t] = 0
+ *                 (the mask rule of StructureCriterion, loss.py);
+ *   otherwise     tokens[r, t+1] = the smallest j whose running sum of w_j = exp((x_j - max x) / tau), over the row's V
+ *                 logits x as stored (bf16 or fp32), in column order, exceeds u * sum_j w_j (none after rounding: the last
+ *                 j with w_j > 0), with the uniform
+ *                   u = ((rand32(seed_fold(seed + seed_dev[0] * golden), r * Tmax + t) >> 8) + 0.5) * 2^-24
+ *                 (icap_common.cuh; seed_dev nullable = 0);
+ *                 logp[r, t] = log_softmax(x)[token] at tau = 1 (fp32): the model's log-probability of the token.
+ * inv_temperature = 1 / tau must be finite and > 0.  The kernel reads nothing before its grid dependency has resolved.
+ * Same seed, seed_dev[0] and logits -> bitwise-identical tokens and logp. */
+int icap_sample_tokens(int dtype, int64_t M, int64_t V, const void* logits, int64_t ldl, float inv_temperature,
+                       uint64_t seed, const int* seed_dev, int64_t t, int64_t Tmax, int* tokens, float* logp, int64_t ldp,
+                       int end_idx, int pad_idx, void* stream);
 /* Beam step for B images: candidates (beam r, token j) score softmax(logits[b*kin+r])[j] + prev[b,r]
  * (log_domain=1: log-softmax, the PolicyNetwork variant); writes the kout best in DESCENDING order:
  * score, parent = r, token = j; gap[b] = score_k - score_{k+1} (nullable).
