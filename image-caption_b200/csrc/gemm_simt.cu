@@ -79,7 +79,9 @@ gemm_f32_kernel(int M, int N, int K, const float* __restrict__ A, int64_t lda, c
   __shared__ __align__(16) float As[2][BK][BM + PAD];
   __shared__ __align__(16) float Bs[2][BK][BN + PAD];
   const int tid = threadIdx.x, tx = tid % 16, ty = tid / 16;
-  const int m0 = blockIdx.y * BM, n0 = blockIdx.x * BN;
+  // tiles in one grid dimension, N fastest: grid.y (at most 65535) would cap M at 8,388,480 rows
+  const int tiles_n = (N + BN - 1) / BN;
+  const int m0 = (int)(blockIdx.x / tiles_n) * BM, n0 = (int)(blockIdx.x % tiles_n) * BN;
   const int kbeg = blockIdx.z * kchunk, kend = min(K, kbeg + kchunk);
   float acc[8][8];
 #pragma unroll
@@ -158,7 +160,9 @@ int icap_gemm_f32_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64
   }
   int vecA = ((uintptr_t)A % 16 == 0) && (lda % 4 == 0);
   int vecB = ((uintptr_t)B % 16 == 0) && (ldb % 4 == 0);
-  dim3 grid((unsigned)ceil_div64(N, BN), (unsigned)ceil_div64(M, BM), (unsigned)split_k);
+  const int64_t tiles = ceil_div64(M, BM) * ceil_div64(N, BN);
+  ICAP_ARG(tiles < (1ll << 31), "icap_gemm(fp32): %lld output tiles exceed the grid", (long long)tiles);
+  dim3 grid((unsigned)tiles, 1u, (unsigned)split_k);
 #define LAUNCH(AK, BKM)                                                                                            \
   icap_launch(gemm_f32_kernel<AK, BKM>, grid, NT, 0, st, (int)M, (int)N, (int)K, A, lda, B, ldb, C, ldc, bias, epi, aux, \
                                                 ldaux, accumulate, kchunk, vecA, vecB)

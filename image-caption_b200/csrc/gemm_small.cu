@@ -225,7 +225,8 @@ bool icap_gemm_small_eligible(int a_kmajor, int b_kmajor, int64_t M, int64_t N, 
   const int mode = e_mode.geti("ICAP_GEMM_SMALL", 1);     // 0 never, 1 automatic, 2 every eligible shape
   if (!mode) return false;
   if (!(a_kmajor && b_kmajor) || c_dtype != ICAP_BF16 || (epi & 15) > 1 || accumulate || split_k > 1) return false;
-  if (((uintptr_t)C & 15) || (ldc % 8)) return false;
+  if (((uintptr_t)C & 15) || (ldc % 8) || (N % 8)) return false;   // TMA stores: see icap_gemm_bf16_launch
+  if (ceil_div64(M, BM) > 65535) return false;              // M tiles go on grid.y
   const int64_t tiles = ceil_div64(M, BM) * ceil_div64(N, BN);
   return tiles <= (int64_t)icap_num_sms() * 3 || mode == 2;
 }

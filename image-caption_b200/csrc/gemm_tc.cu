@@ -462,11 +462,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           } else if (full) {
 #pragma unroll
             for (int j = 0; j < 32; j += 8) {
-              if (g.accumulate == 1) {
+              if (g.accumulate == 1) {      // C + round(v), as the TMA reduce-add of the staged path computes it
                 float o[8];
                 OutVec<TO>::load8(crow + j, o);
 #pragma unroll
-                for (int t = 0; t < 8; ++t) v[j + t] += o[t];
+                for (int t = 0; t < 8; ++t) v[j + t] = to_f32(from_f32<TO>(v[j + t])) + o[t];
               }
               OutVec<TO>::store8(crow + j, v + j);
             }
@@ -474,7 +474,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             for (int j = 0; j < 32; ++j) {
               if (col0 + j < N) {
                 float o = v[j];
-                if (g.accumulate == 1) o += to_f32(crow[j]);
+                if (g.accumulate == 1) o = to_f32(from_f32<TO>(o)) + to_f32(crow[j]);
                 crow[j] = from_f32<TO>(o);
               }
             }
@@ -648,15 +648,16 @@ int icap_gemm_bf16_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int6
   const char* force_bn = e_bn.get("ICAP_GEMM_BN");                     // "128" | "256" | "pair"
   const bool no_pair = e_nopair.get("ICAP_GEMM_NO_PAIR") != nullptr;
   const bool direct_epi = e_direct.get("ICAP_GEMM_DIRECT_EPILOGUE") != nullptr;
+  const bool pair_ok = sms >= 2;               // a CTA pair occupies two SMs: a one-SM grid runs 128x128 tiles instead
   for (int c = 2; c >= 0; --c) {
     if (force_bn && epi != 3) {
-      const int want = force_bn[0] == 'p' ? 2 : (atoi(force_bn) == 256 ? 1 : 0);
+      const int want = force_bn[0] == 'p' ? (pair_ok ? 2 : 0) : (atoi(force_bn) == 256 ? 1 : 0);
       if (want != c) continue;
     }
     const int bn = c == 0 ? 128 : 256, bm = c == 2 ? 256 : 128;
     if (epi == 3 && c != 1) continue;          // row statistics: one partial per 128 columns = per column half of a 128x256 tile
-    if (c >= 1 && N <= 128 && !force_bn) continue;
-    if (c == 2 && !force_bn && (M <= 128 || no_pair)) continue;
+    if (c >= 1 && N <= 128 && !force_bn && epi != 3) continue;
+    if (c == 2 && (!pair_ok || (!force_bn && (M <= 128 || no_pair)))) continue;
     const int64_t tiles = ceil_div64(M, bm) * ceil_div64(N, bn);
     const int workers = c == 2 ? sms / 2 : sms;
     int split = split_k;
@@ -707,8 +708,10 @@ int icap_gemm_bf16_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int6
   if (rc) return rc;
   const int esz = c_dtype == ICAP_F32 ? 4 : 2;
   int vec_ok = ((uintptr_t)C % 16 == 0) && ((ldc * esz) % 16 == 0);
-  // staged TMA epilogue whenever C satisfies the TMA alignment rules; accumulation = TMA reduce-add
-  int store_mode = vec_ok ? (accumulate ? 2 : 1) : 0;
+  // staged TMA epilogue whenever C satisfies the TMA alignment rules and its rows end on a 16-byte boundary (a TMA
+  // store / reduce-add of a row ending inside a 16-byte chunk also writes the rest of that chunk, past N: observed on
+  // B200); accumulation = TMA reduce-add
+  int store_mode = vec_ok && (N * esz) % 16 == 0 ? (accumulate ? 2 : 1) : 0;
   if (direct_epi) store_mode = 0;
   if (epi == 2) vec_ok = vec_ok && ((uintptr_t)aux % 16 == 0) && ((ldaux * esz) % 16 == 0);
   CUtensorMap tc = ta;

@@ -55,6 +55,11 @@ int icap_set_pdl(int on);
  *   ab_dtype ICAP_BF16: TMA + tcgen05.mma + TMEM kernel, C fp32 or bf16 (c_dtype).
  *   accumulate=1: C += ...; split_k>1 (needs accumulate=1, fp32 C, no bias) reduces K-slices with red.add;
  *   split_k<=0 (bf16): the kernel picks the split that fills the SMs (1 unless accumulate=1 and C is fp32).
+ *   bf16 C with accumulate=1: C = bf16(C + bf16(v)), v = the fp32 result of the epilogue; the TMA reduce-add and the
+ *   direct stores (C not 16-byte aligned, or rows of ldc or N elements not whole 16-byte chunks) both round v first, so
+ *   the bits of C do not depend on its alignment.  fp32 C: C + v, rounded once.
+ *   Nothing outside the [M, N] block of C is written, whatever ldc (C's rows leave through TMA stores only when N
+ *   elements fill whole 16-byte chunks).  ICAP_EPI_ROWSTATS takes any N.  The fp32 kernel takes any M < 2^31.
  * Replaces every nn.Linear / torch.matmul weight contraction of the path and their autograd
  * backward: modules.py:42-44,59-60,72-77,86,100-101,113-116; model.py:68,93,235,246,295-306,392-394,433. */
 int icap_gemm(int ab_dtype, int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64_t K, const void* A, int64_t lda,
@@ -66,7 +71,8 @@ int icap_gemm(int ab_dtype, int a_kmajor, int b_kmajor, int64_t M, int64_t N, in
  * buf = NULL: off). */
 int icap_reload_env(void);
 /* Width of the persistent grid of the following icap_gemm(bf16) launches (0 = all SMs): data parallel training leaves a
- * few SMs to the NCCL all-reduce kernels that overlap the backward. */
+ * few SMs to the NCCL all-reduce kernels that overlap the backward.  A 256x256 CTA pair needs two SMs: with n = 1 (or
+ * ICAP_GEMM_SMS=1) every GEMM runs on 128-row tiles, even when ICAP_GEMM_BN=pair asks for the pair. */
 int icap_set_gemm_sms(int n);
 int icap_debug_trace(unsigned long long* buf, int nslots);
 
