@@ -12,19 +12,6 @@
 #include <stdlib.h>
 #include "icap_common.cuh"
 
-// tensor-core (mma.sync) variants for bf16 / head dim 64, attention_mma.cu
-extern "C" int icap_copy2d(const void* src, int src_dtype, int64_t src_ld, void* dst, int dst_dtype, int64_t dst_ld,
-                           int64_t rows, int64_t cols, int accumulate, void* stream);
-bool icap_mha_mma_ok(int dtype, int64_t Lq, int64_t Lk, int64_t dk, int64_t dv, int64_t ldq, int64_t ldk, int64_t ldv,
-                     const void* q, const void* k, const void* v);
-int icap_mha_fwd_mma(int64_t B, int64_t H, int64_t Lq, int64_t Lk, const void* q, int64_t ldq, const void* k,
-                     int64_t ldk, const void* v, int64_t ldv, void* o, int64_t ldo, const uint8_t* kvalid, int causal,
-                     float p_drop, uint64_t seed, const int* seed_dev, cudaStream_t st, int kv_static = 0);
-int icap_mha_bwd_mma(int64_t B, int64_t H, int64_t Lq, int64_t Lk, const void* q, int64_t ldq, const void* k,
-                     int64_t ldk, const void* v, int64_t ldv, const void* dout, int64_t lddo, void* dq, int64_t lddq,
-                     void* dk_out, int64_t lddk, void* dv_out, int64_t lddv, const uint8_t* kvalid, int causal,
-                     float p_drop, uint64_t seed, const int* seed_dev, cudaStream_t st);
-
 namespace {
 
 constexpr int NT = 128;
@@ -260,15 +247,6 @@ mha_bwd_kernel(const T* __restrict__ q, int64_t ldq, const T* __restrict__ k, in
       store4(dk_ + ((int64_t)b * D.Lk + j) * lddk + h * D.dk + c0, acc);
     }
   }
-}
-
-template <typename K>
-int ensure_smem(K kern, size_t smem, size_t* cur) {
-  if (smem > *cur) {   // one process drives one GPU, so a process-wide high-water mark is enough
-    ICAP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    *cur = smem;
-  }
-  return 0;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -936,10 +914,9 @@ int launch_cross_img(int64_t images, int64_t H, int64_t Lk, const void* q, int64
   int chunk_rows = XI_SMEM_MAX / row_bytes;
   if (chunk_rows > Lk) chunk_rows = (int)Lk;
   const size_t smem = (size_t)chunk_rows * row_bytes;
-  static size_t cur = 48 * 1024;
-  if (int rc = ensure_smem(mha_cross_img_kernel<G>, smem, &cur)) return rc;
-  icap_launch(mha_cross_img_kernel<G>, (unsigned)images, (unsigned)(32 * H), smem, st, (int)H, (int)Lk, (const bf16*)q, ldq,
-              (const bf16*)kv, ldkv, (int)dk_tot, (bf16*)o, ldo, kvalid, chunk_rows);
+  if (int rc = ensure_smem<mha_cross_img_kernel<G>>(smem)) return rc;
+  icap_launch(mha_cross_img_kernel<G>, (unsigned)images, (unsigned)(32 * H), smem, st, H, Lk, q, ldq, kv, ldkv, dk_tot, o, ldo,
+              kvalid, chunk_rows);
   ICAP_LAUNCH_CHECK("icap_mha_decode(cross, image per CTA)");
   return 0;
 }
@@ -951,9 +928,8 @@ int launch_decode64(int64_t groups, int64_t H, int64_t Lk, const void* q, int64_
                     float* attn_mean, cudaStream_t st, const void* knew = nullptr, const void* vnew = nullptr,
                     int64_t ldn = 0, int pos_new = 0) {
   const unsigned grid = (unsigned)ceil_div64(groups * H, DEC_WARPS);
-  icap_launch(mha_decode64_kernel<T, G>, grid, DEC_WARPS * 32, 0, st, 
-      (int)groups, (int)H, (int)Lk, (const T*)q, ldq, (const T*)kc, ldk, (const T*)vc, ldv, (int)kv_rows_per_seq, (T*)o,
-      ldo, slot, slot_ld, tokens, tok_ld, pad_idx, kvalid, attn_mean, (const T*)knew, (const T*)vnew, ldn, pos_new);
+  icap_launch(mha_decode64_kernel<T, G>, grid, DEC_WARPS * 32, 0, st, groups, H, Lk, q, ldq, kc, ldk, vc, ldv, kv_rows_per_seq,
+              o, ldo, slot, slot_ld, tokens, tok_ld, pad_idx, kvalid, attn_mean, knew, vnew, ldn, pos_new);
   ICAP_LAUNCH_CHECK("icap_mha_decode(64)");
   return 0;
 }
@@ -983,19 +959,13 @@ extern "C" int icap_mha_fwd(int dtype, int64_t B, int64_t H, int64_t Lq, int64_t
            D.dk, D.dv, smem);
   cudaStream_t st = (cudaStream_t)stream;
   const uint32_t th = dropout_threshold(p_drop);
-  if (dtype == ICAP_F32) {
-    static size_t cur = 48 * 1024;
-    if (int rc = ensure_smem(mha_fwd_kernel<float>, smem, &cur)) return rc;
-    icap_launch(mha_fwd_kernel<float>, (unsigned)(B * H), NT, smem, st, (const float*)q, ldq, (const float*)k, ldk,
-                                                               (const float*)v, ldv, (float*)o, ldo, kvalid, D, causal,
-                                                               p_drop, th, seed, seed_dev, attn_mean);
-  } else {
-    static size_t cur = 48 * 1024;
-    if (int rc = ensure_smem(mha_fwd_kernel<bf16>, smem, &cur)) return rc;
-    icap_launch(mha_fwd_kernel<bf16>, (unsigned)(B * H), NT, smem, st, (const bf16*)q, ldq, (const bf16*)k, ldk, (const bf16*)v,
-                                                              ldv, (bf16*)o, ldo, kvalid, D, causal, p_drop, th, seed,
-                                                              seed_dev, attn_mean);
-  }
+  const int rc = dispatch_act(dtype, [&](auto tag) {
+    if (int rc = ensure_smem<mha_fwd_kernel<decltype(tag)>>(smem)) return rc;
+    icap_launch(mha_fwd_kernel<decltype(tag)>, (unsigned)(B * H), NT, smem, st, q, ldq, k, ldk, v, ldv, o, ldo, kvalid, D, causal,
+                p_drop, th, seed, seed_dev, attn_mean);
+    return 0;
+  });
+  if (rc) return rc;
   ICAP_LAUNCH_CHECK("icap_mha_fwd");
   return 0;
 }
@@ -1018,19 +988,13 @@ extern "C" int icap_mha_bwd(int dtype, int64_t B, int64_t H, int64_t Lq, int64_t
            D.dk, D.dv, smem);
   cudaStream_t st = (cudaStream_t)stream;
   const uint32_t th = dropout_threshold(p_drop);
-  if (dtype == ICAP_F32) {
-    static size_t cur = 48 * 1024;
-    if (int rc = ensure_smem(mha_bwd_kernel<float>, smem, &cur)) return rc;
-    icap_launch(mha_bwd_kernel<float>, (unsigned)(B * H), NT, smem, st, 
-        (const float*)q, ldq, (const float*)k, ldk, (const float*)v, ldv, (const float*)dout, lddo, (float*)dq, lddq,
-        (float*)dk_out, lddk, (float*)dv_out, lddv, kvalid, D, causal, p_drop, th, seed, seed_dev);
-  } else {
-    static size_t cur = 48 * 1024;
-    if (int rc = ensure_smem(mha_bwd_kernel<bf16>, smem, &cur)) return rc;
-    icap_launch(mha_bwd_kernel<bf16>, (unsigned)(B * H), NT, smem, st, 
-        (const bf16*)q, ldq, (const bf16*)k, ldk, (const bf16*)v, ldv, (const bf16*)dout, lddo, (bf16*)dq, lddq,
-        (bf16*)dk_out, lddk, (bf16*)dv_out, lddv, kvalid, D, causal, p_drop, th, seed, seed_dev);
-  }
+  const int rc = dispatch_act(dtype, [&](auto tag) {
+    if (int rc = ensure_smem<mha_bwd_kernel<decltype(tag)>>(smem)) return rc;
+    icap_launch(mha_bwd_kernel<decltype(tag)>, (unsigned)(B * H), NT, smem, st, q, ldq, k, ldk, v, ldv, dout, lddo, dq, lddq,
+                dk_out, lddk, dv_out, lddv, kvalid, D, causal, p_drop, th, seed, seed_dev);
+    return 0;
+  });
+  if (rc) return rc;
   ICAP_LAUNCH_CHECK("icap_mha_bwd");
   return 0;
 }
@@ -1056,16 +1020,15 @@ extern "C" int icap_mha_decode(int dtype, int64_t rows, int64_t H, int64_t Lk, i
       (const bf16*)vc == (const bf16*)kc + H * dk && ldk * 2 <= XI_SMEM_MAX && (ldk * 2) % 16 == 0 &&
       (rows_per_image <= 5 || rows_per_image == 8) && env_flag<7>("ICAP_DECODE_IMG_CROSS")) {
     const int64_t images = rows / rows_per_image;
-#define XIMG(GG) return launch_cross_img<GG>(images, H, Lk, q, ldq, kc, ldk, H * dk, o, ldo, kvalid, st)
+    auto go = [&](auto g) { return launch_cross_img<g>(images, H, Lk, q, ldq, kc, ldk, H * dk, o, ldo, kvalid, st); };
     switch (rows_per_image) {
-      case 1: XIMG(1);
-      case 2: XIMG(2);
-      case 3: XIMG(3);
-      case 4: XIMG(4);
-      case 5: XIMG(5);
-      default: XIMG(8);
+      case 1: return go(int_c<1>{});
+      case 2: return go(int_c<2>{});
+      case 3: return go(int_c<3>{});
+      case 4: return go(int_c<4>{});
+      case 5: return go(int_c<5>{});
+      default: return go(int_c<8>{});
     }
-#undef XIMG
   }
   // cross-attention of a beam group = a tiny full attention (Lq = beams, Lk = regions, shared K/V): tensor-core
   // kernel (mma.sync), ~5x fewer instructions than the SIMT path for 5 beams x 36 regions x 64 dims
@@ -1081,36 +1044,29 @@ extern "C" int icap_mha_decode(int dtype, int64_t rows, int64_t H, int64_t Lk, i
     const int64_t groups = rows / G;
     // odd beam sizes (6, 7, > 8) in cross mode fall through to the generic kernel below
     if (tokens != nullptr || G == rows_per_image) {
-#define DEC(T, GG)                                                                                                   \
-  return launch_decode64<T, GG>(groups, H, Lk, q, ldq, kc, ldk, vc, ldv, kv_rows_per_seq, o, ldo, slot, slot_ld,      \
-                                tokens, tok_ld, pad_idx, kvalid, attn_mean, st)
-#define DECT(T)                                                                                                      \
-  switch (G) {                                                                                                       \
-    case 1: DEC(T, 1);                                                                                               \
-    case 2: DEC(T, 2);                                                                                               \
-    case 3: DEC(T, 3);                                                                                               \
-    case 4: DEC(T, 4);                                                                                               \
-    case 5: DEC(T, 5);                                                                                               \
-    case 8: DEC(T, 8);                                                                                               \
-    default: break;                                                                                                  \
-  }
-      if (dtype == ICAP_F32) { DECT(float) } else { DECT(bf16) }
-#undef DECT
-#undef DEC
+      auto go = [&](auto g) {
+        return dispatch_act(dtype, [&](auto tag) {
+          return launch_decode64<decltype(tag), g>(groups, H, Lk, q, ldq, kc, ldk, vc, ldv, kv_rows_per_seq, o, ldo, slot,
+                                                   slot_ld, tokens, tok_ld, pad_idx, kvalid, attn_mean, st);
+        });
+      };
+      switch (G) {
+        case 1: return go(int_c<1>{});
+        case 2: return go(int_c<2>{});
+        case 3: return go(int_c<3>{});
+        case 4: return go(int_c<4>{});
+        case 5: return go(int_c<5>{});
+        case 8: return go(int_c<8>{});
+        default: break;
+      }
     }
   }
   const size_t smem = (NT / 32) * dk * sizeof(float);
   const unsigned grid = (unsigned)ceil_div64(rows * H, NT / 32);
-  if (dtype == ICAP_F32)
-    icap_launch(mha_decode_kernel<float>, grid, NT, smem, st, (int)rows, (int)H, (int)Lk, (int)dk, (int)dv, (const float*)q, ldq,
-                                                     (const float*)kc, ldk, (const float*)vc, ldv,
-                                                     (int)kv_rows_per_seq, (float*)o, ldo, slot, slot_ld, tokens,
-                                                     tok_ld, pad_idx, kvalid, (int)rows_per_image, attn_mean);
-  else
-    icap_launch(mha_decode_kernel<bf16>, grid, NT, smem, st, (int)rows, (int)H, (int)Lk, (int)dk, (int)dv, (const bf16*)q, ldq,
-                                                    (const bf16*)kc, ldk, (const bf16*)vc, ldv, (int)kv_rows_per_seq,
-                                                    (bf16*)o, ldo, slot, slot_ld, tokens, tok_ld, pad_idx, kvalid,
-                                                    (int)rows_per_image, attn_mean);
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(mha_decode_kernel<decltype(tag)>, grid, NT, smem, st, rows, H, Lk, dk, dv, q, ldq, kc, ldk, vc, ldv,
+                kv_rows_per_seq, o, ldo, slot, slot_ld, tokens, tok_ld, pad_idx, kvalid, rows_per_image, attn_mean);
+  });
   ICAP_LAUNCH_CHECK("icap_mha_decode");
   return 0;
 }
@@ -1147,22 +1103,22 @@ extern "C" int icap_mha_decode_self(int dtype, int64_t rows, int64_t H, int64_t 
       wpb = (int)rows_per_image * wpr;
     const unsigned grid = (unsigned)ceil_div64(rows * wpr, wpb);
     const unsigned nthr = (unsigned)(32 * wpb);
-#define ROWK(T, U)                                                                                                   \
-  icap_launch(mha_decode_row_kernel<T, 8, U>, grid, nthr, 0, st, (int)rows, wpr, (int)(pos + 1), (const T*)q, ldq,   \
-              (T*)kc, ldk, (T*)vc, ldv, (int)kv_rows_per_seq, (T*)o, ldo, slot, slot_ld, tokens, tok_ld, pad_idx,    \
-              (const T*)k_new, (const T*)v_new, ld_new, (int)pos)
-    if (dtype == ICAP_F32) { if (ub_env == 8) ROWK(float, 8); else ROWK(float, 4); }
-    else { if (ub_env == 8) ROWK(bf16, 8); else ROWK(bf16, 4); }
-#undef ROWK
+    dispatch_act(dtype, [&](auto tag) {
+      auto go = [&](auto ub) {
+        icap_launch(mha_decode_row_kernel<decltype(tag), 8, ub>, grid, nthr, 0, st, rows, wpr, pos + 1, q, ldq, kc, ldk, vc, ldv,
+                    kv_rows_per_seq, o, ldo, slot, slot_ld, tokens, tok_ld, pad_idx, k_new, v_new, ld_new, pos);
+      };
+      if (ub_env == 8) go(int_c<8>{}); else go(int_c<4>{});
+    });
     ICAP_LAUNCH_CHECK("icap_mha_decode_self(row)");
     return 0;
   }
   if (dk == 64 && dv == 64 && al && !env_flag<1>("ICAP_DECODE_SLOW")) {
-    if (dtype == ICAP_F32)
-      return launch_decode64<float, 1>(rows, H, pos + 1, q, ldq, kc, ldk, vc, ldv, kv_rows_per_seq, o, ldo, slot, slot_ld,
-                                       tokens, tok_ld, pad_idx, nullptr, nullptr, st, k_new, v_new, ld_new, (int)pos);
-    return launch_decode64<bf16, 1>(rows, H, pos + 1, q, ldq, kc, ldk, vc, ldv, kv_rows_per_seq, o, ldo, slot, slot_ld,
-                                    tokens, tok_ld, pad_idx, nullptr, nullptr, st, k_new, v_new, ld_new, (int)pos);
+    return dispatch_act(dtype, [&](auto tag) {
+      return launch_decode64<decltype(tag), 1>(rows, H, pos + 1, q, ldq, kc, ldk, vc, ldv, kv_rows_per_seq, o, ldo, slot,
+                                               slot_ld, tokens, tok_ld, pad_idx, nullptr, nullptr, st, k_new, v_new, ld_new,
+                                               (int)pos);
+    });
   }
   // generic path: strided copies into the cache, then the plain decode attention
   if (int rc = icap_copy2d(k_new, dtype, ld_new, (char*)kc + pos * ldk * esz, dtype, kv_rows_per_seq * ldk, rows, H * dk, 0, stream))

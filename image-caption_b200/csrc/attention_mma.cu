@@ -350,13 +350,16 @@ mha_bwd_mma_kernel(const bf16* __restrict__ q, int64_t ldq, const bf16* __restri
   }
 }
 
-template <typename K>
-int ensure_smem(K kern, size_t smem, size_t* cur) {
-  if (smem > *cur) {
-    ICAP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    *cur = smem;
+// NT8 * 8 = attn_drop_ld(Lk): the key tile of the kernel is the row stride of the dropout element index
+template <typename F>
+int by_nt8(int64_t Lk, F&& go) {
+  switch (attn_drop_ld(Lk)) {
+    case 16: return go(int_c<2>{});
+    case 32: return go(int_c<4>{});
+    case 48: return go(int_c<6>{});
+    case 64: return go(int_c<8>{});
+    default: return go(int_c<16>{});
   }
-  return 0;
 }
 
 }  // namespace
@@ -368,35 +371,20 @@ bool icap_mha_mma_ok(int dtype, int64_t Lq, int64_t Lk, int64_t dk, int64_t dv, 
          ldv % 8 == 0 && (uintptr_t)q % 16 == 0 && (uintptr_t)k % 16 == 0 && (uintptr_t)v % 16 == 0;
 }
 
-// NT8 * 8 = attn_drop_ld(Lk): the key tile of the kernel is the row stride of the dropout element index
-#define DISPATCH_NT8(LK, CALL)                \
-  do {                                        \
-    switch (attn_drop_ld(LK)) {               \
-      case 16: CALL(2); break;                \
-      case 32: CALL(4); break;                \
-      case 48: CALL(6); break;                \
-      case 64: CALL(8); break;                \
-      default: CALL(16); break;               \
-    }                                         \
-  } while (0)
-
 int icap_mha_fwd_mma(int64_t B, int64_t H, int64_t Lq, int64_t Lk, const void* q, int64_t ldq, const void* k,
                      int64_t ldk, const void* v, int64_t ldv, void* o, int64_t ldo, const uint8_t* kvalid, int causal,
                      float p_drop, uint64_t seed, const int* seed_dev, cudaStream_t st, int kv_static) {
   const int LqP = (int)((Lq + 15) & ~15);
   const int nthreads = 32 * (LqP / 16);
   const uint32_t th = dropout_threshold(p_drop);
-#define CALL(NT)                                                                                                   \
-  {                                                                                                                \
-    static size_t cur = 48 * 1024;                                                                                 \
-    const size_t smem = (size_t)(LqP + 2 * NT * 8) * ROWB;                                                         \
-    if (int rc = ensure_smem(mha_fwd_mma_kernel<NT>, smem, &cur)) return rc;                                       \
-    icap_launch(mha_fwd_mma_kernel<NT>, (unsigned)(B * H), nthreads, smem, st,                                              \
-        (const bf16*)q, ldq, (const bf16*)k, ldk, (const bf16*)v, ldv, (bf16*)o, ldo, kvalid, (int)H, (int)Lq,     \
-        (int)Lk, causal, p_drop, th, seed, seed_dev, kv_static);                                                   \
-  }
-  DISPATCH_NT8(Lk, CALL);
-#undef CALL
+  const int rc = by_nt8(Lk, [&](auto nt) {
+    const size_t smem = (size_t)(LqP + 2 * nt * 8) * ROWB;
+    if (int rc = ensure_smem<mha_fwd_mma_kernel<nt>>(smem)) return rc;
+    icap_launch(mha_fwd_mma_kernel<nt>, (unsigned)(B * H), nthreads, smem, st, q, ldq, k, ldk, v, ldv, o, ldo, kvalid, H, Lq,
+                Lk, causal, p_drop, th, seed, seed_dev, kv_static);
+    return 0;
+  });
+  if (rc) return rc;
   ICAP_LAUNCH_CHECK("icap_mha_fwd(mma)");
   return 0;
 }
@@ -408,18 +396,14 @@ int icap_mha_bwd_mma(int64_t B, int64_t H, int64_t Lq, int64_t Lk, const void* q
   const int LqP = (int)((Lq + 15) & ~15);
   const int nthreads = 32 * (LqP / 16);
   const uint32_t th = dropout_threshold(p_drop);
-#define CALL(NT)                                                                                                   \
-  {                                                                                                                \
-    static size_t cur = 48 * 1024;                                                                                 \
-    const size_t smem = (size_t)(2 * LqP + 2 * NT * 8) * ROWB + 2 * (size_t)LqP * (NT * 16 + 16);                  \
-    if (int rc = ensure_smem(mha_bwd_mma_kernel<NT>, smem, &cur)) return rc;                                       \
-    icap_launch(mha_bwd_mma_kernel<NT>, (unsigned)(B * H), nthreads, smem, st,                                              \
-        (const bf16*)q, ldq, (const bf16*)k, ldk, (const bf16*)v, ldv, (const bf16*)dout, lddo, (bf16*)dq, lddq,   \
-        (bf16*)dk_out, lddk, (bf16*)dv_out, lddv, kvalid, (int)H, (int)Lq, (int)Lk, causal, p_drop, th, seed,      \
-        seed_dev);                                                                                                 \
-  }
-  DISPATCH_NT8(Lk, CALL);
-#undef CALL
+  const int rc = by_nt8(Lk, [&](auto nt) {
+    const size_t smem = (size_t)(2 * LqP + 2 * nt * 8) * ROWB + 2 * (size_t)LqP * (nt * 16 + 16);
+    if (int rc = ensure_smem<mha_bwd_mma_kernel<nt>>(smem)) return rc;
+    icap_launch(mha_bwd_mma_kernel<nt>, (unsigned)(B * H), nthreads, smem, st, q, ldq, k, ldk, v, ldv, dout, lddo, dq, lddq,
+                dk_out, lddk, dv_out, lddv, kvalid, H, Lq, Lk, causal, p_drop, th, seed, seed_dev);
+    return 0;
+  });
+  if (rc) return rc;
   ICAP_LAUNCH_CHECK("icap_mha_bwd(mma)");
   return 0;
 }

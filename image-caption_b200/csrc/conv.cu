@@ -225,8 +225,6 @@ bool al16(const void* p) { return ((uintptr_t)p & 15) == 0; }
 
 }  // namespace
 
-#define BY_DTYPE(dt, CALL_F, CALL_H) do { if ((dt) == ICAP_F32) { CALL_F; } else { CALL_H; } } while (0)
-
 extern "C" int icap_im2col_nhwc(int dtype, const void* x, int64_t N, int64_t H, int64_t W, int64_t C, int kh, int kw,
                                 int stride, int pad, void* out, int64_t ldo, void* stream) {
   ICAP_ARG(x && out && N > 0 && H > 0 && W > 0 && C > 0 && kh > 0 && kw > 0 && stride > 0 && pad >= 0, "icap_im2col_nhwc: bad argument");
@@ -235,11 +233,10 @@ extern "C" int icap_im2col_nhwc(int dtype, const void* x, int64_t N, int64_t H, 
   const int vec = (C % 8 == 0 && ldo % 8 == 0 && al16(x) && al16(out)) ? 1 : 0;
   const int64_t work = N * Ho * Wo * (vec ? ldo / 8 : ldo);
   cudaStream_t st = (cudaStream_t)stream;
-  BY_DTYPE(dtype,
-           icap_launch(im2col_kernel<float>, grid_for(work), NT, 0, st, (const float*)x, (int)N, (int)H, (int)W, (int)C, kh, kw,
-                       stride, pad, (int)Ho, (int)Wo, (float*)out, ldo, vec),
-           icap_launch(im2col_kernel<bf16>, grid_for(work), NT, 0, st, (const bf16*)x, (int)N, (int)H, (int)W, (int)C, kh, kw,
-                       stride, pad, (int)Ho, (int)Wo, (bf16*)out, ldo, vec));
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(im2col_kernel<decltype(tag)>, grid_for(work), NT, 0, st, x, N, H, W, C, kh, kw, stride, pad, Ho, Wo, out, ldo,
+                vec);
+  });
   ICAP_LAUNCH_CHECK("icap_im2col_nhwc");
   return 0;
 }
@@ -254,9 +251,9 @@ extern "C" int icap_bn_scale_shift(int dtype, const void* x, int64_t M, int64_t 
     ICAP_ARG(C / 8 <= NT && NT % (C / 8) == 0, "icap_bn_scale_shift: C / 8 must divide %d", NT);
     const int rows_per_block = 256;
     const unsigned grid = (unsigned)ceil_div64(M, rows_per_block);
-    BY_DTYPE(dtype,
-             icap_launch(bn_stats_kernel<float>, grid, NT, 0, st, (const float*)x, M, (int)C, C, sums, rows_per_block),
-             icap_launch(bn_stats_kernel<bf16>, grid, NT, 0, st, (const bf16*)x, M, (int)C, C, sums, rows_per_block));
+    dispatch_act(dtype, [&](auto tag) {
+      icap_launch(bn_stats_kernel<decltype(tag)>, grid, NT, 0, st, x, M, C, C, sums, rows_per_block);
+    });
     ICAP_LAUNCH_CHECK("icap_bn_scale_shift(stats)");
   }
   icap_launch(bn_finalize_kernel, (unsigned)ceil_div64(C, 128), 128, 0, st, (int)C, sums, M, gamma, beta, running_mean,
@@ -270,11 +267,9 @@ extern "C" int icap_bn_act(int dtype, const void* x, int64_t M, int64_t C, const
   ICAP_ARG(x && y && scale && shift && M > 0 && C > 0 && C % 8 == 0 && al16(x) && al16(y) && al16(residual),
            "icap_bn_act: C must be a multiple of 8 and the tensors 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
-  BY_DTYPE(dtype,
-           icap_launch(bn_act_kernel<float>, grid_for(M * C / 8), NT, 0, st, (const float*)x, M, (int)C, scale, shift,
-                       (const float*)residual, relu, (float*)y),
-           icap_launch(bn_act_kernel<bf16>, grid_for(M * C / 8), NT, 0, st, (const bf16*)x, M, (int)C, scale, shift,
-                       (const bf16*)residual, relu, (bf16*)y));
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(bn_act_kernel<decltype(tag)>, grid_for(M * C / 8), NT, 0, st, x, M, C, scale, shift, residual, relu, y);
+  });
   ICAP_LAUNCH_CHECK("icap_bn_act");
   return 0;
 }
@@ -284,11 +279,10 @@ extern "C" int icap_maxpool_nhwc(int dtype, const void* x, int64_t N, int64_t H,
   ICAP_ARG(x && y && N > 0 && C % 8 == 0 && al16(x) && al16(y), "icap_maxpool_nhwc: C must be a multiple of 8");
   const int64_t Ho = (H + 2 * pad - k) / stride + 1, Wo = (W + 2 * pad - k) / stride + 1;
   cudaStream_t st = (cudaStream_t)stream;
-  BY_DTYPE(dtype,
-           icap_launch(maxpool_kernel<float>, grid_for(N * Ho * Wo * C / 8), NT, 0, st, (const float*)x, (int)N, (int)H, (int)W,
-                       (int)C, k, stride, pad, (int)Ho, (int)Wo, (float*)y),
-           icap_launch(maxpool_kernel<bf16>, grid_for(N * Ho * Wo * C / 8), NT, 0, st, (const bf16*)x, (int)N, (int)H, (int)W,
-                       (int)C, k, stride, pad, (int)Ho, (int)Wo, (bf16*)y));
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(maxpool_kernel<decltype(tag)>, grid_for(N * Ho * Wo * C / 8), NT, 0, st, x, N, H, W, C, k, stride, pad, Ho, Wo,
+                y);
+  });
   ICAP_LAUNCH_CHECK("icap_maxpool_nhwc");
   return 0;
 }
@@ -297,9 +291,7 @@ extern "C" int icap_avgpool_nhwc(int dtype, const void* x, int64_t N, int64_t HW
   ICAP_ARG(x && y && N > 0 && HW > 0 && C % 8 == 0 && al16(x), "icap_avgpool_nhwc: C must be a multiple of 8");
   cudaStream_t st = (cudaStream_t)stream;
   const dim3 grid((unsigned)ceil_div64(C / 8, NT), (unsigned)N);
-  BY_DTYPE(dtype,
-           icap_launch(avgpool_kernel<float>, grid, NT, 0, st, (const float*)x, (int)HW, (int)C, y),
-           icap_launch(avgpool_kernel<bf16>, grid, NT, 0, st, (const bf16*)x, (int)HW, (int)C, y));
+  dispatch_act(dtype, [&](auto tag) { icap_launch(avgpool_kernel<decltype(tag)>, grid, NT, 0, st, x, HW, C, y); });
   ICAP_LAUNCH_CHECK("icap_avgpool_nhwc");
   return 0;
 }

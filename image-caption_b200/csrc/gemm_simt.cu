@@ -163,14 +163,14 @@ int icap_gemm_f32_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64
   const int64_t tiles = ceil_div64(M, BM) * ceil_div64(N, BN);
   ICAP_ARG(tiles < (1ll << 31), "icap_gemm(fp32): %lld output tiles exceed the grid", (long long)tiles);
   dim3 grid((unsigned)tiles, 1u, (unsigned)split_k);
-#define LAUNCH(AK, BKM)                                                                                            \
-  icap_launch(gemm_f32_kernel<AK, BKM>, grid, NT, 0, st, (int)M, (int)N, (int)K, A, lda, B, ldb, C, ldc, bias, epi, aux, \
-                                                ldaux, accumulate, kchunk, vecA, vecB)
-  if (a_kmajor && b_kmajor) LAUNCH(true, true);
-  else if (a_kmajor && !b_kmajor) LAUNCH(true, false);
-  else if (!a_kmajor && !b_kmajor) LAUNCH(false, false);
-  else LAUNCH(false, true);
-#undef LAUNCH
+  auto go = [&](auto ak, auto bkm) {
+    icap_launch(gemm_f32_kernel<ak, bkm>, grid, NT, 0, st, M, N, K, A, lda, B, ldb, C, ldc, bias, epi, aux, ldaux, accumulate,
+                kchunk, vecA, vecB);
+  };
+  if (a_kmajor && b_kmajor) go(std::true_type{}, std::true_type{});
+  else if (a_kmajor && !b_kmajor) go(std::true_type{}, std::false_type{});
+  else if (!a_kmajor && !b_kmajor) go(std::false_type{}, std::false_type{});
+  else go(std::false_type{}, std::true_type{});
   ICAP_LAUNCH_CHECK("icap_gemm(fp32)");
   return 0;
 }

@@ -620,12 +620,6 @@ int icap_num_sms() { return num_sms(); }
 // a few SMs to the NCCL all-reduce kernels that run beside it (a 226 KB-smem GEMM CTA cannot share its SM with them).
 extern "C" int icap_set_gemm_sms(int n) { g_sms_limit = n; return 0; }
 
-unsigned long long* icap_trace_slot();
-bool icap_gemm_small_eligible(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64_t K, int c_dtype, int epi,
-                              int accumulate, int split_k, const void* C, int64_t ldc);
-int icap_gemm_small_launch(int64_t M, int64_t N, int64_t K, const void* A, int64_t lda, const void* B, int64_t ldb, void* C,
-                           int64_t ldc, const float* bias, int relu, int b_static, cudaStream_t st);
-
 int icap_gemm_bf16_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64_t K, const void* A, int64_t lda,
                           const void* B, int64_t ldb, void* C, int64_t ldc, int c_dtype, const float* bias, int epi,
                           const void* aux, int64_t ldaux, int accumulate, int split_k, cudaStream_t st) {
@@ -725,14 +719,15 @@ int icap_gemm_bf16_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int6
   g.debug = e_dbg.geti("ICAP_GEMM_DEBUG", 0);
   g.b_static = b_static;
   g.trace = icap_trace_slot();
-#define GO2(BNV, TW, AK, BKM)                                                                          \
-  (c_dtype == ICAP_F32 ? launch<BNV, TW, AK, BKM, float>(ta, tb, tc, g, st)                              \
-                       : launch<BNV, TW, AK, BKM, bf16>(ta, tb, tc, g, st))
-#define GO(AK, BKM) (two ? GO2(256, true, AK, BKM) : BN == 256 ? GO2(256, false, AK, BKM) : GO2(128, false, AK, BKM))
   if (epi == 3) return launch<256, false, true, true, bf16, true>(ta, tb, tc, g, st);   // the one row-statistics build
-  if (a_kmajor && b_kmajor) return GO(true, true);
-  if (a_kmajor && !b_kmajor) return GO(true, false);
-  return GO(false, false);
-#undef GO
-#undef GO2
+  auto go = [&](auto ak, auto bkm) {
+    auto by_c = [&](auto bn, auto tw) {
+      return dispatch_act(c_dtype, [&](auto tag) { return launch<bn, tw, ak, bkm, decltype(tag)>(ta, tb, tc, g, st); });
+    };
+    return two ? by_c(int_c<256>{}, std::true_type{})
+               : BN == 256 ? by_c(int_c<256>{}, std::false_type{}) : by_c(int_c<128>{}, std::false_type{});
+  };
+  if (a_kmajor && b_kmajor) return go(std::true_type{}, std::true_type{});
+  if (a_kmajor && !b_kmajor) return go(std::true_type{}, std::false_type{});
+  return go(std::false_type{}, std::false_type{});
 }

@@ -5,6 +5,8 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
+#include <type_traits>
+#include "icap_internal.h"
 
 #define ICAP_F32 0
 #define ICAP_BF16 1
@@ -58,6 +60,17 @@ static inline cudaError_t icap_launch(void (*kern)(KArgs...), dim3 grid, dim3 bl
   cfg.numAttrs = icap_g_pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
+// Opts kernel K in to `smem` bytes of dynamic shared memory when it needs more than it was last given (48 KB needs no
+// opt-in).  One process drives one GPU, so a process-wide high-water mark per kernel is enough.
+template <auto K>
+static inline int ensure_smem(size_t smem) {
+  static size_t cur = 48 * 1024;
+  if (smem > cur) {
+    ICAP_CUDA(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cur = smem;
+  }
+  return 0;
+}
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
@@ -92,6 +105,17 @@ __device__ __forceinline__ float to_f32(bf16 x) { return __bfloat162float(x); }
 template <typename T> __device__ __forceinline__ T from_f32(float x);
 template <> __device__ __forceinline__ float from_f32<float>(float x) { return x; }
 template <> __device__ __forceinline__ bf16 from_f32<bf16>(float x) { return __float2bfloat16_rn(x); }
+
+// ---- host dispatch: a runtime dtype or size becomes a compile-time type or constant, so that each launch is written
+// once inside a generic lambda.  dispatch_act calls f(float{}) for ICAP_F32 and f(bf16{}) otherwise; the lambda takes
+// the element type as decltype(tag).  A size chain calls its lambda with int_c<N>{}, which converts to N in a template
+// argument.  icap_launch converts every argument to the kernel's parameter type, so the arguments need no casts.
+template <typename F>
+static inline decltype(auto) dispatch_act(int dtype, F&& f) {
+  if (dtype == ICAP_F32) return f(float{});
+  return f(bf16{});
+}
+template <int N> using int_c = std::integral_constant<int, N>;
 
 // 4-wide vector load/store with conversion to/from fp32 (pointer must be 4-element aligned)
 __device__ __forceinline__ void load4(const float* p, float (&v)[4]) {
@@ -172,7 +196,7 @@ __device__ __forceinline__ void dropout_apply8(float (&v)[8], uint32_t sf, uint3
 // Row stride of the attention dropout element index: probability (b, h, i, j) of icap_mha_fwd / icap_mha_bwd is
 // element ((b*H + h)*Lq + i) * attn_drop_ld(Lk) + j for every kernel, forward and backward, so a forward on one kernel
 // and a backward on another apply the same mask.  For Lk <= 128 it is the key bucket of the mma kernels (16, 32, 48,
-// 64, 128; DISPATCH_NT8 picks the kernel from it), above that Lk rounded up to 4.
+// 64, 128; by_nt8 in attention_mma.cu picks the kernel from it), above that Lk rounded up to 4.
 __host__ __device__ __forceinline__ int attn_drop_ld(int64_t Lk) {
   return Lk <= 16 ? 16 : Lk <= 32 ? 32 : Lk <= 48 ? 48 : Lk <= 64 ? 64 : Lk <= 128 ? 128 : (int)((Lk + 3) & ~3ll);
 }

@@ -896,22 +896,13 @@ extern "C" int icap_xent(int dtype, int64_t M, int64_t V, void* logits, int64_t 
     ICAP_LAUNCH_CHECK("icap_xent");
     return 0;
   }
-  static size_t cur_f = 48 * 1024, cur_b = 48 * 1024;
-  if (dtype == ICAP_F32) {
-    if (smem > cur_f) {
-      ICAP_CUDA(cudaFuncSetAttribute(xent_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      cur_f = smem;
-    }
-    icap_launch(xent_kernel<float>, (unsigned)M, NT, smem, st, (int)V, (float*)logits, ldl, targets, ignore_index, inv_count,
-                                                      row_loss, write_grad, cached, vec);
-  } else {
-    if (smem > cur_b) {
-      ICAP_CUDA(cudaFuncSetAttribute(xent_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      cur_b = smem;
-    }
-    icap_launch(xent_kernel<bf16>, (unsigned)M, NT, smem, st, (int)V, (bf16*)logits, ldl, targets, ignore_index, inv_count,
-                                                     row_loss, write_grad, cached, vec);
-  }
+  const int rc = dispatch_act(dtype, [&](auto tag) {
+    if (int rc = ensure_smem<xent_kernel<decltype(tag)>>(smem)) return rc;
+    icap_launch(xent_kernel<decltype(tag)>, (unsigned)M, NT, smem, st, V, logits, ldl, targets, ignore_index, inv_count,
+                row_loss, write_grad, cached, vec);
+    return 0;
+  });
+  if (rc) return rc;
   ICAP_LAUNCH_CHECK("icap_xent");
   return 0;
 }
@@ -928,8 +919,9 @@ extern "C" int icap_argmax(int dtype, int64_t M, int64_t V, const void* logits, 
                            int64_t out_stride, float* gap, void* stream) {
   ICAP_ARG(M > 0 && V > 0 && logits && out, "icap_argmax: null/empty argument");
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == ICAP_F32) icap_launch(argmax_kernel<float>, (unsigned)M, NT, 0, st, (int)V, (const float*)logits, ldl, out, out_stride, gap);
-  else icap_launch(argmax_kernel<bf16>, (unsigned)M, NT, 0, st, (int)V, (const bf16*)logits, ldl, out, out_stride, gap);
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(argmax_kernel<decltype(tag)>, (unsigned)M, NT, 0, st, V, logits, ldl, out, out_stride, gap);
+  });
   ICAP_LAUNCH_CHECK("icap_argmax");
   return 0;
 }
@@ -943,12 +935,10 @@ extern "C" int icap_sample_tokens(int dtype, int64_t M, int64_t V, const void* l
   ICAP_ARG(ldl >= V && V < (1 << 30) && M < (1ll << 31), "icap_sample_tokens: bad logits shape");
   ICAP_ARG(t >= 0 && t + 1 < Tmax && ldp > t, "icap_sample_tokens: position %lld out of range", (long long)t);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == ICAP_F32)
-    icap_launch(sample_kernel<float>, (unsigned)M, NT, 0, st, (int)V, (const float*)logits, ldl, inv_temperature, seed,
-                seed_dev, (int)t, (int)Tmax, tokens, logp, ldp, end_idx, pad_idx);
-  else
-    icap_launch(sample_kernel<bf16>, (unsigned)M, NT, 0, st, (int)V, (const bf16*)logits, ldl, inv_temperature, seed,
-                seed_dev, (int)t, (int)Tmax, tokens, logp, ldp, end_idx, pad_idx);
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(sample_kernel<decltype(tag)>, (unsigned)M, NT, 0, st, V, logits, ldl, inv_temperature, seed, seed_dev, t, Tmax,
+                tokens, logp, ldp, end_idx, pad_idx);
+  });
   ICAP_LAUNCH_CHECK("icap_sample_tokens");
   return 0;
 }
@@ -964,18 +954,15 @@ extern "C" int icap_beam_select(int dtype, int64_t B, int64_t kin, int64_t V, co
   ICAP_ARG(kin * V > kout, "icap_beam_select: fewer candidates than beams");
   ICAP_ARG(stats == nullptr || V < (1 << 27), "icap_beam_select: V too large for the statistics path");
   cudaStream_t st = (cudaStream_t)stream;
-#define GO_SELECT(T)                                                                                                  \
-  do {                                                                                                                \
-    if (stats)                                                                                                        \
-      icap_launch(beam_select_stats_kernel<T>, (unsigned)B, NT, 0, st, (int)kin, (int)V, (const T*)logits, ldl, prev_score,  \
-                  (int)kout, out_score, out_parent, out_token, gap, log_domain, stats, stats_ld);                    \
-    else                                                                                                              \
-      icap_launch(beam_select_kernel<T>, (unsigned)B, NT, 0, st, (int)kin, (int)V, (const T*)logits, ldl, prev_score,        \
-                  (int)kout, out_score, out_parent, out_token, gap, log_domain);                                     \
-  } while (0)
-  if (dtype == ICAP_F32) GO_SELECT(float);
-  else GO_SELECT(bf16);
-#undef GO_SELECT
+  dispatch_act(dtype, [&](auto tag) {
+    using T = decltype(tag);
+    if (stats)
+      icap_launch(beam_select_stats_kernel<T>, (unsigned)B, NT, 0, st, kin, V, logits, ldl, prev_score, kout, out_score,
+                  out_parent, out_token, gap, log_domain, stats, stats_ld);
+    else
+      icap_launch(beam_select_kernel<T>, (unsigned)B, NT, 0, st, kin, V, logits, ldl, prev_score, kout, out_score, out_parent,
+                  out_token, gap, log_domain);
+  });
   ICAP_LAUNCH_CHECK("icap_beam_select");
   return 0;
 }

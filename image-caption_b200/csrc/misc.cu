@@ -338,12 +338,13 @@ extern "C" int icap_copy2d(const void* src, int src_dtype, int64_t src_ld, void*
                   (src_ld % 4 == 0) && (dst_ld % 4 == 0);
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned g = grid_for(vec ? rows * cols / 4 : rows * cols, 256);
-#define GO(TS, TD) icap_launch(copy2d_kernel<TS, TD>, g, 256, 0, st, (const TS*)src, src_ld, (TD*)dst, dst_ld, rows, cols, accumulate, vec)
-  if (src_dtype == ICAP_F32 && dst_dtype == ICAP_F32) GO(float, float);
-  else if (src_dtype == ICAP_F32 && dst_dtype == ICAP_BF16) GO(float, bf16);
-  else if (src_dtype == ICAP_BF16 && dst_dtype == ICAP_F32) GO(bf16, float);
-  else GO(bf16, bf16);
-#undef GO
+  auto go = [&](auto ts, auto td) {
+    icap_launch(copy2d_kernel<decltype(ts), decltype(td)>, g, 256, 0, st, src, src_ld, dst, dst_ld, rows, cols, accumulate, vec);
+  };
+  if (src_dtype == ICAP_F32 && dst_dtype == ICAP_F32) go(float{}, float{});
+  else if (src_dtype == ICAP_F32 && dst_dtype == ICAP_BF16) go(float{}, bf16{});
+  else if (src_dtype == ICAP_BF16 && dst_dtype == ICAP_F32) go(bf16{}, float{});
+  else go(bf16{}, bf16{});
   ICAP_LAUNCH_CHECK("icap_copy2d");
   return 0;
 }
@@ -356,12 +357,10 @@ extern "C" int icap_rows_gather_add(int dtype, const void* src, int64_t src_ld, 
            "icap_rows_gather_add: leading dimensions must be multiples of 4");
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned g = grid_for(rows * cols / 4, 256);
-  if (dtype == ICAP_F32)
-    icap_launch(rows_gather_add_kernel<float>, g, 256, 0, st, (const float*)src, src_ld, (const float*)base, base_ld, (float*)dst,
-                                                     dst_ld, rows, (int)cols, (int)div, (int)mul, (int)off);
-  else
-    icap_launch(rows_gather_add_kernel<bf16>, g, 256, 0, st, (const bf16*)src, src_ld, (const bf16*)base, base_ld, (bf16*)dst,
-                                                    dst_ld, rows, (int)cols, (int)div, (int)mul, (int)off);
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(rows_gather_add_kernel<decltype(tag)>, g, 256, 0, st, src, src_ld, base, base_ld, dst, dst_ld, rows, cols, div,
+                mul, off);
+  });
   ICAP_LAUNCH_CHECK("icap_rows_gather_add");
   return 0;
 }
@@ -371,12 +370,9 @@ extern "C" int icap_rows_segsum_add(int dtype, const void* src, int64_t src_ld, 
   ICAP_ARG(src && dst && nseg > 0 && seg_len > 0 && cols > 0, "icap_rows_segsum_add: bad argument");
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned g = grid_for(nseg * cols, 256);
-  if (dtype == ICAP_F32)
-    icap_launch(rows_segsum_add_kernel<float>, g, 256, 0, st, (const float*)src, src_ld, (float*)dst, dst_ld, nseg, (int)seg_len,
-                                                     (int)cols, (int)mul, (int)off);
-  else
-    icap_launch(rows_segsum_add_kernel<bf16>, g, 256, 0, st, (const bf16*)src, src_ld, (bf16*)dst, dst_ld, nseg, (int)seg_len,
-                                                    (int)cols, (int)mul, (int)off);
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(rows_segsum_add_kernel<decltype(tag)>, g, 256, 0, st, src, src_ld, dst, dst_ld, nseg, seg_len, cols, mul, off);
+  });
   ICAP_LAUNCH_CHECK("icap_rows_segsum_add");
   return 0;
 }
@@ -401,12 +397,11 @@ extern "C" int icap_gather_regions(int dtype, const void* cache, const uint8_t* 
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t rows = B * R;
   const unsigned g = (unsigned)ceil_div64(rows, 8);
-  if (idx_is_int64)
-    icap_launch(gather_regions_kernel<long long>, g, 256, 0, st, (const uint4*)cache, valid_cache, (const long long*)idx,
-                rows, (int)R, (int)(row_bytes / 16), n_images, (uint4*)xcat, kvalid, rowscale, err);
-  else
-    icap_launch(gather_regions_kernel<int>, g, 256, 0, st, (const uint4*)cache, valid_cache, (const int*)idx, rows,
-                (int)R, (int)(row_bytes / 16), n_images, (uint4*)xcat, kvalid, rowscale, err);
+  auto go = [&](auto ti) {
+    icap_launch(gather_regions_kernel<decltype(ti)>, g, 256, 0, st, cache, valid_cache, idx, rows, R, row_bytes / 16,
+                n_images, xcat, kvalid, rowscale, err);
+  };
+  if (idx_is_int64) go(0ll); else go(0);
   ICAP_LAUNCH_CHECK("icap_gather_regions");
   return 0;
 }
@@ -419,12 +414,11 @@ extern "C" int icap_caption_prep(const void* captions, int cap_is_int64, int64_t
   cudaStream_t st = (cudaStream_t)stream;
   ICAP_CUDA(cudaMemsetAsync(count_i, 0, sizeof(int), st));
   const unsigned g = grid_for(B * (L - 1), 256);
-  if (cap_is_int64)
-    icap_launch(caption_prep_kernel<long long>, g, 256, 0, st, (const long long*)captions, (int)B, (int)L, pad_idx, inp, tgt,
-                                                      tok_valid, rowscale, count_i);
-  else
-    icap_launch(caption_prep_kernel<int>, g, 256, 0, st, (const int*)captions, (int)B, (int)L, pad_idx, inp, tgt, tok_valid,
-                                                rowscale, count_i);
+  auto go = [&](auto ti) {
+    icap_launch(caption_prep_kernel<decltype(ti)>, g, 256, 0, st, captions, B, L, pad_idx, inp, tgt, tok_valid, rowscale,
+                count_i);
+  };
+  if (cap_is_int64) go(0ll); else go(0);
   icap_launch(count_finish_kernel, 1, 1, 0, st, count_i, count_f2);
   ICAP_LAUNCH_CHECK("icap_caption_prep");
   return 0;
@@ -435,12 +429,13 @@ extern "C" int icap_embed_fwd(int table_dtype, int out_dtype, const int* tokens,
   ICAP_ARG(tokens && table && out && M > 0 && E % 4 == 0, "icap_embed_fwd: bad argument (E must be a multiple of 4)");
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned g = grid_for(M * E / 4, 256);
-  if (table_dtype == ICAP_F32 && out_dtype == ICAP_F32)
-    icap_launch(embed_fwd_kernel<float, float>, g, 256, 0, st, tokens, tok_stride, M, (int)E, (const float*)table, (float*)out, rowscale, pad_idx);
-  else if (table_dtype == ICAP_BF16 && out_dtype == ICAP_BF16)
-    icap_launch(embed_fwd_kernel<bf16, bf16>, g, 256, 0, st, tokens, tok_stride, M, (int)E, (const bf16*)table, (bf16*)out, rowscale, pad_idx);
-  else if (table_dtype == ICAP_F32 && out_dtype == ICAP_BF16)
-    icap_launch(embed_fwd_kernel<float, bf16>, g, 256, 0, st, tokens, tok_stride, M, (int)E, (const float*)table, (bf16*)out, rowscale, pad_idx);
+  auto go = [&](auto tt, auto to) {
+    icap_launch(embed_fwd_kernel<decltype(tt), decltype(to)>, g, 256, 0, st, tokens, tok_stride, M, E, table, out, rowscale,
+                pad_idx);
+  };
+  if (table_dtype == ICAP_F32 && out_dtype == ICAP_F32) go(float{}, float{});
+  else if (table_dtype == ICAP_BF16 && out_dtype == ICAP_BF16) go(bf16{}, bf16{});
+  else if (table_dtype == ICAP_F32 && out_dtype == ICAP_BF16) go(float{}, bf16{});
   else ICAP_ARG(false, "icap_embed_fwd: unsupported dtype combination");
   ICAP_LAUNCH_CHECK("icap_embed_fwd");
   return 0;
@@ -451,8 +446,9 @@ extern "C" int icap_embed_bwd(int dtype, const int* tokens, int64_t M, int64_t E
   ICAP_ARG(tokens && dout && dtable && M > 0 && E > 0, "icap_embed_bwd: null/empty argument");
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned g = grid_for(M * E, 256);
-  if (dtype == ICAP_F32) icap_launch(embed_bwd_kernel<float>, g, 256, 0, st, tokens, M, (int)E, pad_idx, (const float*)dout, dtable);
-  else icap_launch(embed_bwd_kernel<bf16>, g, 256, 0, st, tokens, M, (int)E, pad_idx, (const bf16*)dout, dtable);
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(embed_bwd_kernel<decltype(tag)>, g, 256, 0, st, tokens, M, E, pad_idx, dout, dtable);
+  });
   ICAP_LAUNCH_CHECK("icap_embed_bwd");
   return 0;
 }
@@ -467,8 +463,7 @@ extern "C" int icap_colsum(int dtype, int64_t M, int64_t N, const void* x, int64
     if (splits < 1) splits = 1;
     const int rpb = (int)ceil_div64(M, splits);
     dim3 grid8((unsigned)cb, (unsigned)ceil_div64(M, rpb)), block8(32, 8);
-    if (dtype == ICAP_F32) icap_launch(colsum8_kernel<float>, grid8, block8, 0, st, (const float*)x, ld, M, N, out, rpb);
-    else icap_launch(colsum8_kernel<bf16>, grid8, block8, 0, st, (const bf16*)x, ld, M, N, out, rpb);
+    dispatch_act(dtype, [&](auto tag) { icap_launch(colsum8_kernel<decltype(tag)>, grid8, block8, 0, st, x, ld, M, N, out, rpb); });
     ICAP_LAUNCH_CHECK("icap_colsum");
     return 0;
   }
@@ -478,8 +473,9 @@ extern "C" int icap_colsum(int dtype, int64_t M, int64_t N, const void* x, int64
   if (row_splits < 1) row_splits = 1;
   const int rows_per_block = (int)ceil_div64(M, row_splits);
   dim3 grid((unsigned)col_blocks, (unsigned)ceil_div64(M, rows_per_block)), block(32, 8);
-  if (dtype == ICAP_F32) icap_launch(colsum_kernel<float>, grid, block, 0, st, (const float*)x, ld, M, N, out, rows_per_block);
-  else icap_launch(colsum_kernel<bf16>, grid, block, 0, st, (const bf16*)x, ld, M, N, out, rows_per_block);
+  dispatch_act(dtype, [&](auto tag) {
+    icap_launch(colsum_kernel<decltype(tag)>, grid, block, 0, st, x, ld, M, N, out, rows_per_block);
+  });
   ICAP_LAUNCH_CHECK("icap_colsum");
   return 0;
 }
@@ -519,12 +515,6 @@ extern "C" int icap_scale(float* x, int64_t n, const float* s_dev, float s, void
 }
 
 // --------------------------------------------------------------------------- GEMM dispatcher
-int icap_gemm_f32_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64_t K, const float* A, int64_t lda,
-                         const float* B, int64_t ldb, float* C, int64_t ldc, const float* bias, int epi,
-                         const float* aux, int64_t ldaux, int accumulate, int split_k, cudaStream_t st);
-int icap_gemm_bf16_launch(int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64_t K, const void* A, int64_t lda,
-                          const void* B, int64_t ldb, void* C, int64_t ldc, int c_dtype, const float* bias, int epi,
-                          const void* aux, int64_t ldaux, int accumulate, int split_k, cudaStream_t st);
 
 extern "C" int icap_gemm(int ab_dtype, int a_kmajor, int b_kmajor, int64_t M, int64_t N, int64_t K, const void* A,
                          int64_t lda, const void* B, int64_t ldb, void* C, int64_t ldc, int c_dtype, const float* bias,

@@ -568,52 +568,43 @@ extern "C" int icap_add_ln_fwd(int a_dtype, int act_dtype, int64_t M, int64_t d,
   cudaStream_t st = (cudaStream_t)stream;
   dim3 grid((unsigned)ceil_div64(M, 8));
   const uint32_t th = dropout_threshold(p_drop);
+  // go(a element, act element): the three (a, act) combinations that exist; false for any other
+  auto by_dtypes = [&](auto go) {
+    if (a_dtype == ICAP_F32 && act_dtype == ICAP_F32) go(float{}, float{});
+    else if (a_dtype == ICAP_BF16 && act_dtype == ICAP_BF16) go(bf16{}, bf16{});
+    else if (a_dtype == ICAP_F32 && act_dtype == ICAP_BF16) go(float{}, bf16{});
+    else return false;
+    return true;
+  };
+  bool ok;
   if (d % 8 == 0 && M * (d / 8) < (1ll << 30) && aligned16(a) && aligned16(res) && aligned16(y) && aligned16(gamma) &&
       aligned16(beta) && !env_flag<4>("ICAP_LN_NARROW")) {
     static IcapEnv e_rpw;
     const int rpw = e_rpw.geti("ICAP_LN_RPW", 1);     // rows per warp (1 or 2)
     dim3 grid8((unsigned)ceil_div64(M, 8 * (rpw == 1 ? 1 : 2)));
-#define GO8R(NIT, R, TA, TR, TY)                                                                                  \
-  icap_launch(add_ln_fwd8_kernel<NIT, R, TA, TR, TY>, grid8, 256, 0, st, (int)M, (int)d, (TA*)a, (const TR*)res, \
-                                                             (int)res_rows, gamma, beta, rowscale, (TY*)y,       \
-                                                             mean_out, rstd_out, write_sum, p_drop, th, seed, seed_dev, eps)
-#define GO8(NIT, TA, TR, TY)                                                                                      \
-  do {                                                                                                            \
-    if (rpw == 1) GO8R(NIT, 1, TA, TR, TY); else GO8R(NIT, 2, TA, TR, TY);                                        \
-  } while (0)
-#define GOT8(TA, TR, TY)                                                                                          \
-  do {                                                                                                            \
-    if (d <= 256) GO8(1, TA, TR, TY);                                                                             \
-    else if (d <= 512) GO8(2, TA, TR, TY);                                                                        \
-    else GO8(4, TA, TR, TY);                                                                                      \
-  } while (0)
-    if (a_dtype == ICAP_F32 && act_dtype == ICAP_F32) GOT8(float, float, float);
-    else if (a_dtype == ICAP_BF16 && act_dtype == ICAP_BF16) GOT8(bf16, bf16, bf16);
-    else if (a_dtype == ICAP_F32 && act_dtype == ICAP_BF16) GOT8(float, bf16, bf16);
-    else ICAP_ARG(false, "icap_add_ln_fwd: unsupported dtype combination a=%d act=%d", a_dtype, act_dtype);
-#undef GO8R
-#undef GOT8
-#undef GO8
-    ICAP_LAUNCH_CHECK("icap_add_ln_fwd");
-    return 0;
+    ok = by_dtypes([&](auto ta, auto tr) {
+      auto go = [&](auto nit, auto r) {
+        icap_launch(add_ln_fwd8_kernel<nit, r, decltype(ta), decltype(tr), decltype(tr)>, grid8, 256, 0, st, M, d, a, res,
+                    res_rows, gamma, beta, rowscale, y, mean_out, rstd_out, write_sum, p_drop, th, seed, seed_dev, eps);
+      };
+      auto by_rpw = [&](auto nit) { if (rpw == 1) go(nit, int_c<1>{}); else go(nit, int_c<2>{}); };
+      if (d <= 256) by_rpw(int_c<1>{});
+      else if (d <= 512) by_rpw(int_c<2>{});
+      else by_rpw(int_c<4>{});
+    });
+  } else {
+    ok = by_dtypes([&](auto ta, auto tr) {
+      auto go = [&](auto nit) {
+        icap_launch(add_ln_fwd_kernel<nit, decltype(ta), decltype(tr), decltype(tr)>, grid, 256, 0, st, M, d, a, res, res_rows,
+                    gamma, beta, rowscale, y, mean_out, rstd_out, write_sum, p_drop, th, seed, seed_dev, eps);
+      };
+      if (d <= 128) go(int_c<1>{});
+      else if (d <= 256) go(int_c<2>{});
+      else if (d <= 512) go(int_c<4>{});
+      else go(int_c<8>{});
+    });
   }
-#define GO1(NIT, TA, TR, TY)                                                                                      \
-  icap_launch(add_ln_fwd_kernel<NIT, TA, TR, TY>, grid, 256, 0, st, (int)M, (int)d, (TA*)a, (const TR*)res,               \
-                                                            (int)res_rows, gamma, beta, rowscale, (TY*)y,        \
-                                                            mean_out, rstd_out, write_sum, p_drop, th, seed, seed_dev, eps)
-#define GO(TA, TR, TY)                                                                                            \
-  do {                                                                                                            \
-    if (d <= 128) GO1(1, TA, TR, TY);                                                                             \
-    else if (d <= 256) GO1(2, TA, TR, TY);                                                                        \
-    else if (d <= 512) GO1(4, TA, TR, TY);                                                                        \
-    else GO1(8, TA, TR, TY);                                                                                      \
-  } while (0)
-  if (a_dtype == ICAP_F32 && act_dtype == ICAP_F32) GO(float, float, float);
-  else if (a_dtype == ICAP_BF16 && act_dtype == ICAP_BF16) GO(bf16, bf16, bf16);
-  else if (a_dtype == ICAP_F32 && act_dtype == ICAP_BF16) GO(float, bf16, bf16);
-  else ICAP_ARG(false, "icap_add_ln_fwd: unsupported dtype combination a=%d act=%d", a_dtype, act_dtype);
-#undef GO
-#undef GO1
+  ICAP_ARG(ok, "icap_add_ln_fwd: unsupported dtype combination a=%d act=%d", a_dtype, act_dtype);
   ICAP_LAUNCH_CHECK("icap_add_ln_fwd");
   return 0;
 }
@@ -648,54 +639,41 @@ static int add_ln_bwd_impl(int which, int act_dtype, int64_t M, int64_t d, const
     if (splits8 > ceil_div64(M, 16)) splits8 = ceil_div64(M, 16);
     const int rpb8 = (int)ceil_div64(M, splits8);
     dim3 cgrid8((unsigned)col_blocks8, (unsigned)ceil_div64(M, rpb8));
-#define GOB8R(NIT, R, T)                                                                                          \
-  icap_launch(add_ln_bwd_rows8_kernel<NIT, R, T>, row_blocks8, 256, 0, st, (int)M, (int)d, (const T*)dy1,         \
-              (const T*)dy2, (const T*)s, mean, rstd, gamma, rowscale, (T*)ds, (T*)da, p_drop, th, seed, seed_dev)
-#define GOB8(NIT, T)                                                                                              \
-  do {                                                                                                            \
-    if (rpw == 1) GOB8R(NIT, 1, T); else GOB8R(NIT, 2, T);                                                        \
-  } while (0)
-#define GOBT8(T)                                                                                                  \
-  do {                                                                                                            \
-    if ((ds || da) && (which & 1)) {                                                                              \
-      if (d <= 256) GOB8(1, T);                                                                                   \
-      else if (d <= 512) GOB8(2, T);                                                                              \
-      else GOB8(4, T);                                                                                            \
-    }                                                                                                             \
-    if (dgamma || dbeta || dbias2)                                                                                \
-      icap_launch(add_ln_bwd_cols8_kernel<T>, cgrid8, cblock, 0, st, (int)M, (int)d, (const T*)dy1, (const T*)dy2,         \
-                                                            (const T*)s, mean, rstd, rowscale, (const T*)dab,    \
-                                                            dgamma, dbeta, dbias2, rpb8);                        \
-  } while (0)
-    if (act_dtype == ICAP_F32) GOBT8(float);
-    else GOBT8(bf16);
-#undef GOBT8
-#undef GOB8
-#undef GOB8R
+    dispatch_act(act_dtype, [&](auto tag) {
+      using T = decltype(tag);
+      if ((ds || da) && (which & 1)) {
+        auto go = [&](auto nit, auto r) {
+          icap_launch(add_ln_bwd_rows8_kernel<nit, r, T>, row_blocks8, 256, 0, st, M, d, dy1, dy2, s, mean, rstd, gamma,
+                      rowscale, ds, da, p_drop, th, seed, seed_dev);
+        };
+        auto by_rpw = [&](auto nit) { if (rpw == 1) go(nit, int_c<1>{}); else go(nit, int_c<2>{}); };
+        if (d <= 256) by_rpw(int_c<1>{});
+        else if (d <= 512) by_rpw(int_c<2>{});
+        else by_rpw(int_c<4>{});
+      }
+      if (dgamma || dbeta || dbias2)
+        icap_launch(add_ln_bwd_cols8_kernel<T>, cgrid8, cblock, 0, st, M, d, dy1, dy2, s, mean, rstd, rowscale, dab, dgamma,
+                    dbeta, dbias2, rpb8);
+    });
     ICAP_LAUNCH_CHECK("icap_add_ln_bwd");
     return 0;
   }
-#define GOB(NIT, T)                                                                                               \
-  icap_launch(add_ln_bwd_rows_kernel<NIT, T>, row_blocks, 256, 0, st, (int)M, (int)d, (const T*)dy1, (const T*)dy2,        \
-                                                             (const T*)s, mean, rstd, gamma, rowscale, (T*)ds,   \
-                                                             (T*)da, p_drop, th, seed, seed_dev)
-#define GOBT(T)                                                                                                   \
-  do {                                                                                                            \
-    if ((ds || da) && (which & 1)) {                                                                              \
-      if (d <= 128) GOB(1, T);                                                                                    \
-      else if (d <= 256) GOB(2, T);                                                                               \
-      else if (d <= 512) GOB(4, T);                                                                               \
-      else GOB(8, T);                                                                                             \
-    }                                                                                                             \
-    if ((dgamma || dbeta || dbias2) && (which & 2))                                                               \
-      icap_launch(add_ln_bwd_cols_kernel<T>, cgrid, cblock, 0, st, (int)M, (int)d, (const T*)dy1, (const T*)dy2,           \
-                                                          (const T*)s, mean, rstd, rowscale, (const T*)dab,      \
-                                                          dgamma, dbeta, dbias2, rows_per_block);                 \
-  } while (0)
-  if (act_dtype == ICAP_F32) GOBT(float);
-  else GOBT(bf16);
-#undef GOBT
-#undef GOB
+  dispatch_act(act_dtype, [&](auto tag) {
+    using T = decltype(tag);
+    if ((ds || da) && (which & 1)) {
+      auto go = [&](auto nit) {
+        icap_launch(add_ln_bwd_rows_kernel<nit, T>, row_blocks, 256, 0, st, M, d, dy1, dy2, s, mean, rstd, gamma, rowscale, ds,
+                    da, p_drop, th, seed, seed_dev);
+      };
+      if (d <= 128) go(int_c<1>{});
+      else if (d <= 256) go(int_c<2>{});
+      else if (d <= 512) go(int_c<4>{});
+      else go(int_c<8>{});
+    }
+    if ((dgamma || dbeta || dbias2) && (which & 2))
+      icap_launch(add_ln_bwd_cols_kernel<T>, cgrid, cblock, 0, st, M, d, dy1, dy2, s, mean, rstd, rowscale, dab, dgamma, dbeta,
+                  dbias2, rows_per_block);
+  });
   ICAP_LAUNCH_CHECK("icap_add_ln_bwd");
   return 0;
 }
@@ -737,20 +715,15 @@ extern "C" int icap_decode_embed_ln(int act_dtype, int64_t rows, int64_t d, int6
            "icap_decode_embed_ln: the beam reorder is out of place and needs token / tok_out (and slot_out with slot_in)");
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned grid = (unsigned)ceil_div64(rows, 8);
-#define GODE(NIT, T)                                                                                                   \
-  icap_launch(decode_embed_ln_kernel<NIT, T>, grid, 256, 0, st, (int)rows, (int)d, (int)k, (int)Tmax, (int)t, parent, token,  \
-              tok_in, tok_out, slot_in, slot_out, (const T*)table, (const T*)pos_row, gamma, beta, (T*)y, rowscale, pad_idx, \
-              eps)
-#define GODET(T)                                                                                                       \
-  do {                                                                                                                 \
-    if (d <= 256) GODE(1, T);                                                                                          \
-    else if (d <= 512) GODE(2, T);                                                                                     \
-    else GODE(4, T);                                                                                                   \
-  } while (0)
-  if (act_dtype == ICAP_F32) GODET(float);
-  else GODET(bf16);
-#undef GODET
-#undef GODE
+  dispatch_act(act_dtype, [&](auto tag) {
+    auto go = [&](auto nit) {
+      icap_launch(decode_embed_ln_kernel<nit, decltype(tag)>, grid, 256, 0, st, rows, d, k, Tmax, t, parent, token, tok_in, tok_out,
+                  slot_in, slot_out, table, pos_row, gamma, beta, y, rowscale, pad_idx, eps);
+    };
+    if (d <= 256) go(int_c<1>{});
+    else if (d <= 512) go(int_c<2>{});
+    else go(int_c<4>{});
+  });
   ICAP_LAUNCH_CHECK("icap_decode_embed_ln");
   return 0;
 }
