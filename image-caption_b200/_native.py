@@ -36,6 +36,8 @@ SIGNATURES = {
     "icap_argmax": [I, L, L, P, L, P, L, P, P],
     "icap_sample_tokens": [I, L, L, P, L, F, U, P, L, L, P, P, L, I, I, P],
     "icap_beam_select": [I, L, L, L, P, L, P, L, P, P, P, P, I, P, L, P],
+    "icap_beam_select_eos": [I, L, L, L, P, L, P, L, P, P, P, P, I, P, L, P, L, L, I, I, P],
+    "icap_beam_finalize": [L, L, L, P, P, I, I, F, L, P, P, P, P],
     "icap_beam_reorder": [L, L, L, L, P, P, P, P, P, P, P],
     "icap_decode_embed_ln": [I, L, L, L, L, L, P, P, P, P, P, P, P, P, P, P, P, P, I, F, P],
     "icap_log_softmax_argmax": [L, L, P, L, P, L, P, P],

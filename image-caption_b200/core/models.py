@@ -76,6 +76,17 @@ class MODEL_init:
         return self.model.sample_captions(cache.batch(image_idxs), None, num_samples=num_samples,
                                           temperature=temperature, seed=seed)
 
+    def generate_caption_ids_nbest(self, object_features, position_features, beam_size=5, n_best=None,
+                                   length_penalty=0.0):
+        """The n_best captions per image of the beam search that stops at <END> (Transformer.beam_search_nbest): (ids
+        [B, n, L], log-probabilities [B, n], lengths [B, n]) on the device, best first."""
+        return self.model.beam_search_nbest(object_features.to(DEVICE), position_features.to(DEVICE),
+                                            beam_size=beam_size, n_best=n_best, length_penalty=length_penalty)
+
+    def generate_caption_ids_nbest_cached(self, cache, image_idxs, beam_size=5, n_best=None, length_penalty=0.0):
+        return self.model.beam_search_nbest(cache.batch(image_idxs), None, beam_size=beam_size, n_best=n_best,
+                                            length_penalty=length_penalty)
+
     def decode_captions(self, caption_vector):
         return decode_captions(captions=caption_vector, index_to_word=self.idx_to_word)
 

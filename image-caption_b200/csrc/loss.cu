@@ -9,6 +9,8 @@
 //   beam  : Softmax(logits) + prev_score, cat over beams, topk(k),
 //           parent = idx // V, token = idx % V                           model.py:181-198
 //           (LogSoftmax in the PolicyNetwork variant, model_RL.py:72)
+// Not in the reference: the <END>-aware variant of the beam step (EOS template flag of the beam_select kernels; finished
+// hypotheses carry their score unchanged) and the final length-normalised ranking of the beams (beam_finalize_kernel).
 #include "icap_common.cuh"
 
 namespace {
@@ -374,15 +376,30 @@ constexpr int KMAX = 8;   // beam width limit; lists hold KMAX+1 entries so the 
 struct Cand { float s; int i; };
 __device__ __forceinline__ bool better(float s, int i, float s2, int i2) { return s > s2 || (s == s2 && i < i2); }
 
+// End-of-sequence handling of icap_beam_select_eos: hypothesis `row` is finished at step t >= 1 when its token at
+// position t is end_idx or pad_idx (the rule of icap_sample_tokens); a finished row offers the one candidate
+// (token pad_idx, score prev[row]) instead of its V logits.
+struct EosArgs {
+  const int* tokens;
+  int Tmax, t, end_idx, pad_idx;
+};
+__device__ __forceinline__ bool eos_finished(const EosArgs& e, int row) {
+  if (e.t < 1) return false;
+  const int tk = e.tokens[(int64_t)row * e.Tmax + e.t];
+  return tk == e.end_idx || tk == e.pad_idx;
+}
+
 // Exact selection without a candidate bound: every thread keeps the sorted best L of the candidates it scans, the block
 // merges the lists.  The fall-back of both beam_select kernels when more than CAND_CAP candidates tie with the bound
 // (degenerate logits); needs the softmax maximum / denominator of every row in s_mx / s_den.  Whole block, convergent.
-template <typename T>
+// EOS: rows with s_fin[r] set scan nothing; thread 0 offers their single candidate (prev, r * V + pad_idx).
+template <typename T, bool EOS = false>
 __device__ __forceinline__ void beam_select_exact(int b, int kin, int V, const T* __restrict__ logits, int64_t ldl,
                                                const float* __restrict__ prev, int kout, float* __restrict__ out_score,
                                                int* __restrict__ out_parent, int* __restrict__ out_token,
                                                float* __restrict__ gap, int log_domain, const float* s_mx,
-                                               const float* s_den, float* h_s, int* h_i, int* h_t) {
+                                               const float* s_den, float* h_s, int* h_i, int* h_t,
+                                               const int* s_fin = nullptr, int pad_idx = 0) {
   const bool vec = ((uintptr_t)logits % 16 == 0) && (ldl * sizeof(T)) % 16 == 0;
   const int L = kout + 1;
   Cand lst[KMAX + 1];                      // sorted, best first; only static indices (stays in registers)
@@ -390,7 +407,26 @@ __device__ __forceinline__ void beam_select_exact(int b, int kin, int V, const T
   for (int t = 0; t <= KMAX; ++t) { lst[t].s = -INFINITY; lst[t].i = 0x7fffffff; }
   float worst_s = -INFINITY;               // == lst[L-1]: the entry a candidate has to beat
   int worst_i = 0x7fffffff;
+  auto push = [&](float sc, int idx) {     // sc, idx beat (worst_s, worst_i): insert, keep the list sorted
+#pragma unroll
+    for (int t = 0; t <= KMAX; ++t) if (t == L - 1) { lst[t].s = sc; lst[t].i = idx; }
+#pragma unroll
+    for (int t = KMAX; t > 0; --t) {
+      if (t < L && better(lst[t].s, lst[t].i, lst[t - 1].s, lst[t - 1].i)) {
+        Cand c = lst[t]; lst[t] = lst[t - 1]; lst[t - 1] = c;
+      }
+    }
+#pragma unroll
+    for (int t = 0; t <= KMAX; ++t) if (t == L - 1) { worst_s = lst[t].s; worst_i = lst[t].i; }
+  };
   for (int r = 0; r < kin; ++r) {
+    if constexpr (EOS) {
+      if (s_fin[r]) {
+        const float pv = prev ? prev[b * kin + r] : 0.f;
+        if (threadIdx.x == 0 && better(pv, r * V + pad_idx, worst_s, worst_i)) push(pv, r * V + pad_idx);
+        continue;
+      }
+    }
     const T* x = logits + ((int64_t)b * kin + r) * ldl;
     const float mx = s_mx[r], den = s_den[r], pv = prev ? prev[b * kin + r] : 0.f;
     // Cheap pre-filter in the logit domain: the score is monotonic in the logit, so only logits above
@@ -414,16 +450,7 @@ __device__ __forceinline__ void beam_select_exact(int b, int kin, int V, const T
         const float sc = (log_domain ? (xv - mx - den) : (expf(xv - mx) / den)) + pv;
         const int idx = r * V + j0 + i;
         if (better(sc, idx, worst_s, worst_i)) {
-#pragma unroll
-          for (int t = 0; t <= KMAX; ++t) if (t == L - 1) { lst[t].s = sc; lst[t].i = idx; }
-#pragma unroll
-          for (int t = KMAX; t > 0; --t) {
-            if (t < L && better(lst[t].s, lst[t].i, lst[t - 1].s, lst[t - 1].i)) {
-              Cand c = lst[t]; lst[t] = lst[t - 1]; lst[t - 1] = c;
-            }
-          }
-#pragma unroll
-          for (int t = 0; t <= KMAX; ++t) if (t == L - 1) { worst_s = lst[t].s; worst_i = lst[t].i; }
+          push(sc, idx);
           refresh_tl();
         }
       }
@@ -469,11 +496,11 @@ __device__ __forceinline__ void beam_select_exact(int b, int kin, int V, const T
   }
 }
 
-template <typename T>
+template <typename T, bool EOS = false>
 __global__ void __launch_bounds__(NT)
 beam_select_kernel(int kin, int V, const T* __restrict__ logits, int64_t ldl, const float* __restrict__ prev,
                    int kout, float* __restrict__ out_score, int* __restrict__ out_parent, int* __restrict__ out_token,
-                   float* __restrict__ gap, int log_domain) {
+                   float* __restrict__ gap, int log_domain, EosArgs eos) {
   pdl_prologue();
   __shared__ float red[NT / 32];
   __shared__ float s_mx[KMAX], s_den[KMAX];
@@ -488,7 +515,20 @@ beam_select_kernel(int kin, int V, const T* __restrict__ logits, int64_t ldl, co
   __shared__ int c_i[CAND_CAP];
   __shared__ int c_n;
   __shared__ float s_tau;
+  __shared__ int s_fin[KMAX];                         // EOS: row r is finished
+  if constexpr (EOS) {
+    if (threadIdx.x < kin) s_fin[threadIdx.x] = eos_finished(eos, b * kin + threadIdx.x);
+    __syncthreads();
+  }
   for (int r = 0; r < kin; ++r) {
+    if constexpr (EOS) {
+      if (s_fin[r]) {                                 // no logits read: the row's statistics stay empty
+        if ((threadIdx.x & 31) == 0) {
+          s_w1[r][threadIdx.x >> 5] = -INFINITY; s_w2[r][threadIdx.x >> 5] = -INFINITY; s_we[r][threadIdx.x >> 5] = 0.f;
+        }
+        continue;
+      }
+    }
     const T* x = logits + ((int64_t)b * kin + r) * ldl;
     // ONE pass: the thread's two largest logits (t1 >= t2) and its online softmax sum  es = sum exp(x - t1)
     float t1 = -INFINITY, t2 = -INFINITY, es = 0.f;
@@ -553,6 +593,9 @@ beam_select_kernel(int kin, int V, const T* __restrict__ logits, int64_t ldl, co
             const float pv = prev ? prev[b * kin + r] : 0.f;
             sc = (log_domain ? (lg - s_mx[r] - s_den[r]) : (expf(lg - s_mx[r]) / s_den[r])) + pv;
           }
+          if constexpr (EOS) {                         // a finished row's single candidate
+            if (s_fin[r] && e % PER == 0) sc = prev ? prev[b * kin + r] : 0.f;
+          }
         }
         cs[u] = sc;
       }
@@ -581,6 +624,16 @@ beam_select_kernel(int kin, int V, const T* __restrict__ logits, int64_t ldl, co
     __syncthreads();
     const float tau = s_tau;
     for (int r = 0; r < kin; ++r) {
+      if constexpr (EOS) {
+        if (s_fin[r]) {
+          const float pv = prev ? prev[b * kin + r] : 0.f;
+          if (threadIdx.x == 0 && pv >= tau) {
+            const int pos = atomicAdd(&c_n, 1);
+            if (pos < CAND_CAP) { c_s[pos] = pv; c_i[pos] = r * V + eos.pad_idx; }
+          }
+          continue;
+        }
+      }
       const T* x = logits + ((int64_t)b * kin + r) * ldl;
       const float mx = s_mx[r], den = s_den[r], pv = prev ? prev[b * kin + r] : 0.f;
       float tl;                                        // logit whose score is tau, minus a safety margin
@@ -638,8 +691,8 @@ beam_select_kernel(int kin, int V, const T* __restrict__ logits, int64_t ldl, co
     }
     // more than CAND_CAP candidates tie with tau (degenerate logits): exact but slow path below
   }
-  beam_select_exact<T>(b, kin, V, logits, ldl, prev, kout, out_score, out_parent, out_token, gap, log_domain, s_mx, s_den,
-                       h_s, h_i, h_t);
+  beam_select_exact<T, EOS>(b, kin, V, logits, ldl, prev, kout, out_score, out_parent, out_token, gap, log_domain, s_mx,
+                            s_den, h_s, h_i, h_t, EOS ? s_fin : nullptr, eos.pad_idx);
 }
 
 // The same selection fed with the classifier GEMM's ICAP_EPI_ROWSTATS buffer: (largest, second largest, sum exp(x -
@@ -659,12 +712,12 @@ __device__ __forceinline__ void top2sum_merge(float& t1, float& t2, float& es, f
   t1 = n1;
 }
 
-template <typename T>
+template <typename T, bool EOS = false>
 __global__ void __launch_bounds__(NT)
 beam_select_stats_kernel(int kin, int V, const T* __restrict__ logits, int64_t ldl, const float* __restrict__ prev,
                          int kout, float* __restrict__ out_score, int* __restrict__ out_parent,
                          int* __restrict__ out_token, float* __restrict__ gap, int log_domain,
-                         const float* __restrict__ stats, int64_t stats_ld) {
+                         const float* __restrict__ stats, int64_t stats_ld, EosArgs eos) {
   pdl_prologue();
   constexpr int NW = NT / 32, PER = 2 * NW;
   __shared__ float s_mx[KMAX], s_den[KMAX], s_pv[KMAX], s_tl[KMAX];
@@ -678,6 +731,7 @@ beam_select_stats_kernel(int kin, int V, const T* __restrict__ logits, int64_t l
   __shared__ float r_s[KMAX + 1];
   __shared__ float h_s[NT];
   __shared__ int h_i[NT], h_t[NT];
+  __shared__ int s_fin[KMAX];                          // EOS: row r is finished
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int L = kout + 1, np = (V + 127) / 128;
   const float4* sp0 = reinterpret_cast<const float4*>(stats + (int64_t)b * kin * stats_ld);
@@ -688,7 +742,18 @@ beam_select_stats_kernel(int kin, int V, const T* __restrict__ logits, int64_t l
   // ---- warp r owns row r: softmax maximum / sum of the row and, as candidates for the bound, the two largest logits of each
   // of 8 lane groups (partials pi with pi % 32 in [4g, 4g + 4)).  A loop and five shuffle rounds: small code -- the first
   // version, unrolled over the rows, spent 40 % of its samples waiting for instruction fetches.
-  if (warp < kin) {
+  bool fin = false;                                    // EOS: a finished row reads no statistics, offers one candidate
+  if constexpr (EOS) {
+    if (warp < kin) {
+      fin = eos_finished(eos, b * kin + warp);
+      if (lane == 0) s_fin[warp] = fin;
+      if (fin) {
+        if (lane < NW) { s_w1[warp][lane] = -INFINITY; s_w2[warp][lane] = -INFINITY; }
+        if (lane == 0) { s_mx[warp] = 0.f; s_den[warp] = 0.f; s_pv[warp] = prev ? prev[b * kin + warp] : 0.f; }
+      }
+    }
+  }
+  if (warp < kin && !fin) {
     const int r = warp;
     const float4* sp = sp0 + r * sld4;
     float t1 = -INFINITY, t2 = -INFINITY, es = 0.f;
@@ -718,6 +783,9 @@ beam_select_stats_kernel(int kin, int V, const T* __restrict__ logits, int64_t l
     const float lg = (tid & 1) ? s_w2[r][w] : s_w1[r][w];
     float sc = -INFINITY;
     if (lg > -INFINITY) sc = (log_domain ? (lg - s_mx[r] - s_den[r]) : (__expf(lg - s_mx[r]) / s_den[r])) + s_pv[r];
+    if constexpr (EOS) {
+      if (s_fin[r] && tid % PER == 0) sc = s_pv[r];
+    }
     b_s[tid] = sc;
   }
   __syncthreads();
@@ -742,7 +810,13 @@ beam_select_stats_kernel(int kin, int V, const T* __restrict__ logits, int64_t l
   }
   __syncthreads();
   // ---- the 128-logit segments whose maximum exceeds tl (about L of kin * V / 128) ...
-  if (warp < kin) {
+  if constexpr (EOS) {
+    if (fin && lane == 0 && s_pv[warp] >= tau) {
+      const int pos = atomicAdd(&c_n, 1);
+      if (pos < CAND_CAP) { c_s[pos] = s_pv[warp]; c_i[pos] = warp * V + eos.pad_idx; }
+    }
+  }
+  if (warp < kin && !fin) {
     const int r = warp;
     const float tl = s_tl[r];
     const float4* sp = sp0 + r * sld4;
@@ -805,8 +879,8 @@ beam_select_stats_kernel(int kin, int V, const T* __restrict__ logits, int64_t l
     return;
   }
   // too many segments / candidates tie with the bound (degenerate logits): exact path over the logits
-  beam_select_exact<T>(b, kin, V, logits, ldl, prev, kout, out_score, out_parent, out_token, gap, log_domain, s_mx, s_den,
-                       h_s, h_i, h_t);
+  beam_select_exact<T, EOS>(b, kin, V, logits, ldl, prev, kout, out_score, out_parent, out_token, gap, log_domain, s_mx,
+                            s_den, h_s, h_i, h_t, EOS ? s_fin : nullptr, eos.pad_idx);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -876,6 +950,61 @@ __global__ void beam_reorder_kernel(int B, int k, int Tmax, int t, const int* __
     tok_out[(int64_t)row * Tmax + j] = (j == t + 1) ? token[row] : tok_in[(int64_t)src * Tmax + j];
     if (slot_in) slot_out[(int64_t)row * Tmax + j] = (j == t + 1) ? row : slot_in[(int64_t)src * Tmax + j];
   }
+}
+
+// End of an <END>-aware beam search, one warp per image: lane s measures hypothesis s (generated tokens up to and including
+// the first end_idx; before a first pad_idx; Tmax - 1 if neither), normalises its score by ((5 + len) / 6)^alpha, and
+// ranks it by a count over the k normalised scores (ties: lower beam index); the warp then copies the n best token rows.
+__global__ void __launch_bounds__(32)
+beam_finalize_kernel(int k, int Tmax, const int* __restrict__ tokens, const float* __restrict__ score, int end_idx,
+                     int pad_idx, float alpha, int n, int* __restrict__ out_ids, float* __restrict__ out_score,
+                     int* __restrict__ out_len) {
+  pdl_prologue();
+  const int b = blockIdx.x, lane = threadIdx.x;
+  int len = 0;
+  float sc = 0.f, nrm = -INFINITY;
+  if (lane < k) {
+    const int* row = tokens + ((int64_t)b * k + lane) * Tmax;
+    len = Tmax - 1;
+    for (int j = 1; j < Tmax; ++j) {
+      const int tk = row[j];
+      if (tk == end_idx) { len = j; break; }
+      if (tk == pad_idx) { len = j - 1; break; }
+    }
+    sc = score[b * k + lane];
+    nrm = sc / powf((5.f + (float)len) / 6.f, alpha);
+  }
+  int rank = 0;
+  for (int s = 0; s < k; ++s) {
+    const float o = __shfl_sync(0xffffffffu, nrm, s);
+    rank += (o > nrm || (o == nrm && s < lane)) ? 1 : 0;
+  }
+  if (lane < k && rank < n) {
+    out_score[b * n + rank] = sc;
+    out_len[b * n + rank] = len;
+  }
+  for (int s = 0; s < k; ++s) {
+    const int rs = __shfl_sync(0xffffffffu, rank, s);
+    if (rs >= n) continue;
+    const int* src = tokens + ((int64_t)b * k + s) * Tmax;
+    int* dst = out_ids + ((int64_t)b * n + rs) * Tmax;
+    for (int j = lane; j < Tmax; j += 32) dst[j] = src[j];
+  }
+}
+
+template <bool EOS>
+void launch_beam_select(int dtype, int64_t B, int64_t kin, int64_t V, const void* logits, int64_t ldl,
+                        const float* prev_score, int64_t kout, float* out_score, int* out_parent, int* out_token, float* gap,
+                        int log_domain, const float* stats, int64_t stats_ld, EosArgs eos, cudaStream_t st) {
+  dispatch_act(dtype, [&](auto tag) {
+    using T = decltype(tag);
+    if (stats)
+      icap_launch(beam_select_stats_kernel<T, EOS>, (unsigned)B, NT, 0, st, kin, V, logits, ldl, prev_score, kout, out_score,
+                  out_parent, out_token, gap, log_domain, stats, stats_ld, eos);
+    else
+      icap_launch(beam_select_kernel<T, EOS>, (unsigned)B, NT, 0, st, kin, V, logits, ldl, prev_score, kout, out_score,
+                  out_parent, out_token, gap, log_domain, eos);
+  });
 }
 
 }  // namespace
@@ -953,17 +1082,46 @@ extern "C" int icap_beam_select(int dtype, int64_t B, int64_t kin, int64_t V, co
   ICAP_ARG(kin >= 1 && kin <= KMAX && kout >= 1 && kout <= KMAX, "icap_beam_select: beam width must be in [1, %d]", KMAX);
   ICAP_ARG(kin * V > kout, "icap_beam_select: fewer candidates than beams");
   ICAP_ARG(stats == nullptr || V < (1 << 27), "icap_beam_select: V too large for the statistics path");
-  cudaStream_t st = (cudaStream_t)stream;
-  dispatch_act(dtype, [&](auto tag) {
-    using T = decltype(tag);
-    if (stats)
-      icap_launch(beam_select_stats_kernel<T>, (unsigned)B, NT, 0, st, kin, V, logits, ldl, prev_score, kout, out_score,
-                  out_parent, out_token, gap, log_domain, stats, stats_ld);
-    else
-      icap_launch(beam_select_kernel<T>, (unsigned)B, NT, 0, st, kin, V, logits, ldl, prev_score, kout, out_score, out_parent,
-                  out_token, gap, log_domain);
-  });
+  launch_beam_select<false>(dtype, B, kin, V, logits, ldl, prev_score, kout, out_score, out_parent, out_token, gap,
+                            log_domain, stats, stats_ld, EosArgs{}, (cudaStream_t)stream);
   ICAP_LAUNCH_CHECK("icap_beam_select");
+  return 0;
+}
+
+extern "C" int icap_beam_select_eos(int dtype, int64_t B, int64_t kin, int64_t V, const void* logits, int64_t ldl,
+                                    const float* prev_score, int64_t kout, float* out_score, int* out_parent,
+                                    int* out_token, float* gap, int log_domain, const float* stats, int64_t stats_ld,
+                                    const int* tokens, int64_t Tmax, int64_t t, int end_idx, int pad_idx, void* stream) {
+  ICAP_ARG(stats == nullptr || (((uintptr_t)stats & 15) == 0 && stats_ld % 4 == 0 && stats_ld >= 4 * ((V + 127) / 128)),
+           "icap_beam_select_eos: the statistics buffer needs 16-byte alignment and >= 4 * ceil(V / 128) floats per row");
+  ICAP_ARG(B > 0 && V > 0 && logits && out_score && out_parent && out_token && tokens,
+           "icap_beam_select_eos: null/empty argument");
+  ICAP_ARG(kin >= 1 && kin <= KMAX && kout >= 1 && kout <= KMAX, "icap_beam_select_eos: beam width must be in [1, %d]",
+           KMAX);
+  ICAP_ARG(log_domain == 1, "icap_beam_select_eos: scores are log-probabilities (log_domain = 1)");
+  ICAP_ARG(t >= 0 && t + 1 < Tmax && Tmax < (1 << 30), "icap_beam_select_eos: position %lld out of range", (long long)t);
+  ICAP_ARG(pad_idx >= 0 && pad_idx < V, "icap_beam_select_eos: pad_idx must be a token");
+  // at t >= 1 every row offers at least one candidate (a finished row exactly one); at t = 0 no row is finished
+  ICAP_ARG(t >= 1 ? kin >= kout : kin * V > kout, "icap_beam_select_eos: fewer candidates than beams");
+  ICAP_ARG(stats == nullptr || V < (1 << 27), "icap_beam_select_eos: V too large for the statistics path");
+  launch_beam_select<true>(dtype, B, kin, V, logits, ldl, prev_score, kout, out_score, out_parent, out_token, gap,
+                           log_domain, stats, stats_ld, EosArgs{tokens, (int)Tmax, (int)t, end_idx, pad_idx},
+                           (cudaStream_t)stream);
+  ICAP_LAUNCH_CHECK("icap_beam_select_eos");
+  return 0;
+}
+
+extern "C" int icap_beam_finalize(int64_t B, int64_t k, int64_t Tmax, const int* tokens, const float* score, int end_idx,
+                                  int pad_idx, float alpha, int64_t n, int* out_ids, float* out_score, int* out_len,
+                                  void* stream) {
+  ICAP_ARG(B > 0 && Tmax > 1 && Tmax < (1 << 30) && tokens && score && out_ids && out_score && out_len,
+           "icap_beam_finalize: null/empty argument");
+  ICAP_ARG(k >= 1 && k <= KMAX && n >= 1 && n <= k, "icap_beam_finalize: need 1 <= n <= k <= %d", KMAX);
+  ICAP_ARG(isfinite(alpha) && alpha >= 0.f, "icap_beam_finalize: the length penalty must be finite and >= 0 (%g)",
+           (double)alpha);
+  icap_launch(beam_finalize_kernel, (unsigned)B, 32, 0, (cudaStream_t)stream, (int)k, (int)Tmax, tokens, score, end_idx,
+              pad_idx, alpha, (int)n, out_ids, out_score, out_len);
+  ICAP_LAUNCH_CHECK("icap_beam_finalize");
   return 0;
 }
 

@@ -955,7 +955,8 @@ class CaptionEngine:
     # ------------------------------------------------------------------ KV-cached decoding
     def decode(self, feats: torch.Tensor, pos: torch.Tensor, beam_size: int = 1, log_domain: bool = False,
                want_attention: bool = False, want_gaps: bool = False, num_samples: int = 0, temperature: float = 1.0,
-               sample_counter: Optional[torch.Tensor] = None):
+               sample_counter: Optional[torch.Tensor] = None, stop_at_end: bool = False, length_penalty: float = 0.0,
+               n_best: int = 0):
         """Greedy (beam_size=1: Transformer.generate_caption_vector, model.py:101-132) or beam search
         (Transformer.beam_search, model.py:135-200) with a KV cache: the reference re-runs the decoder on
         the whole prefix every step (and once per beam); here every step computes ONE position for all
@@ -969,9 +970,16 @@ class CaptionEngine:
         and log-probability 0.  The uniforms are keyed by the int32 device counter `sample_counter` (the engine's
         sample_dev by default), which the decode advances by one at its end.
 
+        stop_at_end: beam search that stops at <END> instead (also for beam_size = 1; icap_beam_select_eos): log-probability
+        scores, a hypothesis whose last token is <END> or <NULL> is finished and continues with <NULL> at an unchanged
+        score; after the last step the beams are ranked by score / ((5 + len) / 6)^length_penalty (icap_beam_finalize)
+        and the n_best (0: all beam_size) best are kept.
+
         Returns dict(ids int32 [B, T+1] (col 0 = <START>), attention fp32 [T, B, R] | None,
-                     gaps fp32 [T, B] | None)  -- all device tensors, no host sync.
-        Sampling: dict(ids int32 [B, n, T+1], logp fp32 [B, n, T] (log_softmax of the token at temperature 1))."""
+                     gaps fp32 [T, B] | None, score fp32 [B] (beam slot 0) | None)  -- all device tensors, no host sync.
+        Sampling: dict(ids int32 [B, n, T+1], logp fp32 [B, n, T] (log_softmax of the token at temperature 1)).
+        stop_at_end: dict(ids int32 [B, n, T+1], score fp32 [B, n] (log-probability), len int32 [B, n], gaps | None),
+        best first."""
         cfg = self.cfg
         assert self.tape is None
         self.training = False
@@ -984,7 +992,12 @@ class CaptionEngine:
             if sample_counter is None:
                 sample_counter = self.sample_dev
         k = int(num_samples) if sampling else int(beam_size)        # rows per image
-        beam = not sampling and k > 1
+        if stop_at_end:
+            assert not (sampling or want_attention), "the <END>-aware beam search returns ids, scores and lengths"
+            assert math.isfinite(length_penalty) and length_penalty >= 0, "the length penalty must be finite and >= 0"
+            n_best = int(n_best) or k
+            assert 1 <= n_best <= k, "n_best must be in [1, beam_size]"
+        beam = not sampling and (k > 1 or stop_at_end)
         B, R, _ = feats.shape
         T, d, V, E = cfg.T, cfg.decode_input_size, cfg.num_vocab, cfg.dim_word_embedding
         H, dk_tot, dv_tot, hid = cfg.decode_num_heads, cfg.decode_q_k_dim, cfg.decode_v_dim, cfg.decode_hidden_size
@@ -1109,10 +1122,14 @@ class CaptionEngine:
                     x, rowscale = step_input(t + 1, tk)
             else:
                 kin = 1 if t == 0 else k       # step 0: all beams hold <START>, only beam 0 competes (model.py:146-166)
-                call("icap_beam_select", self.act, B, kin, V, logits.data_ptr(), ldl * (k if t == 0 else 1),
-                     score[cur].data_ptr() if t > 0 else None, k, score[cur ^ 1].data_ptr(), parent.data_ptr(),
-                     newtok.data_ptr(), gaps[t].data_ptr() if gaps is not None else None, int(log_domain),
-                     _ptr(stats), (stats.shape[1] * (k if t == 0 else 1)) if stats is not None else 0, s())
+                args = (self.act, B, kin, V, logits.data_ptr(), ldl * (k if t == 0 else 1),
+                        score[cur].data_ptr() if t > 0 else None, k, score[cur ^ 1].data_ptr(), parent.data_ptr(),
+                        newtok.data_ptr(), gaps[t].data_ptr() if gaps is not None else None)
+                stats_args = (_ptr(stats), (stats.shape[1] * (k if t == 0 else 1)) if stats is not None else 0)
+                if stop_at_end:
+                    call("icap_beam_select_eos", *args, 1, *stats_args, tk.data_ptr(), Tmax, t, END_IDX, cfg.pad_idx, s())
+                else:
+                    call("icap_beam_select", *args, int(log_domain), *stats_args, s())
                 if t + 1 < T:       # bookkeeping of this step + input of the next one in one launch
                     x, rowscale = step_input(t + 1, tk, (parent, newtok, tok[cur ^ 1], slot[cur], slot[cur ^ 1]))
                 else:
@@ -1122,7 +1139,14 @@ class CaptionEngine:
         if sampling:
             call("icap_step_tick", sample_counter.data_ptr(), s())        # the next decode draws fresh uniforms
             return {"ids": tok[cur].view(B, k, Tmax), "logp": logp.view(B, k, T)}
+        if stop_at_end:
+            out_ids = torch.empty(B, n_best, Tmax, dtype=torch.int32, device=self.dev)
+            out_score = torch.empty(B, n_best, dtype=torch.float32, device=self.dev)
+            out_len = torch.empty(B, n_best, dtype=torch.int32, device=self.dev)
+            call("icap_beam_finalize", B, k, Tmax, tok[cur].data_ptr(), score[cur].data_ptr(), END_IDX, cfg.pad_idx,
+                 float(length_penalty), n_best, out_ids.data_ptr(), out_score.data_ptr(), out_len.data_ptr(), s())
+            return {"ids": out_ids, "score": out_score, "len": out_len, "gaps": gaps}
         ids = tok[cur].view(B, k, Tmax)[:, 0, :]
         if attn is not None:
             attn = attn.view(T, B, k, R)[:, :, 0, :]
-        return {"ids": ids, "attention": attn, "gaps": gaps}
+        return {"ids": ids, "attention": attn, "gaps": gaps, "score": score[cur][:, 0] if beam else None}

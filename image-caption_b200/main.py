@@ -142,8 +142,14 @@ def train(num_images=64, max_iters=None, region_cache=REGION_CACHE, reward='ngra
             break
 
 
-def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cache=REGION_CACHE):
+def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cache=REGION_CACHE, length_penalty=None):
+    """`--length-penalty A` decodes with the beam search that stops at <END> (beam width `--beam-size`, default 5) and
+    scores the best caption of each image by score / ((5 + len) / 6)^A; without it the reference's decoding runs."""
     model = _model()
+    nbest = length_penalty is not None
+    if nbest:
+        beam_size, length_penalty = int(beam_size or 5), float(length_penalty)
+        logps = []
     model_path = os.path.join(OUTPUT_PATH, f'model/model_{epoch}.pt')
     if os.path.exists(model_path):
         model.load(path=model_path)
@@ -159,7 +165,13 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
         loader = DataLoader(IndexedCaptions(ds, with_captions=False, unique_images=True), batch_size=BATCH_SIZE,
                             shuffle=False, collate_fn=_collate_idx)
         for (idxs,) in loader:
-            ids, _ = model.generate_caption_ids_cached(cache, idxs, beam_size=beam_size)
+            if nbest:
+                ids, logp, _ = model.generate_caption_ids_nbest_cached(cache, idxs, beam_size=beam_size, n_best=1,
+                                                                       length_penalty=length_penalty)
+                ids = ids[:, 0]
+                logps.append(logp[:, 0])
+            else:
+                ids, _ = model.generate_caption_ids_cached(cache, idxs, beam_size=beam_size)
             id_batches.append((idxs, ids))
             captions = model.decode_captions(ids.cpu().numpy())
             for i, idx in enumerate(idxs):
@@ -169,8 +181,14 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
         # host -> device copies of batch i + 1 run on a copy stream while batch i decodes
         loader = DataLoader(ds, batch_size=BATCH_SIZE, shuffle=False, pin_memory=True)
         for features, positions, idxs in PrefetchLoader(loader, DEVICE):
-            ids, _ = model.generate_caption_ids(object_features=features, position_features=positions,
-                                                beam_size=beam_size)
+            if nbest:
+                ids, logp, _ = model.generate_caption_ids_nbest(features, positions, beam_size=beam_size, n_best=1,
+                                                                length_penalty=length_penalty)
+                ids = ids[:, 0]
+                logps.append(logp[:, 0])
+            else:
+                ids, _ = model.generate_caption_ids(object_features=features, position_features=positions,
+                                                    beam_size=beam_size)
             id_batches.append((idxs, ids))
             captions = model.decode_captions(ids.cpu().numpy())
             for i, idx in enumerate(idxs.tolist()):
@@ -181,6 +199,9 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
     save_pickle(captions_out, os.path.join(target_dir, f'{split}.candidate.captions.pkl'))
     print(f'[evaluation] {len(captions_out)} captions in {dt:.2f}s ({len(captions_out) / dt:.1f} captions/s); '
           f'METEOR needs Java and is out of scope')
+    if nbest:
+        print(f'[evaluation] beam {beam_size} stopping at <END>, length penalty {length_penalty:g}: mean log-probability '
+              f'of the best caption {float(torch.cat(logps).mean()):.4f}')
     # the references: the split's caption file, or the synthetic split generated with its captions (same seed, so the
     # same images)
     scorer = _scorer(ds if 'captions' in ds.data else _dataset(True, num_images, split), model.num_vocab)
@@ -192,10 +213,12 @@ def evaluation(split='test', epoch=90, beam_size=None, num_images=64, region_cac
 
 
 def demo(image_path=None, beam_size=None, epoch=90, save_img=False, max_obj=False, features_path=None, num_samples=None,
-         temperature=1.0, seed=None):
+         temperature=1.0, seed=None, n_best=None, length_penalty=0.0):
     """The reference runs YOLOv5 + ResNet-101 on `image_path` first (main.py:195-197); offline, pass
     `--features-path file.pt` holding {'features': [R,2048], 'positions': [R,84]} or omit it for a synthetic image.
-    `--num-samples N [--temperature T] [--seed S]` prints N captions sampled from the model instead."""
+    `--num-samples N [--temperature T] [--seed S]` prints N captions sampled from the model instead.
+    `--n-best N [--beam-size k] [--length-penalty A]` prints the N best captions of the beam search that stops at <END>
+    (k defaults to max(N, 5)) with their log-probabilities."""
     model = _model()
     start = time.time()
     if features_path:
@@ -215,6 +238,15 @@ def demo(image_path=None, beam_size=None, epoch=90, save_img=False, max_obj=Fals
         captions = model.decode_captions(ids[0].cpu().numpy())
         for caption, lp in zip(captions, logp[0].sum(dim=1).tolist()):
             print(f'Sampled Caption: {caption}  (log-probability {lp:.3f})')
+        print('Spending Time:', time.time() - start)
+        return captions
+    if n_best is not None:
+        n = int(n_best)
+        ids, logp, lens = model.generate_caption_ids_nbest(feature, position, beam_size=int(beam_size or max(n, 5)),
+                                                           n_best=n, length_penalty=float(length_penalty))
+        captions = model.decode_captions(ids[0].cpu().numpy())
+        for caption, lp, ln in zip(captions, logp[0].tolist(), lens[0].tolist()):
+            print(f'Beam Caption: {caption}  (log-probability {lp:.3f}, {ln} tokens)')
         print('Spending Time:', time.time() - start)
         return captions
     caption, attention_list = model.generate_caption(object_features=feature, position_features=position,

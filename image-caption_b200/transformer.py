@@ -332,13 +332,16 @@ class Transformer(nn.Module):
         return lg[:, :self.num_vocab].float().view(B, T, self.num_vocab)
 
     def _decode(self, f, p, beam_size: int, log_domain: bool, want_attention: bool, num_samples: int = 0,
-                temperature: float = 1.0, seed: Optional[int] = None):
+                temperature: float = 1.0, seed: Optional[int] = None, stop_at_end: bool = False,
+                length_penalty: float = 0.0, n_best: int = 0):
         """KV-cached decode of one batch; the whole fixed-trip-count loop (encoder + max_length-1 steps, ~2000
         launches) is ONE CUDA graph per (batch, regions, beam) shape -- per (batch, regions, samples, temperature) when
         sampling -- unless ICAP_DECODE_GRAPH=0.  seed (sampling): the value of the sampling counter for this call."""
         eng = self._engine()
         eng.shadow_fresh = False                       # an external optimizer may have stepped the fp32 weights
         sample_kw = dict(num_samples=int(num_samples), temperature=float(temperature)) if num_samples else {}
+        if stop_at_end:
+            sample_kw.update(stop_at_end=True, length_penalty=float(length_penalty), n_best=int(n_best))
         if os.environ.get("ICAP_DECODE_GRAPH", "1") == "0":
             if seed is not None:
                 eng.sample_dev.fill_(seed)
@@ -346,7 +349,7 @@ class Transformer(nn.Module):
                               want_gaps=not num_samples, **sample_kw)
         cache = f.cache if isinstance(f, RegionBatch) else None
         key = (f.shape[0], f.shape[1], int(beam_size), bool(log_domain), bool(want_attention), id(eng), id(cache),
-               int(num_samples), float(temperature))
+               int(num_samples), float(temperature), bool(stop_at_end), float(length_penalty), int(n_best))
         gd = self._decode_graphs.get(key)
         if gd is None:
             if len(self._decode_graphs) >= 4:          # each graph owns its KV-cache pool: keep only a few shapes
@@ -378,6 +381,32 @@ class Transformer(nn.Module):
             out = self._decode(f, p, int(beam_size), self.log_domain_beam, False)
             self.last_gaps = out["gaps"]
             return out["ids"].long().contiguous()
+
+    def beam_search_nbest(self, object_features, position_features, beam_size=5, n_best=None, length_penalty=0.0):
+        """Beam search that stops at <END> (not the reference's beam_search, which stays the default): scores are
+        accumulated log-probabilities; a hypothesis whose last token is <END> (or <NULL>) is finished and continues with
+        <NULL> at an unchanged score; after max_length - 1 steps the beam_size hypotheses are ranked by
+        score / ((5 + len) / 6)^length_penalty, len = generated tokens up to and including the first <END> (before a
+        <NULL>; max_length - 1 if unfinished).  Inputs are tensors or a RegionBatch (position_features=None), as for
+        beam_search; sets last_gaps (score gap between the k-th and (k+1)-th candidate of every step, [T, B]).
+        -> (ids LongTensor [B, n_best, max_length] with <START> first, scores FloatTensor [B, n_best] (log-probability,
+            not normalised), lengths LongTensor [B, n_best]), best first; n_best defaults to beam_size."""
+        k = beam_size
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= int(k) <= 8:
+            raise ValueError(f"beam_size must be an integer in [1, 8], got {beam_size}")
+        k = int(k)
+        n = k if n_best is None else n_best
+        if isinstance(n, bool) or not isinstance(n, (int, np.integer)) or not 1 <= int(n) <= k:
+            raise ValueError(f"n_best must be an integer in [1, beam_size = {k}], got {n_best}")
+        alpha = float(length_penalty)
+        if not (math.isfinite(alpha) and alpha >= 0):
+            raise ValueError(f"length_penalty must be finite and >= 0, got {length_penalty}")
+        with torch.no_grad():
+            eng = self._engine()
+            f, p, _ = eng.prepare_inputs(object_features, position_features)
+            out = self._decode(f, p, k, True, False, stop_at_end=True, length_penalty=alpha, n_best=int(n))
+            self.last_gaps = out["gaps"]
+            return out["ids"].long(), out["score"].clone(), out["len"].long()
 
     def sample_captions(self, object_features, position_features, num_samples=1, temperature=1.0, seed=None):
         """num_samples captions per image drawn from the model: every token from softmax(logits / temperature) by the
@@ -742,7 +771,7 @@ class GraphedDecode:
 
     def __init__(self, model: Transformer, batch: int, regions: int, beam_size: int, log_domain: bool = False,
                  want_attention: bool = False, want_gaps: bool = False, cache=None, num_samples: int = 0,
-                 temperature: float = 1.0):
+                 temperature: float = 1.0, stop_at_end: bool = False, length_penalty: float = 0.0, n_best: int = 0):
         eng = model._engine()
         cfg = model.cfg
         self.eng = eng
@@ -751,6 +780,8 @@ class GraphedDecode:
         self.sampling = num_samples > 0                # the graph ticks the sampling counter: replays draw new samples
         if self.sampling:
             self.kw.update(num_samples=int(num_samples), temperature=float(temperature))
+        if stop_at_end:
+            self.kw.update(stop_at_end=True, length_penalty=float(length_penalty), n_best=int(n_best))
         self.cache = cache
         if cache is not None:                          # inputs = image numbers into a device-resident RegionCache
             assert regions == cache.regions
@@ -805,9 +836,12 @@ class GraphedDecode:
                         main.wait_stream(self._streams[i])
                     self.out = {
                         "ids": torch.cat([o["ids"] for o in outs], dim=0),
-                        "attention": torch.cat([o["attention"] for o in outs], dim=1) if outs[0]["attention"] is not None else None,
+                        "attention": torch.cat([o["attention"] for o in outs], dim=1) if outs[0].get("attention") is not None else None,
                         "gaps": torch.cat([o["gaps"] for o in outs], dim=1) if outs[0]["gaps"] is not None else None,
                     }
+                    if "len" in outs[0]:                               # <END>-aware beam search: per-image outputs
+                        self.out.update(score=torch.cat([o["score"] for o in outs], dim=0),
+                                        len=torch.cat([o["len"] for o in outs], dim=0))
 
     def run(self, feats: torch.Tensor, pos: Optional[torch.Tensor] = None, seed: Optional[int] = None):
         """Returns the engine's output dict (static device tensors, overwritten by the next run).  With a region

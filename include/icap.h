@@ -173,6 +173,30 @@ int icap_sample_tokens(int dtype, int64_t M, int64_t V, const void* logits, int6
 int icap_beam_select(int dtype, int64_t B, int64_t kin, int64_t V, const void* logits, int64_t ldl,
                      const float* prev_score, int64_t kout, float* out_score, int* out_parent, int* out_token,
                      float* gap, int log_domain, const float* stats, int64_t stats_ld, void* stream);
+/* Beam step of a search that stops at <END> (not in the reference, which extends every beam to max_length and scores it
+ * by summed probabilities, model.py:160-198).  Arguments as icap_beam_select, plus the hypotheses' token rows
+ * tokens[b*kin + r, 0..Tmax) (positions 0..t filled), the step t and the <END> / <NULL> ids:
+ *   - hypothesis r is FINISHED if t >= 1 and tokens[b*kin + r, t] is end_idx or pad_idx (the rule of icap_sample_tokens);
+ *   - an unfinished r offers every token j with score prev[b,r] + log_softmax(x_r)[j], x_r its logits as stored (bf16
+ *     or fp32): the arithmetic, in the same order, of icap_beam_select with log_domain = 1;
+ *   - a finished r offers exactly one candidate: token pad_idx with score prev[b,r], unchanged;
+ *   - the kout best candidates survive, written in descending order; ties go to the lower r*V + j; gap[b] = score_k -
+ *     score_{k+1} (+inf when there are only k candidates).
+ * A finished row reads no logits (no statistics either, with `stats`).  log_domain must be 1; 0 <= pad_idx < V;
+ * 0 <= t < Tmax - 1; at t = 0 kin*V > kout, at t >= 1 kin >= kout (every row offers at least one candidate). */
+int icap_beam_select_eos(int dtype, int64_t B, int64_t kin, int64_t V, const void* logits, int64_t ldl,
+                         const float* prev_score, int64_t kout, float* out_score, int* out_parent, int* out_token,
+                         float* gap, int log_domain, const float* stats, int64_t stats_ld, const int* tokens, int64_t Tmax,
+                         int64_t t, int end_idx, int pad_idx, void* stream);
+/* Final order of an <END>-aware beam search over k hypotheses per image (tokens rows b*k + s of Tmax ids, position 0 =
+ * <START>; score [B, k] accumulated log-probabilities), one warp per image:
+ *   len_s  = generated tokens up to and including the first end_idx; the tokens before a first pad_idx; Tmax - 1 if
+ *            neither occurs;
+ *   norm_s = score_s / ((5 + len_s) / 6)^alpha   (fp32; alpha finite and >= 0; alpha = 0 orders by log-probability);
+ *   the n best by norm (ties: lower s) in descending order: out_ids [B, n, Tmax] (the token rows), out_score [B, n]
+ *   (score_s, not normalised), out_len [B, n].  1 <= n <= k <= 8. */
+int icap_beam_finalize(int64_t B, int64_t k, int64_t Tmax, const int* tokens, const float* score, int end_idx, int pad_idx,
+                       float alpha, int64_t n, int* out_ids, float* out_score, int* out_len, void* stream);
 /* PolicyNetwork.sample (model_RL.py:93-97) on fp32 logits [M, V]: logp = log_softmax(x) per row, idx[row] (int64,
  * nullable) = arg-max (lowest index on ties, as torch.argmax on the CPU).  icap_log_softmax_bwd is its backward:
  * dx = dlogp - exp(logp) * rowsum(dlogp)  (the self-critical loss gathers log-probabilities, loss.py:90-103,145-158). */
