@@ -60,11 +60,20 @@ static inline cudaError_t icap_launch(void (*kern)(KArgs...), dim3 grid, dim3 bl
   cfg.numAttrs = icap_g_pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
-// Opts kernel K in to `smem` bytes of dynamic shared memory when it needs more than it was last given (48 KB needs no
-// opt-in).  One process drives one GPU, so a process-wide high-water mark per kernel is enough.
+// Opts kernel K in to `smem` bytes of dynamic shared memory when it needs more than it may use now.  Without the opt-in
+// a kernel gets 48 KB of shared memory in all, its static shared memory included, so the starting limit is the kernel's
+// own (48 KB of dynamic shared memory next to 32 static bytes fail to launch).  One process drives one GPU, so a
+// process-wide high-water mark per kernel is enough.
 template <auto K>
 static inline int ensure_smem(size_t smem) {
-  static size_t cur = 48 * 1024;
+  static size_t cur = 0;
+  static bool known = false;
+  if (!known) {
+    cudaFuncAttributes a;
+    ICAP_CUDA(cudaFuncGetAttributes(&a, K));
+    cur = (size_t)a.maxDynamicSharedSizeBytes;
+    known = true;
+  }
   if (smem > cur) {
     ICAP_CUDA(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cur = smem;

@@ -1012,6 +1012,7 @@ void launch_beam_select(int dtype, int64_t B, int64_t kin, int64_t V, const void
 extern "C" int icap_xent(int dtype, int64_t M, int64_t V, void* logits, int64_t ldl, const int* targets,
                          int ignore_index, const float* inv_count, float* row_loss, int write_grad, void* stream) {
   ICAP_ARG(M > 0 && V > 0 && logits && targets && row_loss && inv_count, "icap_xent: null/empty argument");
+  ICAP_ARG(ldl >= V && V < (1ll << 31) && M < (1ll << 31), "icap_xent: bad logits shape");
   const int esz = dtype == ICAP_F32 ? 4 : 2;
   const int vec = ((uintptr_t)logits % 16 == 0) && ((ldl * esz) % 16 == 0);
   size_t smem = (size_t)V * 4;
@@ -1039,6 +1040,7 @@ extern "C" int icap_xent(int dtype, int64_t M, int64_t V, void* logits, int64_t 
 extern "C" int icap_xent_finalize(int64_t M, const float* row_loss, const float* inv_count, int focal, float* out2,
                                   void* stream) {
   ICAP_ARG(M > 0 && row_loss && inv_count && out2, "icap_xent_finalize: null/empty argument");
+  ICAP_ARG(M < (1ll << 31), "icap_xent_finalize: too many rows");
   icap_launch(xent_finalize_kernel, 1, NT, 0, (cudaStream_t)stream, (int)M, row_loss, inv_count, focal, out2);
   ICAP_LAUNCH_CHECK("icap_xent_finalize");
   return 0;
@@ -1047,6 +1049,7 @@ extern "C" int icap_xent_finalize(int64_t M, const float* row_loss, const float*
 extern "C" int icap_argmax(int dtype, int64_t M, int64_t V, const void* logits, int64_t ldl, int* out,
                            int64_t out_stride, float* gap, void* stream) {
   ICAP_ARG(M > 0 && V > 0 && logits && out, "icap_argmax: null/empty argument");
+  ICAP_ARG(ldl >= V && V < (1ll << 31) && M < (1ll << 31), "icap_argmax: bad logits shape");
   cudaStream_t st = (cudaStream_t)stream;
   dispatch_act(dtype, [&](auto tag) {
     icap_launch(argmax_kernel<decltype(tag)>, (unsigned)M, NT, 0, st, V, logits, ldl, out, out_stride, gap);
@@ -1128,6 +1131,7 @@ extern "C" int icap_beam_finalize(int64_t B, int64_t k, int64_t Tmax, const int*
 extern "C" int icap_log_softmax_argmax(int64_t M, int64_t V, const float* x, int64_t ldx, float* logp, int64_t ldo,
                                        long long* idx, void* stream) {
   ICAP_ARG(M > 0 && V > 0 && x && logp, "icap_log_softmax_argmax: null/empty argument");
+  ICAP_ARG(ldx >= V && ldo >= V && V < (1ll << 31) && M < (1ll << 31), "icap_log_softmax_argmax: bad logits shape");
   icap_launch(log_softmax_argmax_kernel, (unsigned)M, NT, 0, (cudaStream_t)stream, (int)V, x, ldx, logp, ldo, idx);
   ICAP_LAUNCH_CHECK("icap_log_softmax_argmax");
   return 0;
@@ -1136,6 +1140,8 @@ extern "C" int icap_log_softmax_argmax(int64_t M, int64_t V, const float* x, int
 extern "C" int icap_log_softmax_bwd(int64_t M, int64_t V, const float* logp, int64_t ldp, const float* dlogp, int64_t ldd,
                                     float* dx, int64_t ldx, void* stream) {
   ICAP_ARG(M > 0 && V > 0 && logp && dlogp && dx, "icap_log_softmax_bwd: null/empty argument");
+  ICAP_ARG(ldp >= V && ldd >= V && ldx >= V && V < (1ll << 31) && M < (1ll << 31),
+           "icap_log_softmax_bwd: bad logits shape");
   icap_launch(log_softmax_bwd_kernel, (unsigned)M, NT, 0, (cudaStream_t)stream, (int)V, logp, ldp, dlogp, ldd, dx, ldx);
   ICAP_LAUNCH_CHECK("icap_log_softmax_bwd");
   return 0;

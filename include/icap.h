@@ -140,14 +140,14 @@ int icap_gemm_ln(int64_t M, int64_t N, int64_t K, const void* A, int64_t lda, co
                  float* rstd_out, float eps, float p_drop, uint64_t seed, const int* seed_dev, void* stream);
 /* Fused log-softmax + NLL per row; with write_grad=1 the logits are overwritten IN PLACE by
  * (softmax - onehot) * inv_count[0] (zero rows for ignored targets).  row_loss: fp32 [M].
- * Replaces CrossEntropyLoss(ignore_index=pad_idx, 'mean'), model.py:76,93-96. */
+ * Replaces CrossEntropyLoss(ignore_index=pad_idx, 'mean'), model.py:76,93-96.  Rows of stride ldl >= V; M, V < 2^31. */
 int icap_xent(int dtype, int64_t M, int64_t V, void* logits, int64_t ldl, const int* targets, int ignore_index,
               const float* inv_count, float* row_loss, int write_grad, void* stream);
 /* out2[0] = mean loss (focal=1: (1-exp(-ce))^2 * ce, loss.py:20-28); out2[1] = d loss / d ce. */
 int icap_xent_finalize(int64_t M, const float* row_loss, const float* inv_count, int focal, float* out2, void* stream);
 
 /* out[row*out_stride] = argmax_j logits[row][j] (lowest index on ties); gap = top1 - top2 (nullable).
- * Replaces argmax(Softmax(classifer(.))), model.py:125-128. */
+ * Replaces argmax(Softmax(classifer(.))), model.py:125-128.  Rows of stride ldl >= V; M, V < 2^31. */
 int icap_argmax(int dtype, int64_t M, int64_t V, const void* logits, int64_t ldl, int* out, int64_t out_stride,
                 float* gap, void* stream);
 /* Sampled decoding step for M rows (row r = image * n + sample; tokens / logp rows of stride Tmax / ldp):

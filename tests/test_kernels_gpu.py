@@ -471,54 +471,6 @@ def test_mha_decode_matches_full_attention():
 
 
 # ------------------------------------------------------------------------------------------ loss / selection
-@pytest.mark.parametrize("act", [F32, BF16])
-@pytest.mark.parametrize("M,V", [(50, 397), (64, 10000), (8, 60000)])
-def test_xent_and_finalize(act, M, V):
-    g = torch.Generator(device="cuda").manual_seed(V)
-    ldl = (V + 7) // 8 * 8
-    logits = (torch.randn(M, ldl, device=dev(), generator=g) * 2).to(dt(act))
-    tgt = torch.randint(0, V, (M,), device=dev(), generator=g, dtype=torch.int32)
-    tgt[::5] = 0
-    n = int((tgt != 0).sum())
-    inv = torch.tensor([1.0 / n], device=dev())
-    x64 = logits[:, :V].double().requires_grad_(True)
-    ref = torch.nn.functional.cross_entropy(x64, tgt.long(), ignore_index=0)
-    ref.backward()
-    row_loss = torch.empty(M, device=dev())
-    out2 = torch.empty(2, device=dev())
-    work = logits.clone()
-    N.call("icap_xent", act, M, V, work.data_ptr(), ldl, tgt.data_ptr(), 0, inv.data_ptr(), row_loss.data_ptr(), 1, S())
-    N.call("icap_xent_finalize", M, row_loss.data_ptr(), inv.data_ptr(), 0, out2.data_ptr(), S())
-    torch.cuda.synchronize()
-    assert abs(float(out2[0]) - float(ref)) / float(ref) < 2e-6
-    assert float(out2[1]) == 1.0
-    assert rel_err(work[:, :V], x64.grad) < (1e-5 if act == F32 else 1e-2)
-    # focal (loss.py:20-28)
-    N.call("icap_xent_finalize", M, row_loss.data_ptr(), inv.data_ptr(), 1, out2.data_ptr(), S())
-    ce = ref.detach().clone().requires_grad_(True)
-    fl = (1 - torch.exp(-ce)) ** 2 * ce
-    fl.backward()
-    torch.cuda.synchronize()
-    assert abs(float(out2[0]) - float(fl)) / float(fl) < 1e-5
-    assert abs(float(out2[1]) - float(ce.grad)) / float(ce.grad) < 1e-5
-
-
-def test_argmax_and_gap():
-    M, V = 33, 10000
-    g = torch.Generator(device="cuda").manual_seed(9)
-    x = torch.randn(M, V, device=dev(), generator=g)
-    x[3, 17] = x[3, 5000] = 50.0          # exact tie -> lowest index
-    out = torch.zeros(M, 4, dtype=torch.int32, device=dev())
-    gap = torch.empty(M, device=dev())
-    N.call("icap_argmax", F32, M, V, x.data_ptr(), V, out.data_ptr() + 4 * 2, 4, gap.data_ptr(), S())
-    torch.cuda.synchronize()
-    assert torch.equal(out[:, 2].long(), x.argmax(1))
-    assert int(out[3, 2]) == 17 and float(gap[3]) == 0.0
-    top2 = x.topk(2, dim=1).values
-    assert torch.allclose(gap, top2[:, 0] - top2[:, 1])
-    assert int(out[:, [0, 1, 3]].abs().sum()) == 0
-
-
 @pytest.mark.parametrize("log_domain", [0, 1])
 @pytest.mark.parametrize("kin,kout,V", [(1, 3, 397), (3, 3, 10000), (5, 5, 10000), (5, 5, 401)])
 def test_beam_select(log_domain, kin, kout, V):

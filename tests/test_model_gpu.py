@@ -255,6 +255,10 @@ def test_model_a_vs_oracle(precision, tol_logits, tol_loss):
     loss = m(f, p, c)["loss"]
     assert abs(float(loss) - float(ref_loss)) / float(ref_loss) < tol_loss
     loss.backward()
+    assert_grads_match(m, ref_grads, precision)
+
+
+def assert_grads_match(m, ref_grads, precision):
     # Gradients: Frobenius-relative error per parameter.  (A max-abs criterion is not robust here: a ReLU
     # pre-activation within rounding distance of 0 flips its mask bit and moves one row of dW1 by ~1e-3 of
     # max|dW1| -- observed, and inherent to any re-ordered fp32 summation.)  bf16 mode: activations AND
@@ -351,7 +355,8 @@ def test_odd_shapes_vs_oracle(B, R):
 
 def test_config5_scaled_shapes_vs_oracle():
     """BASELINE configs[4] shapes (scaled variant): d_model 1024, 16 heads, FFN 4096, 100 regions, vocab 30k (2+2
-    blocks here so the CPU oracle finishes in seconds): logits fp32 / bf16, beam-5 ids in fp32."""
+    blocks here so the CPU oracle finishes in seconds): logits fp32 / bf16, beam-5 ids in fp32, loss and every
+    parameter gradient in both precisions (the vocabulary-30000 cross-entropy and bias-gradient kernels)."""
     kw = dict(num_vocab=30000, max_length=22, encode_dim_positions=84, encode_dim_features=2048, output_name="x",
               dropout=0.0, encode_input_size=1024, encode_q_k_dim=1024, encode_v_dim=1024, encode_hidden_size=4096,
               encode_num_blocks=2, encode_num_heads=16, dim_word_embedding=1024, decode_input_size=1024,
@@ -366,11 +371,17 @@ def test_config5_scaled_shapes_vs_oracle():
     out = m.beam_search(f, p, beam_size=5)
     assert out.shape == ref.shape
     assert not ids_match_except_near_ties(out, ref, ref_trace, tol=1e-6, what="beam-5")
+    ref_loss, ref_grads = O.loss_and_grads(sd, cfg, f, p, c)
+    loss = m(f, p, c)["loss"]
+    assert abs(float(loss) - float(ref_loss)) / float(ref_loss) < 1e-5
+    loss.backward()
+    assert_grads_match(m, ref_grads, "fp32")
     mb = build(kw, sd, "bf16")
     assert rel(mb.logits(f, p, c), ref_logits) < 2e-2
     loss = mb(f, p, c)["loss"]
-    ref_loss, _ = O.loss_and_grads(sd, cfg, f, p, c)
     assert abs(float(loss) - float(ref_loss)) / float(ref_loss) < 2e-2
+    loss.backward()
+    assert_grads_match(mb, ref_grads, "bf16")
 
 
 def test_full_size_decode_properties_bf16(monkeypatch):
